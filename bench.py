@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- MCTS simulations/sec of the batched search hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
            bench.py --gpus N --steps K --warmup W
 
@@ -22,6 +22,9 @@ One JSON line on stdout.  Top level = the headline workload:
 Without --workload the line also carries
   workloads  {cartpole_4096x50 (configs[2]), selfplay_pendulum_32768x200 (configs[4])}: the same record for each
   strong     (N > 1) the headline workload with the 65536 trees SPLIT over the N GPUs (BASELINE config 4 as worded)
+`--dump-outputs DIR` writes what the last timed step of the headline workload returned (rank 0's trees) as DIR/<name>.npy, so
+that two builds can be compared output for output: the root results (actions, counts, Q, V_target, n_children), or for a
+self-play workload the tensors of SelfPlayDriver.step.
 `--impl reference` times the CPU port alone (the reference itself is Python + gym and cannot travel to the
 GPU box; its single-core numbers measured in the build container are in BASELINE.md / DESIGN.md).
 """
@@ -72,6 +75,7 @@ EXTRA_WORKLOADS = ("cartpole_4096x50", "selfplay_pendulum_32768x200")
 SELFPLAY_BROADCAST_EVERY = 4
 FLOP_PER_EVAL = {"discrete": 2 * 17280, "continuous": 2 * 34048}  # SURVEY 8d
 PARITY_SAMPLE = 256  # trees per rank compared with the oracle inside the bench
+DUMP_LIMIT_BYTES = 64 << 20  # --dump-outputs: larger outputs are written as a fixed sample of their rows
 
 
 def make_roots(variant: str, B: int, seed: int = 34) -> np.ndarray:
@@ -198,6 +202,24 @@ def measure_traffic(workload: str):
         return None, f"ncu failed: {exc}"
 
 
+def dump_outputs(outs: dict, directory: str) -> None:
+    """Write each tensor of `outs` (one row per tree or environment) as directory/<name>.npy: float32 as it is, every other
+    dtype as float64 (exact for the int32 counts).  Above DUMP_LIMIT_BYTES only a seeded sample of rows is written, the
+    same rows for every array, and their indices go to rows.npy."""
+    arrs = {k: v.cpu().numpy() for k, v in outs.items()}
+    arrs = {k: a if a.dtype == np.float32 else a.astype(np.float64) for k, a in arrs.items()}
+    n_rows = len(next(iter(arrs.values())))
+    row_bytes = sum(a.nbytes for a in arrs.values()) / n_rows
+    budget = DUMP_LIMIT_BYTES - 4096  # room for the .npy headers
+    if row_bytes * n_rows > budget:
+        rows = np.sort(np.random.default_rng(0).choice(n_rows, int(budget // (row_bytes + 8)), replace=False))
+        arrs = {k: a[rows] for k, a in arrs.items()}
+        arrs["rows"] = rows.astype(np.float64)
+    os.makedirs(directory, exist_ok=True)
+    for k, a in arrs.items():
+        np.save(os.path.join(directory, k + ".npy"), a)
+
+
 def cpu_port_throughput(variant: str, N: int, roots: np.ndarray, weights: np.ndarray, seconds: float, threads: int):
     """Time the CPU oracle (C port of the reference search) on a bounded sample; returns (sims/s, sample text)."""
     from oracle import azo
@@ -300,8 +322,10 @@ class Ctx:
             self.dist.destroy_process_group()
 
 
-def measure(ctx: Ctx, args, name: str, trees_per_gpu=None, scaling: str = "weak", cpu_baseline: bool = True, traffic: bool = True) -> dict:
-    """One workload on every rank; returns the record (meaningful on rank 0)."""
+def measure(ctx: Ctx, args, name: str, trees_per_gpu=None, scaling: str = "weak", cpu_baseline: bool = True, traffic: bool = True,
+            dump_dir=None) -> dict:
+    """One workload on every rank; returns the record (meaningful on rank 0).  With dump_dir, rank 0 writes the outputs of the
+    last timed step there (dump_outputs)."""
     torch, dist = ctx.torch, ctx.dist
     from alphazero_gym_b200.engine import SearchEngine
     variant, B_full, N = WORKLOADS[name]
@@ -405,6 +429,8 @@ def measure(ctx: Ctx, args, name: str, trees_per_gpu=None, scaling: str = "weak"
     ctx.barrier()
     ms = e0.elapsed_time(e1)
     eng.status()
+    if dump_dir and rank == 0:  # before the e2e and roofline passes below reuse the engine
+        dump_outputs(drv.t if selfplay else res, dump_dir)
     counters = eng.counters()
     launches_per_step = counters["launches"] + extra_launches
     if selfplay:
@@ -638,14 +664,18 @@ def main():
                     help="whole-search persistent kernel (AZG_FLAG_FUSED); auto = the engine's default")
     ap.add_argument("--eval", default="q8", choices=["fp32", "q8"],
                     help="leaf evaluation arithmetic: int8-sliced tcgen05 products (default) or FP32 FMA (mlp.cuh)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the headline workload's last timed step as DIR/<name>.npy (float32/float64, at most 64 MB)")
     args = ap.parse_args()
     head = args.workload or HEADLINE
     variant, B, N = WORKLOADS[head]
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs needs --impl ours")
         run_reference(args, variant, B, N, int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1")))
         return
     ctx = Ctx()
-    rec = measure(ctx, args, head)
+    rec = measure(ctx, args, head, dump_dir=args.dump_outputs)
     extras, strong = {}, None
     if args.workload is None and not args.no_extra:
         for name in EXTRA_WORKLOADS:

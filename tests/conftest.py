@@ -1,8 +1,6 @@
 import os
 import sys
 
-import pytest
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -10,12 +8,3 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "needs_reference: imports /root/reference live (build container only)")
-
-
-def pytest_collection_modifyitems(config, items):
-    have_ref = os.path.isdir("/root/reference/alphazero")
-    skip_ref = pytest.mark.skip(reason="/root/reference not present (GPU box)")
-    for item in items:
-        if "needs_reference" in item.keywords and not have_ref:
-            item.add_marker(skip_ref)

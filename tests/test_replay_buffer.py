@@ -1,7 +1,6 @@
 """DeviceReplayBuffer (alphazero_gym_b200/selfplay.py) keeps the semantics of the reference's list-based ReplayBuffer
 (alphazero/agent/buffers.py): FIFO with overwrite of the oldest entry, shuffled mini-batches with the remainder folded into
 the last batch.  Runs on CPU tensors here; the same code holds CUDA tensors in the self-play driver."""
-import numpy as np
 import pytest
 import torch
 
@@ -60,20 +59,17 @@ def test_batches_cover_the_buffer_once_per_epoch():
     assert sorted(seen) == [float(i) for i in range(37)]
 
 
-@pytest.mark.needs_reference
+# What the reference's ReplayBuffer(max_size=10, batch_size=4) holds after the rows 0..26 were stored one by one: V of its
+# experience list in list order, and the sizes of the mini-batches it yields after reshuffle().  Recorded here because the
+# reference is not part of this repository.
+REF_EXPERIENCE_V = [20, 21, 22, 23, 24, 25, 26, 17, 18, 19]
+REF_BATCH_SIZES = [4, 6]
+
+
 def test_against_the_reference_class():
-    import sys
-    sys.path.insert(0, "/root/reference")
-    from alphazero.agent.buffers import ReplayBuffer
-    ref = ReplayBuffer(max_size=10, batch_size=4)
     rb = DeviceReplayBuffer(max_size=10, batch_size=4, obs_dim=3, cmax=3, device="cpu")
     for lo in range(0, 27, 3):
-        rows = _rows(lo, lo + 3)
-        rb.store(rows)
-        for i in range(3):
-            ref.store(tuple(rows[k][i].numpy() for k in ROW_KEYS))
-    assert [float(e[4]) for e in ref.experience] == rb.data["V_target"][: len(rb)].tolist()
-    np.random.seed(0)
-    ref.reshuffle()
+        rb.store(_rows(lo, lo + 3))
+    assert [float(v) for v in REF_EXPERIENCE_V] == rb.data["V_target"][: len(rb)].tolist()
     rb.reshuffle()
-    assert [len(b[0]) for b in ref] == [b["obs"].shape[0] for b in rb]
+    assert REF_BATCH_SIZES == [b["obs"].shape[0] for b in rb]
