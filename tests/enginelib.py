@@ -17,8 +17,10 @@ def engine_config(cfg: azo.Config, max_trees: int, **kw) -> EngineConfig:
     return EngineConfig(**d)
 
 
-def run_engine(cfg: azo.Config, weights, root_state, root_n_init=None, tree_id0=0, tapes=None, dump=True, host=False, **kw):
-    """One batched search on cuda:0 through the C ABI; returns oracle-shaped dict (results [+ dump] + counters)."""
+def run_engine(cfg: azo.Config, weights, root_state, root_n_init=None, tree_id0=0, tapes=None, dump=True, host=False, kernel=False,
+               **kw):
+    """One batched search on cuda:0 through the C ABI; returns oracle-shaped dict (results [+ dump] + counters [+ kernel: the
+    whole-search kernel that ran, "none" for one launch per kernel and simulation])."""
     root_state = np.ascontiguousarray(root_state, np.float64)
     B = root_state.shape[0]
     eng = SearchEngine(engine_config(cfg, B, **kw))
@@ -43,6 +45,8 @@ def run_engine(cfg: azo.Config, weights, root_state, root_n_init=None, tree_id0=
         c = eng.counters(B)
         out["counters"] = np.array([c["sims"], c["levels"], c["children_scanned"], c["pw_inserts"], c["evals"],
                                     c["rng_draws"], c["terminal_leaf_sims"], c["launches"]], np.int64)
+        if kernel:
+            out["kernel"] = eng.fused_stats()["kernel"]
         return out
     finally:
         eng.close()
