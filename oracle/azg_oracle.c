@@ -328,7 +328,12 @@ static void net_free(net_t* n) {
 static inline float act_fn(const azo_config* c, float v) {
     if (c->activation == AZO_ACT_RELU) return v > 0.0f ? v : 0.0f;
     if (c->activation == AZO_ACT_LEAKYRELU) return v > 0.0f ? v : v * 0.01f;
-    if (c->activation == AZO_ACT_RELU6) return fminf(fmaxf(v, 0.0f), 6.0f);
+    if (c->activation == AZO_ACT_RELU6) {
+        /* a NaN is a missing operand of fmaxf, as on the GPU: 0.  (glibc's fmaxf returns NaN for a signaling NaN, and fminf
+         * then returns 6; tests/test_primitives_gpu.py compares every f32 input.) */
+        if (v != v) return 0.0f;
+        return fminf(fmaxf(v, 0.0f), 6.0f);
+    }
     if (c->activation == AZO_ACT_SILU) {
         if (v != v) return v;
         const float e = c->math_mode == AZO_MATH_DET ? azo_det_expf(-v) : expf(-v);
@@ -1082,4 +1087,79 @@ int azo_search(const azo_config* cfg, const float* weights, int64_t n_weights, i
     free(pw_table);
     if (!cfg->use_eval_tape) net_free(&net);
     return rc;
+}
+
+/* ------------------------------------------------------------------------------------------------
+ * Building blocks for the primitive tests (azg_oracle.h): batched deterministic functions, and the
+ * MT19937 generators on a caller-held state.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct { int32_t fn; const void* in; void* out; int64_t i0, i1; } eval_job_t;
+
+static void* eval_worker(void* arg) {
+    const eval_job_t* J = (const eval_job_t*)arg;
+    const float* fi = (const float*)J->in; float* fo = (float*)J->out;
+    const double* di = (const double*)J->in; double* dout = (double*)J->out;
+    azo_config c;
+    memset(&c, 0, sizeof c);
+    c.math_mode = AZO_MATH_DET;
+    c.activation = J->fn - AZO_FN_ACT;
+    for (int64_t i = J->i0; i < J->i1; ++i) {
+        switch (J->fn) {
+            case AZO_FN_EXPF: fo[i] = azo_det_expf(fi[i]); break;
+            case AZO_FN_EXPM1F: fo[i] = azo_det_expm1f(fi[i]); break;
+            case AZO_FN_TANHF: fo[i] = azo_det_tanhf(fi[i]); break;
+            case AZO_FN_SIN: dout[i] = azo_det_sin(di[i]); break;
+            case AZO_FN_COS: dout[i] = azo_det_cos(di[i]); break;
+            case AZO_FN_LOG: dout[i] = azo_det_log(di[i]); break;
+            default: fo[i] = act_fn(&c, fi[i]); break;
+        }
+    }
+    return NULL;
+}
+
+int azo_det_eval(int32_t fn, const void* in, void* out, int64_t n, int32_t n_threads) {
+    if (!((fn >= AZO_FN_EXPF && fn <= AZO_FN_LOG) || (fn >= AZO_FN_ACT && fn <= AZO_FN_ACT + AZO_ACT_HARDSWISH))) return -2;
+    if (n_threads < 1) n_threads = 1;
+    if (n_threads > 256) n_threads = 256;
+    eval_job_t jobs[256];
+    pthread_t th[256];
+    for (int i = 0; i < n_threads; ++i) {
+        eval_job_t j = {fn, in, out, n * i / n_threads, n * (i + 1) / n_threads};
+        jobs[i] = j;
+    }
+    for (int i = 1; i < n_threads; ++i) pthread_create(&th[i], NULL, eval_worker, &jobs[i]);
+    eval_worker(&jobs[0]);
+    for (int i = 1; i < n_threads; ++i) pthread_join(th[i], NULL);
+    return 0;
+}
+
+/* st = 624 state words + the index word; the generators of rng_t run on a copy */
+static void mt_load(rng_t* g, const uint32_t* st) { memcpy(g->mt, st, 624 * 4); g->mti = (int)st[624]; g->draws = 0; }
+static void mt_store(const rng_t* g, uint32_t* st) { memcpy(st, g->mt, 624 * 4); st[624] = (uint32_t)g->mti; }
+
+void azo_mt_seed(uint32_t* st, uint64_t seed) { rng_t g; mt_seed(&g, seed); mt_store(&g, st); }
+uint32_t azo_mt_u32(uint32_t* st) { rng_t g; mt_load(&g, st); const uint32_t r = mt_next(&g); mt_store(&g, st); return r; }
+double azo_mt_random(uint32_t* st) {
+    rng_t g; mt_load(&g, st); g.mt_mode = 1;
+    const double r = rng_random(&g);
+    mt_store(&g, st);
+    return r;
+}
+int32_t azo_mt_below(uint32_t* st, int32_t n) {
+    rng_t g; mt_load(&g, st); g.mt_mode = 1;
+    const int32_t r = rng_below(&g, n);
+    mt_store(&g, st);
+    return r;
+}
+void azo_torch_seed(uint32_t* st, uint64_t seed) { rng_t g; torch_manual_seed(&g, seed); memcpy(st, g.tmt, 624 * 4); st[624] = (uint32_t)g.tmti; }
+double azo_torch_uniform(uint32_t* st) {
+    rng_t g; memcpy(g.tmt, st, 624 * 4); g.tmti = (int)st[624]; g.tdraws = 0;
+    const double r = torch_uniform(&g);
+    memcpy(st, g.tmt, 624 * 4); st[624] = (uint32_t)g.tmti;
+    return r;
+}
+
+void azo_rng_block_batch(uint64_t seed, const int64_t* tree, const int32_t* stream, const int64_t* idx, const int32_t* block, int64_t n,
+                         uint32_t* out) {
+    for (int64_t i = 0; i < n; ++i) rng_block(seed, tree[i], stream[i], idx[i], block[i], out + 4 * i);
 }

@@ -180,6 +180,9 @@ int32_t azo_pw_limit(double c_pw, double kappa, int32_t n); /* ceil(c_pw*(n+1)**
 /* ---- building blocks exported for known-answer tests and the golden harness ------- */
 uint32_t azo_rng_u32(uint64_t seed, int64_t tree, int32_t stream, int64_t idx, int32_t block, int32_t word);
 /* noise for the j-th progressive-widening insert of `tree`: component uniform + K standard normals */
+/* rng_block of n counters: out[i][0..3] = the four words of (tree[i], stream[i], idx[i], block[i]) */
+void azo_rng_block_batch(uint64_t seed, const int64_t* tree, const int32_t* stream, const int64_t* idx, const int32_t* block, int64_t n,
+                         uint32_t* out);
 void azo_noise(uint64_t seed, int64_t tree, int64_t j, int32_t K, float* u_comp, float* z);
 /* batched MLP forward (deterministic fmaf order): out_V [n], out_head [n][P] raw head outputs */
 void azo_mlp_forward(const azo_config* cfg, const float* weights, int32_t n, const float* x, float* out_V, float* out_head);
@@ -195,6 +198,29 @@ float azo_det_tanhf(float x);
 double azo_det_sin(double x);
 double azo_det_cos(double x);
 double azo_det_log(double x);
+
+/* Batched evaluation of one deterministic function over n elements with n_threads threads (exhaustive accuracy sweeps
+ * and engine comparisons run at C speed).  fn = AZO_FN_*: expf / expm1f / tanhf and AZO_FN_ACT + AZO_ACT_* (act_fn in
+ * AZO_MATH_DET mode) read and write float; sin / cos / log read and write double. */
+#define AZO_FN_EXPF 0
+#define AZO_FN_EXPM1F 1
+#define AZO_FN_TANHF 2
+#define AZO_FN_SIN 3
+#define AZO_FN_COS 4
+#define AZO_FN_LOG 5
+#define AZO_FN_ACT 16
+int azo_det_eval(int32_t fn, const void* in, void* out, int64_t n, int32_t n_threads);
+
+/* The MT19937 generators of AZO_RNG_MT19937 on a caller-held state of 625 words (624 state words + the index word).
+ * CPython `random`: azo_mt_seed = random.seed(int) (init_by_array), azo_mt_u32 = getrandbits(32), azo_mt_random =
+ * random(), azo_mt_below(n) = _randbelow(n).  torch's CPU generator: azo_torch_seed = torch.manual_seed (init_genrand of the
+ * low 32 bits), azo_torch_uniform = one double uniform (53 bits of two outputs). */
+void azo_mt_seed(uint32_t* st, uint64_t seed);
+uint32_t azo_mt_u32(uint32_t* st);
+double azo_mt_random(uint32_t* st);
+int32_t azo_mt_below(uint32_t* st, int32_t n);
+void azo_torch_seed(uint32_t* st, uint64_t seed);
+double azo_torch_uniform(uint32_t* st);
 
 #ifdef __cplusplus
 }

@@ -102,6 +102,15 @@ def lib():
         for n in ("sin", "cos", "log"):
             f = getattr(L, "azo_det_" + n)
             f.restype, f.argtypes = C.c_double, [C.c_double]
+        L.azo_det_eval.restype, L.azo_det_eval.argtypes = C.c_int, [C.c_int32, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32]
+        L.azo_rng_block_batch.restype = None
+        L.azo_rng_block_batch.argtypes = [C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]
+        L.azo_mt_seed.restype, L.azo_mt_seed.argtypes = None, [C.c_void_p, C.c_uint64]
+        L.azo_mt_u32.restype, L.azo_mt_u32.argtypes = C.c_uint32, [C.c_void_p]
+        L.azo_mt_random.restype, L.azo_mt_random.argtypes = C.c_double, [C.c_void_p]
+        L.azo_mt_below.restype, L.azo_mt_below.argtypes = C.c_int32, [C.c_void_p, C.c_int32]
+        L.azo_torch_seed.restype, L.azo_torch_seed.argtypes = None, [C.c_void_p, C.c_uint64]
+        L.azo_torch_uniform.restype, L.azo_torch_uniform.argtypes = C.c_double, [C.c_void_p]
         _lib = L
     return _lib
 
@@ -281,6 +290,54 @@ def obs(cfg: Config, state: np.ndarray) -> np.ndarray:
 
 def rng_u32(seed: int, tree: int, stream: int, idx: int, block: int = 0, word: int = 0) -> int:
     return int(lib().azo_rng_u32(seed, tree, stream, idx, block, word))
+
+
+def rng_blocks(seed: int, tree: np.ndarray, stream: np.ndarray, idx: np.ndarray, block: np.ndarray) -> np.ndarray:
+    """The four Philox words of every counter (tree[i], stream[i], idx[i], block[i]) under key `seed`: uint32 [n, 4]."""
+    tree, idx = np.ascontiguousarray(tree, np.int64), np.ascontiguousarray(idx, np.int64)
+    stream, block = np.ascontiguousarray(stream, np.int32), np.ascontiguousarray(block, np.int32)
+    out = np.empty((tree.size, 4), np.uint32)
+    lib().azo_rng_block_batch(seed, _p(tree), _p(stream), _p(idx), _p(block), tree.size, _p(out))
+    return out
+
+
+FN_EXPF, FN_EXPM1F, FN_TANHF, FN_SIN, FN_COS, FN_LOG, FN_ACT = 0, 1, 2, 3, 4, 5, 16
+_FN = {"expf": FN_EXPF, "expm1f": FN_EXPM1F, "tanhf": FN_TANHF, "sin": FN_SIN, "cos": FN_COS, "log": FN_LOG}
+
+
+def det_eval(fn, x: np.ndarray, n_threads: int = 8) -> np.ndarray:
+    """Deterministic function `fn` ("expf", "expm1f", "tanhf" on float32; "sin", "cos", "log" on float64; or an ACT_* code:
+    the activation in MATH_DET mode, float32) over every element of x, in threaded C."""
+    code = _FN[fn] if isinstance(fn, str) else FN_ACT + int(fn)
+    dt = np.float64 if code in (FN_SIN, FN_COS, FN_LOG) else np.float32
+    x = np.ascontiguousarray(x, dt)
+    out = np.empty_like(x)
+    rc = lib().azo_det_eval(code, _p(x), _p(out), x.size, n_threads)
+    if rc != 0:
+        raise ValueError(f"azo_det_eval: unknown function {fn!r}")
+    return out
+
+
+class MT19937:
+    """The oracle's MT19937 generators (AZO_RNG_MT19937): kind "python" is CPython's `random` seeded with random.seed(seed),
+    kind "torch" is torch's CPU generator after torch.manual_seed(seed)."""
+
+    def __init__(self, seed: int, kind: str = "python"):
+        self.kind = kind
+        self.st = np.zeros(625, np.uint32)
+        (lib().azo_mt_seed if kind == "python" else lib().azo_torch_seed)(_p(self.st), seed)
+
+    def u32(self) -> int:
+        return int(lib().azo_mt_u32(_p(self.st)))
+
+    def random(self) -> float:
+        return lib().azo_mt_random(_p(self.st))
+
+    def below(self, n: int) -> int:
+        return int(lib().azo_mt_below(_p(self.st), n))
+
+    def uniform(self) -> float:
+        return lib().azo_torch_uniform(_p(self.st))
 
 
 def noise(seed: int, tree: int, j: int, K: int):
