@@ -15,6 +15,7 @@
 #include <map>
 #include <string>
 #include <tuple>
+#include <type_traits>
 #include <utility>
 #include <vector>
 
@@ -92,6 +93,7 @@ struct azg_engine {
     cudaLaunchAttribute l2attr;
     int l2_on = 0;
     bool fused = false;  // AZG_FLAG_FUSED: the whole continuous search in one persistent kernel (qmlp2.cuh)
+    bool mcc = false;    // AZG_FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS: the continuous kernels are instantiated for env::MountainCarContinuous
     // results staging (device) + pinned host staging for the *_host entry point
     float* r_actions = nullptr;
     int32_t* r_counts = nullptr;
@@ -172,12 +174,15 @@ extern "C" int azg_create(const azg_config* cfg, azg_engine** out) {
     if (c.activation < AZG_ACT_RELU || c.activation > AZG_ACT_HARDSWISH) return fail(AZG_EINVAL, "activation must be one of AZG_ACT_*");
     if ((c.flags & AZG_FLAG_EVAL_Q8) && c.activation > AZG_ACT_ELU)
         return fail(AZG_EINVAL, "AZG_FLAG_EVAL_Q8 serves relu and elu (the configured activations); the others run on the FP32 kernel");
+    const bool mcc = (c.flags & AZG_FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS) != 0;
+    if (mcc && (c.variant != AZG_CONTINUOUS || c.state_dim != 2))
+        return fail(AZG_EINVAL, "AZG_FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS needs the continuous variant and state_dim 2");
     if (c.variant == AZG_DISCRETE) {
         if (c.num_actions != 2 || c.state_dim != 4)
             return fail(AZG_EINVAL, "discrete variant is CartPole: num_actions must be 2 and state_dim 4");
         if (c.max_rollouts + 2 > 65534) return fail(AZG_EINVAL, "max_rollouts too large for 16-bit child links");
     } else {
-        if (c.state_dim != 3) return fail(AZG_EINVAL, "continuous variant is Pendulum: state_dim must be 3");
+        if (!mcc && c.state_dim != 3) return fail(AZG_EINVAL, "continuous variant is Pendulum: state_dim must be 3");
         if (c.num_components < 1 || c.num_components > AZG_MAX_K) return fail(AZG_EINVAL, "num_components must be in 1..8");
         if (c.max_rollouts + 2 > 255) return fail(AZG_EINVAL, "continuous variant supports n_rollouts <= 253 (8-bit row links)");
     }
@@ -188,6 +193,7 @@ extern "C" int azg_create(const azg_config* cfg, azg_engine** out) {
     CK(cudaSetDevice(c.device));
     azg_engine* e = new azg_engine();
     e->cfg = c;
+    e->mcc = mcc;
     e->R = c.max_rollouts + 2;
     e->P = head_dim_of(c);
     e->PO_PAD = ((1 + e->P) + 3) / 4 * 4;
@@ -228,9 +234,9 @@ extern "C" int azg_create(const azg_config* cfg, azg_engine** out) {
         delete e;
         return fail(AZG_EINVAL, "AZG_FLAG_RNG_MT19937 with the continuous search runs one launch per simulation (no AZG_FLAG_FUSED)");
     }
-    if (e->fused && !(e->q8 && c.state_dim == (c.variant == AZG_CONTINUOUS ? 3 : 4))) {
+    if (e->fused && !(e->q8 && c.state_dim == (c.variant == AZG_CONTINUOUS ? (mcc ? 2 : 3) : 4))) {
         delete e;
-        return fail(AZG_EINVAL, "AZG_FLAG_FUSED needs AZG_FLAG_EVAL_Q8 and the shipped envs (state_dim 3 continuous / 4 discrete)");
+        return fail(AZG_EINVAL, "AZG_FLAG_FUSED needs AZG_FLAG_EVAL_Q8 and the shipped envs (state_dim 3 Pendulum / 2 MountainCarContinuous / 4 CartPole)");
     }
     const size_t B = c.max_trees, R = e->R;
     std::vector<int32_t> pwt;
@@ -555,40 +561,41 @@ static cudaError_t launch_mlp_t(const azg_engine* e, const MlpParams& m, cudaStr
     return launch_ex(e, k_mlp<H, S, ACT>, grid, MLP_THREADS(H), e->mlp_smem, st, m);
 }
 
-template <int S, int ACT, int NL>
+// ENV (env.cuh) selects the tree and env of the whole-search kernels; the evaluation-only launch reads ENV::S (layer 0) alone
+template <class ENV, int ACT, int NL>
 static cudaError_t launch_qmlp_t(const azg_engine* e, const MlpParams& m, cudaStream_t st, bool set_attr) {
     if (set_attr) {
-        cudaError_t ce = cudaFuncSetAttribute(k_qmlp2<S, ACT, NL, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)e->qmlp_smem);
+        cudaError_t ce = cudaFuncSetAttribute(k_qmlp2<ENV, ACT, NL, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)e->qmlp_smem);
         if (ce != cudaSuccess) return ce;
-        ce = cudaFuncSetAttribute(k_qmlp2<S, ACT, NL, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)e->qmlp_smem);
+        ce = cudaFuncSetAttribute(k_qmlp2<ENV, ACT, NL, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)e->qmlp_smem);
         if (ce != cudaSuccess) return ce;
-        if constexpr (S == 4) {  // trees in shared memory: everything the SM has beyond the kernel's static allocation
+        if constexpr (ENV::DISCRETE) {  // trees in shared memory: everything the SM has beyond the kernel's static allocation
             cudaFuncAttributes fa;
-            ce = cudaFuncGetAttributes(&fa, k_qmlp2<S, ACT, NL, true, true>);
+            ce = cudaFuncGetAttributes(&fa, k_qmlp2<ENV, ACT, NL, true, true>);
             if (ce != cudaSuccess) return ce;
             const_cast<azg_engine*>(e)->tsm_smem_max = e->smem_optin - std::min(e->smem_optin, fa.sharedSizeBytes);
-            ce = cudaFuncSetAttribute(k_qmlp2<S, ACT, NL, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)e->tsm_smem_max);
+            ce = cudaFuncSetAttribute(k_qmlp2<ENV, ACT, NL, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)e->tsm_smem_max);
             if (ce != cudaSuccess) return ce;
         }
         // search_wg.cuh raises its 16 tree + evaluation warps to 104 registers with setmaxnreg: the CTA's pool (640 threads x the
         // kernel's register count) must hold 512 x 104 + 128 x 56, or the instruction would wait forever
         cudaFuncAttributes fa;
-        ce = cudaFuncGetAttributes(&fa, k_search_wg<S, ACT, NL>);
+        ce = cudaFuncGetAttributes(&fa, k_search_wg<ENV, ACT, NL>);
         if (ce != cudaSuccess) return ce;
         if (fa.numRegs * WG_THREADS < WG_EPI_THREADS * WG_EPI_REGS + 128 * WG_MMA_REGS) return cudaErrorLaunchOutOfResources;
-        return cudaFuncSetAttribute(k_search_wg<S, ACT, NL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)e->wg_smem);
+        return cudaFuncSetAttribute(k_search_wg<ENV, ACT, NL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)e->wg_smem);
     }
     const int grid = std::max(1, std::min((m.n + 127) / 128, e->sm_count));
     TreeParams none;
     memset(&none, 0, sizeof none);
-    return launch_ex(e, k_qmlp2<S, ACT, NL, false>, grid, Q2_THREADS, e->qmlp_smem, st, m, none, 0, 0, 0);
+    return launch_ex(e, k_qmlp2<ENV, ACT, NL, false>, grid, Q2_THREADS, e->qmlp_smem, st, m, none, 0, 0, 0);
 }
 
 // whole-search kernel (AZG_FLAG_FUSED): one persistent launch per chunk of at most sm_count x Q2_MAX_TILES x 128 trees
-template <int S, int ACT, int NL>
+template <class ENV, int ACT, int NL>
 static cudaError_t launch_fused_t(const azg_engine* e, const MlpParams& m, const TreeParams& p, int N, cudaStream_t st, int* launches) {
     int chunk = e->sm_count * Q2_MAX_TILES * 128;
-    if constexpr (S == 4) {
+    if constexpr (ENV::DISCRETE) {
         // Discrete search: up to two full waves of shared-memory-resident trees (cap per SM x SMs each) beat the two-phase kernel on
         // rows in HBM, whose simulation takes 32 us whatever the batch (measured, profiles/README.md r2p: 8192 trees 248 M sims/s
         // there against 2 x 4096 at 337 M) -- so such a batch is cut into equal chunks, one launch each
@@ -610,7 +617,7 @@ static cudaError_t launch_fused_t(const azg_engine* e, const MlpParams& m, const
         // Discrete search, thin batch: when the rows of ceil(trees / SMs) trees fit in an SM's shared memory next to the evaluation's
         // operands, the CTA keeps its trees there for the whole search (tree_discrete.cuh ds_step; BASELINE config 3: 28 trees per SM)
         int tsm_per = 0;
-        if constexpr (S == 4) {
+        if constexpr (ENV::DISCRETE) {
             const int per = (hi - lo + e->sm_count - 1) / e->sm_count;
             if (two_phase && !p.rng_mt && !getenv("AZG_NO_TSM") && per <= 128 &&
                 qmlp2_tsm_smem_bytes(NL, e->qfl_count, per, p.R, e->PO_PAD) <= e->tsm_smem_max)
@@ -618,18 +625,18 @@ static cudaError_t launch_fused_t(const azg_engine* e, const MlpParams& m, const
         }
         const_cast<azg_engine*>(e)->last_fused_kind = tsm_per ? 3 : (two_phase ? 1 : 2);
         if (tsm_per) {
-            if constexpr (S == 4) {
+            if constexpr (ENV::DISCRETE) {
                 const int grid = (hi - lo + tsm_per - 1) / tsm_per;
-                ce = launch_ex(e, k_qmlp2<S, ACT, NL, true, true>, grid, Q2_THREADS, qmlp2_tsm_smem_bytes(NL, e->qfl_count, tsm_per, p.R, e->PO_PAD), st, m, p, N, lo, hi);
+                ce = launch_ex(e, k_qmlp2<ENV, ACT, NL, true, true>, grid, Q2_THREADS, qmlp2_tsm_smem_bytes(NL, e->qfl_count, tsm_per, p.R, e->PO_PAD), st, m, p, N, lo, hi);
             }
         } else if (two_phase) {
             const int grid = std::max(1, std::min((hi - lo + 127) / 128, e->sm_count));
-            ce = launch_ex(e, k_qmlp2<S, ACT, NL, true>, grid, Q2_THREADS, e->qmlp_smem, st, m, p, N, lo, hi);
+            ce = launch_ex(e, k_qmlp2<ENV, ACT, NL, true>, grid, Q2_THREADS, e->qmlp_smem, st, m, p, N, lo, hi);
         } else {
             // four warpgroups per CTA, each with its own tile: small batches are spread over every SM (a CTA's trees over its four
             // warpgroups), large ones use all SMs with up to WG_MAX_ROUNDS x 4 tiles each
             const int grid = std::max(1, std::min((hi - lo + 3) / 4, e->sm_count));
-            ce = launch_ex(e, k_search_wg<S, ACT, NL>, grid, WG_THREADS, e->wg_smem, st, m, p, N, lo, hi);
+            ce = launch_ex(e, k_search_wg<ENV, ACT, NL>, grid, WG_THREADS, e->wg_smem, st, m, p, N, lo, hi);
         }
         ++*launches;
         if (ce != cudaSuccess) return ce;
@@ -637,10 +644,22 @@ static cudaError_t launch_fused_t(const azg_engine* e, const MlpParams& m, const
     return cudaSuccess;
 }
 
+// The S of the CartPole / Pendulum tables below names the env (azg_create: state_dim 4 is CartPole, 3 Pendulum); MountainCarContinuous
+// has tables of its own, selected by its flag (their instantiations run in tests/test_mountain_car_gpu.py)
+template <int S>
+using ShippedEnv = std::conditional_t<S == 4, env::CartPole, env::Pendulum>;
+
 static cudaError_t launch_fused(const azg_engine* e, const MlpParams& m, const TreeParams& p, int N, cudaStream_t st, int* launches) {
     const int S = e->cfg.state_dim, A = e->cfg.activation, NL = e->cfg.n_hidden - 1;
+    if (e->mcc) {
+#define FUSED_MCC_CASE(a, nl) \
+    if (A == a && NL == nl) return launch_fused_t<env::MountainCarContinuous, a, nl>(e, m, p, N, st, launches);
+        FUSED_MCC_CASE(0, 1) FUSED_MCC_CASE(1, 1) FUSED_MCC_CASE(0, 2) FUSED_MCC_CASE(1, 2)
+#undef FUSED_MCC_CASE
+        return cudaErrorInvalidValue;
+    }
 #define FUSED_CASE(s, a, nl) \
-    if (S == s && A == a && NL == nl) return launch_fused_t<s, a, nl>(e, m, p, N, st, launches);
+    if (S == s && A == a && NL == nl) return launch_fused_t<ShippedEnv<s>, a, nl>(e, m, p, N, st, launches);
     FUSED_CASE(3, 0, 1) FUSED_CASE(3, 1, 1) FUSED_CASE(3, 0, 2) FUSED_CASE(3, 1, 2)
     FUSED_CASE(4, 0, 1) FUSED_CASE(4, 1, 1) FUSED_CASE(4, 0, 2) FUSED_CASE(4, 1, 2)
 #undef FUSED_CASE
@@ -651,11 +670,26 @@ static cudaError_t launch_mlp(const azg_engine* e, const MlpParams& m, cudaStrea
     const int H = e->cfg.hidden, S = e->cfg.state_dim, A = e->cfg.activation;
     if (e->q8) {
         const int NL = e->cfg.n_hidden - 1;
+        if (e->mcc) {
+#define QMLP_MCC_CASE(a, nl) \
+    if (A == a && NL == nl) return launch_qmlp_t<env::MountainCarContinuous, a, nl>(e, m, st, set_attr);
+            QMLP_MCC_CASE(0, 1) QMLP_MCC_CASE(1, 1) QMLP_MCC_CASE(0, 2) QMLP_MCC_CASE(1, 2)
+#undef QMLP_MCC_CASE
+            return cudaErrorInvalidValue;
+        }
 #define QMLP_CASE(s, a, nl) \
-    if (S == s && A == a && NL == nl) return launch_qmlp_t<s, a, nl>(e, m, st, set_attr);
+    if (S == s && A == a && NL == nl) return launch_qmlp_t<ShippedEnv<s>, a, nl>(e, m, st, set_attr);
         QMLP_CASE(4, 0, 1) QMLP_CASE(4, 1, 1) QMLP_CASE(3, 0, 1) QMLP_CASE(3, 1, 1)
         QMLP_CASE(4, 0, 2) QMLP_CASE(4, 1, 2) QMLP_CASE(3, 0, 2) QMLP_CASE(3, 1, 2)
 #undef QMLP_CASE
+        return cudaErrorInvalidValue;
+    }
+    if (e->mcc) {  // layer 0 with two inputs
+#define MLP_MCC_CASE(h, a) \
+    if (H == h && A == a) return launch_mlp_t<h, 2, a>(e, m, st, set_attr);
+        MLP_MCC_CASE(128, 0) MLP_MCC_CASE(128, 1) MLP_MCC_CASE(128, 2) MLP_MCC_CASE(128, 3) MLP_MCC_CASE(128, 4) MLP_MCC_CASE(128, 5)
+        MLP_MCC_CASE(64, 0) MLP_MCC_CASE(64, 1) MLP_MCC_CASE(64, 2) MLP_MCC_CASE(64, 3) MLP_MCC_CASE(64, 4) MLP_MCC_CASE(64, 5)
+#undef MLP_MCC_CASE
         return cudaErrorInvalidValue;
     }
 #define MLP_CASE(h, s, a) \
@@ -672,7 +706,8 @@ static cudaError_t launch_mlp(const azg_engine* e, const MlpParams& m, cudaStrea
 
 template <bool BK, bool SEL>
 static cudaError_t launch_step_continuous(const azg_engine* e, const TreeParams& p, cudaStream_t st) {
-    return launch_ex(e, k_step_continuous<BK, SEL>, (p.B + 127) / 128, 128, 0, st, p);
+    if (e->mcc) return launch_ex(e, k_step_continuous<env::MountainCarContinuous, BK, SEL>, (p.B + 127) / 128, 128, 0, st, p);
+    return launch_ex(e, k_step_continuous<env::Pendulum, BK, SEL>, (p.B + 127) / 128, 128, 0, st, p);
 }
 
 // per-launch CUDA-event timing used by azg_profile_search (classes: 0 tree step, 1 evaluation, 2 setup)
@@ -726,7 +761,8 @@ static int enqueue_search(azg_engine* e, int B, int N, int64_t tree_id0, cudaStr
         }
         LK(0, (k_step_discrete<true, false><<<tg, tb, 0, st>>>(p)));
     } else {
-        LK(2, (k_init_continuous<<<tg, tb, 0, st>>>(p)));
+        if (e->mcc) LK(2, (k_init_continuous<env::MountainCarContinuous><<<tg, tb, 0, st>>>(p)));
+        else LK(2, (k_init_continuous<env::Pendulum><<<tg, tb, 0, st>>>(p)));
         if (!tape) LK(1, ce = launch_mlp(e, m, st, false));
         LK(2, (k_root_insert_continuous<<<tg, tb, 0, st>>>(p)));
         for (int it = 0; it < N; ++it) {
@@ -1157,7 +1193,8 @@ extern "C" int azg_selfplay_step(azg_engine* e, int32_t B, const azg_selfplay_io
     sp.drows = e->drows; sp.R = e->R;
     const int tb = 128, tg = (B + tb - 1) / tb;
     if (disc) k_selfplay_discrete<<<tg, tb, 0, st>>>(sp);
-    else k_selfplay_continuous<<<tg, tb, 0, st>>>(sp);
+    else if (e->mcc) k_selfplay_continuous<env::MountainCarContinuous><<<tg, tb, 0, st>>>(sp);
+    else k_selfplay_continuous<env::Pendulum><<<tg, tb, 0, st>>>(sp);
     CK(cudaGetLastError());
     return AZG_OK;
 }
@@ -1267,7 +1304,19 @@ extern "C" int azg_mlp_forward(azg_engine* e, int32_t n, const float* d_x, float
     return AZG_OK;
 }
 
-__global__ void k_env_step(int variant, int n, const double* s, const float* a, double* o, double* rew, int32_t* term, float* obs) {
+template <class ENV>
+__device__ __forceinline__ void env_step_continuous(int i, const double* s, const float* a, double* o, double* rew, int32_t* term, float* obs) {
+    double n0, n1, r;
+    const bool t = ENV::step(s[i * 2], s[i * 2 + 1], a[i], n0, n1, r);
+    o[i * 2] = n0; o[i * 2 + 1] = n1;
+    const float4 ob = ENV::obs(n0, n1);
+    obs[i * ENV::S] = ob.x; obs[i * ENV::S + 1] = ob.y;
+    if (ENV::S > 2) obs[i * ENV::S + 2] = ob.z;
+    rew[i] = r;
+    term[i] = t;
+}
+
+__global__ void k_env_step(int variant, bool mcc, int n, const double* s, const float* a, double* o, double* rew, int32_t* term, float* obs) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     if (variant == AZG_DISCRETE) {
@@ -1277,14 +1326,10 @@ __global__ void k_env_step(int variant, int n, const double* s, const float* a, 
         for (int k = 0; k < 4; ++k) { o[i * 4 + k] = out[k]; obs[i * 4 + k] = (float)out[k]; }
         rew[i] = r;
         term[i] = t;
+    } else if (mcc) {
+        env_step_continuous<env::MountainCarContinuous>(i, s, a, o, rew, term, obs);
     } else {
-        double nth, nthdot, r;
-        const bool t = env::pendulum_step(s[i * 2], s[i * 2 + 1], a[i], nth, nthdot, r);
-        o[i * 2] = nth; o[i * 2 + 1] = nthdot;
-        const float4 ob = env::pendulum_obs(nth, nthdot);
-        obs[i * 3] = ob.x; obs[i * 3 + 1] = ob.y; obs[i * 3 + 2] = ob.z;
-        rew[i] = r;
-        term[i] = t;
+        env_step_continuous<env::Pendulum>(i, s, a, o, rew, term, obs);
     }
 }
 
@@ -1293,7 +1338,7 @@ extern "C" int azg_env_step(azg_engine* e, int32_t n, const double* d_state, con
     if (!e || !d_state || !d_action || !d_next || !d_reward || !d_terminal || !d_obs) return fail(AZG_EINVAL, "null argument");
     if (n < 1) return fail(AZG_EINVAL, "n must be >= 1");
     CK(cudaSetDevice(e->cfg.device));
-    k_env_step<<<(n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(e->cfg.variant, n, d_state, d_action, d_next, d_reward, d_terminal, d_obs);
+    k_env_step<<<(n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(e->cfg.variant, e->mcc, n, d_state, d_action, d_next, d_reward, d_terminal, d_obs);
     CK(cudaGetLastError());
     return AZG_OK;
 }

@@ -1,4 +1,4 @@
-// env.cuh -- CartPole-v0 / Pendulum-v0 transition functions (gym 0.17.2 / 0.19.0 classic_control,
+// env.cuh -- CartPole-v0 / Pendulum-v0 / MountainCarContinuous-v0 transition functions (gym 0.17.2 / 0.19.0 classic_control,
 // third-party to the reference; reached through rl/make_game.py:59-62 and stepped by the search at
 // alphazero/search/mcts.py:449 and :686).  Replaces `copy.deepcopy(Env)` + replay from the root
 // (mcts.py:443, :680): the hidden state is kept per node and stepped once at expansion.
@@ -62,5 +62,61 @@ __device__ __forceinline__ float4 pendulum_obs(double th, double thdot) {
     det::sincos_(th, s, c);
     return make_float4((float)c, (float)s, (float)thdot, 0.0f);
 }
+
+// MountainCarContinuous-v0 (gym 0.17-0.19 classic_control/continuous_mountain_car.py); returns done.  The f32 action enters f64
+// arithmetic exactly (numpy-1.x promotion, as for Pendulum); the clips are Python's max / min (a NaN passes, -0 stays -0); the
+// reward uses the unclipped action, and 0 - x with the int 0 is 0.0 - x (+0 for a zero action).
+__device__ __forceinline__ bool mountain_car_step(double pos, double vel, float action, double& newpos, double& newvel, double& reward) {
+    const double min_position = -1.2, max_position = 0.6, max_speed = 0.07, goal_position = 0.45, power = 0.0015;
+    const double a = (double)action;
+    double force = -1.0 > a ? -1.0 : a;  // min(max(action[0], min_action), max_action)
+    force = 1.0 < force ? 1.0 : force;
+    vel = vel + (force * power - 0.0025 * det::cos_(3 * pos));
+    if (vel > max_speed) vel = max_speed;
+    if (vel < -max_speed) vel = -max_speed;
+    pos = pos + vel;
+    if (pos > max_position) pos = max_position;
+    if (pos < min_position) pos = min_position;
+    if (pos == min_position && vel < 0) vel = 0.0;
+    const bool done = pos >= goal_position && vel >= 0.0;
+    reward = (done ? 100.0 : 0.0) - (a * a) * 0.1;  // math.pow(action[0], 2) of an f32 is exact in f64
+    newpos = pos;
+    newvel = vel;
+    return done;
+}
+
+// The env of a continuous search as a compile-time type: the hidden state is two doubles (CRow sector 1), the network input the
+// first S lanes of a float4.  CartPole names the discrete tree in the kernels that serve both variants.
+struct CartPole {
+    static constexpr int S = 4;
+    static constexpr bool DISCRETE = true;
+};
+struct Pendulum {
+    static constexpr int S = 3;
+    static constexpr bool DISCRETE = false;
+    static __device__ __forceinline__ bool step(double th, double thdot, float a, double& nth, double& nthdot, double& r) {
+        return pendulum_step(th, thdot, a, nth, nthdot, r);
+    }
+    static __device__ __forceinline__ float4 obs(double th, double thdot) { return pendulum_obs(th, thdot); }
+    // Env.reset from the uniforms u0, u1: th ~ U(-pi, pi), thdot ~ U(-1, 1)
+    static __device__ __forceinline__ void reset(double u0, double u1, double& th, double& thdot) {
+        const double pi = 3.141592653589793;
+        th = -pi + (pi - -pi) * u0;
+        thdot = -1.0 + (1.0 - -1.0) * u1;
+    }
+};
+struct MountainCarContinuous {
+    static constexpr int S = 2;
+    static constexpr bool DISCRETE = false;
+    static __device__ __forceinline__ bool step(double pos, double vel, float a, double& npos, double& nvel, double& r) {
+        return mountain_car_step(pos, vel, a, npos, nvel, r);
+    }
+    static __device__ __forceinline__ float4 obs(double pos, double vel) { return make_float4((float)pos, (float)vel, 0.0f, 0.0f); }
+    // Env.reset: position ~ U(-0.6, -0.4), velocity +0
+    static __device__ __forceinline__ void reset(double u0, double, double& pos, double& vel) {
+        pos = -0.6 + (-0.4 - -0.6) * u0;
+        vel = 0.0;
+    }
+};
 
 }  // namespace env

@@ -368,7 +368,8 @@ __device__ __forceinline__ void mlp_unit(const MlpParams& p, const float* w, flo
         if (need) {
             if (p.xstride == 4) {
                 const float4 v = *reinterpret_cast<const float4*>(p.X + (size_t)gr * 4);
-                x[0] = v.x; x[1] = v.y; x[2] = v.z;
+                x[0] = v.x; x[1] = v.y;
+                if constexpr (S > 2) x[2] = v.z;
                 if (S > 3) x[S - 1] = v.w;
             } else {
 #pragma unroll

@@ -169,7 +169,8 @@ __device__ __forceinline__ float q2_layer0(const Q2Ctx& c, const MlpParams& p, i
         if (valid) {
             if (p.xstride == 4) {
                 const float4 v = *reinterpret_cast<const float4*>(p.X + (size_t)gr * 4);
-                x[0] = v.x; x[1] = v.y; x[2] = v.z;
+                x[0] = v.x; x[1] = v.y;
+                if constexpr (S > 2) x[2] = v.z;
                 if (S > 3) x[S - 1] = v.w;
             } else {
 #pragma unroll
@@ -327,7 +328,8 @@ __device__ __forceinline__ void q2_eval_rep(const Q2Ctx& c, const MlpParams& p, 
         for (int s = 0; s < S; ++s) x[s] = 0.0f;
         if (r < nv) {
             const float4 v = *reinterpret_cast<const float4*>(p.X + (size_t)(row0 + r) * 4);  // xstride 4 in the whole-search kernel
-            x[0] = v.x; x[1] = v.y; x[2] = v.z;
+            x[0] = v.x; x[1] = v.y;
+            if constexpr (S > 2) x[2] = v.z;
             if (S > 3) x[S - 1] = v.w;
         }
 #pragma unroll
@@ -412,10 +414,13 @@ __device__ __forceinline__ void q2_eval_rep(const Q2Ctx& c, const MlpParams& p, 
 //   an SM with two dedicated tree warpgroups; at 48 registers per tree thread and with both code paths fighting for the
 //   instruction cache it reached 80 us per simulation against 74 us for separate launches.
 // TSM (FUSED, discrete tree, thin batches): the CTA's trees live in shared memory for the whole search (tree_discrete.cuh ds_step).
-template <int S, int ACT, int NL, bool FUSED, bool TSM = false>
+// ENV (env.cuh): CartPole = the discrete tree, Pendulum | MountainCarContinuous = the continuous tree stepping that env; its S is the
+// width of layer 0.
+template <class ENV, int ACT, int NL, bool FUSED, bool TSM = false>
 __global__ void __launch_bounds__(Q2_THREADS, 1)
 k_qmlp2(const MlpParams p_in, const TreeParams tp, const int n_sims, const int chunk_begin, const int chunk_end) {
-    static_assert(!TSM || (FUSED && S == 4), "trees in shared memory: whole-search kernel of the discrete tree");
+    constexpr int S = ENV::S;
+    static_assert(!TSM || (FUSED && ENV::DISCRETE), "trees in shared memory: whole-search kernel of the discrete tree");
     extern __shared__ __align__(1024) uint8_t qsm_raw[];
     __shared__ __align__(8) uint64_t wbar, full[2], ready[2], freeb[2], hfull[2], hfree[2], phase_bar;
     __shared__ uint32_t tmem_base_s;
@@ -636,8 +641,8 @@ k_qmlp2(const MlpParams p_in, const TreeParams tp, const int n_sims, const int c
         if (FUSED) {  // MCTSContinuous.initialize_search for every tree of the CTA
             for (int i = tid; i < nrows; i += Q2_EPI_THREADS) {
                 if (TSM) ds_init(tp, smt, i, row_begin + i);
-                else if (S == 4) d_init(tp, row_begin + i);  // state_dim 4 = CartPole = the discrete tree (engine.cu checks it)
-                else c_init(tp, row_begin + i);
+                else if constexpr (ENV::DISCRETE) d_init(tp, row_begin + i);
+                else c_init<ENV>(tp, row_begin + i);
             }
             phase_sync(&phase_bar, pph);
         }
@@ -761,11 +766,11 @@ k_qmlp2(const MlpParams p_in, const TreeParams tp, const int n_sims, const int c
 #pragma unroll 1
             for (int i = tid; i < nrows; i += Q2_EPI_THREADS) {
                 const int gr = row_begin + i;
-                if (S == 4) {
+                if constexpr (ENV::DISCRETE) {
                     d_step(tp, tabs, gr, s > 0, s + 1 < n_evals);
                 } else {
                     if (s == 0) c_root_insert(tp, gr);                // the add_pw_action(root) before the loop (mcts.py:673)
-                    c_step(tp, tabs, gr, s > 0, s + 1 < n_evals);     // backup of simulation s, descent + expansion of simulation s + 1
+                    c_step<ENV>(tp, tabs, gr, s > 0, s + 1 < n_evals);  // backup of simulation s, descent + expansion of simulation s + 1
                 }
             }
             phase_sync(&phase_bar, pph);

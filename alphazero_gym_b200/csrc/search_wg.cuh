@@ -131,7 +131,8 @@ __device__ __forceinline__ void wg_evaluate(const MlpParams& p, WgSlot& sl, cons
         for (int s = 0; s < S; ++s) x[s] = 0.0f;
         if (valid) {
             const float4 v = *reinterpret_cast<const float4*>(p.X + (size_t)gr * 4);
-            x[0] = v.x; x[1] = v.y; x[2] = v.z;
+            x[0] = v.x; x[1] = v.y;
+            if constexpr (S > 2) x[2] = v.z;
             if (S > 3) x[S - 1] = v.w;
         }
 #pragma unroll 1
@@ -236,9 +237,11 @@ __device__ __forceinline__ void wg_evaluate(const MlpParams& p, WgSlot& sl, cons
     tc_fence_before();
 }
 
-template <int S, int ACT, int NL>
+// ENV (env.cuh): CartPole = the discrete tree, Pendulum | MountainCarContinuous = the continuous tree stepping that env
+template <class ENV, int ACT, int NL>
 __global__ void __launch_bounds__(WG_THREADS, 1)
 k_search_wg(const MlpParams p, const TreeParams tp, const int n_sims, const int chunk_begin, const int chunk_end) {
+    constexpr int S = ENV::S;
     extern __shared__ __align__(1024) uint8_t wsm_raw[];
     __shared__ __align__(8) uint64_t wbar, ready[2], full[2][2], accfree[2][2], slotfree[2][2];
     __shared__ uint32_t tmem_base_s;
@@ -372,8 +375,8 @@ k_search_wg(const MlpParams p, const TreeParams tp, const int n_sims, const int 
         for (int rd = 0; rd < rounds; ++rd) {
             const int tile = 4 * rd + g, row0 = row_begin + tile * th;
             if (tile < ntiles && row0 + r < min(row0 + th, row_end)) {
-                if (S == 4) d_init(tp, row0 + r);  // state_dim 4 = CartPole = the discrete tree (engine.cu checks it)
-                else c_init(tp, row0 + r);
+                if constexpr (ENV::DISCRETE) d_init(tp, row0 + r);
+                else c_init<ENV>(tp, row0 + r);
             }
         }
 #pragma unroll 1
@@ -420,11 +423,11 @@ k_search_wg(const MlpParams p, const TreeParams tp, const int n_sims, const int 
                     ++nev;
                     ev_row = gr;
                 }
-                if (S == 4) {
+                if constexpr (ENV::DISCRETE) {
                     d_step(tp, tabs, gr, s > 0, s + 1 < n_evals);
                 } else {
                     if (s == 0) c_root_insert(tp, gr);             // the add_pw_action(root) before the loop (mcts.py:673)
-                    c_step(tp, tabs, gr, s > 0, s + 1 < n_evals);  // backup of simulation s, descent + expansion of simulation s + 1
+                    c_step<ENV>(tp, tabs, gr, s > 0, s + 1 < n_evals);  // backup of simulation s, descent + expansion of simulation s + 1
                 }
             }
             cyc_slot += c1 - c0;

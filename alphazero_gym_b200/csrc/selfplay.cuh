@@ -11,7 +11,8 @@
 //        discrete:   agent.mcts_forward(action, state)         run_discrete.py:122 -> mcts.py:495-526; evaluation(root) re-creates
 //                                                              the root's edges, so only root.n survives (SURVEY 7-7)
 // Randomness: the engine is re-keyed for every step (azg_selfplay_step); stream 2 = the discrete agent's action draw,
-// stream 3 = Env.reset (gym: CartPole U(-0.05, 0.05)^4, Pendulum th ~ U(-pi, pi), thdot ~ U(-1, 1)).
+// stream 3 = Env.reset (gym: CartPole U(-0.05, 0.05)^4, Pendulum th ~ U(-pi, pi), thdot ~ U(-1, 1), MountainCarContinuous
+// position ~ U(-0.6, -0.4), velocity 0).
 #pragma once
 #include "common.cuh"
 #include "env.cuh"
@@ -32,7 +33,7 @@ struct SelfPlayParams {
     const double* Q;
     const int32_t* n_children;
     // outputs
-    float* obs;          // [B][S] observation the search started from
+    float* obs;          // [B][S] observation the search started from (S = 4 | 3 | 2)
     float* action_taken; // [B]
     double* reward;      // [B]
     int32_t* done;       // [B]
@@ -43,6 +44,7 @@ struct SelfPlayParams {
 
 __device__ __forceinline__ double u32_to_unit_f64(uint32_t x) { return ((double)x + 0.5) * 2.3283064365386963e-10; }
 
+template <class ENV>
 __global__ void k_selfplay_continuous(const SelfPlayParams p) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= p.B) return;
@@ -58,18 +60,17 @@ __global__ void k_selfplay_continuous(const SelfPlayParams p) {
     }
     const float a = act[best];
     const double th = p.env_state[(size_t)t * 2], thdot = p.env_state[(size_t)t * 2 + 1];
-    const float4 ob = env::pendulum_obs(th, thdot);
-    p.obs[(size_t)t * 3] = ob.x; p.obs[(size_t)t * 3 + 1] = ob.y; p.obs[(size_t)t * 3 + 2] = ob.z;
+    const float4 ob = ENV::obs(th, thdot);
+    p.obs[(size_t)t * ENV::S] = ob.x; p.obs[(size_t)t * ENV::S + 1] = ob.y;
+    if (ENV::S > 2) p.obs[(size_t)t * ENV::S + 2] = ob.z;
     double nth, nthdot, rew;
-    const bool term = env::pendulum_step(th, thdot, a, nth, nthdot, rew);
+    const bool term = ENV::step(th, thdot, a, nth, nthdot, rew);
     const int step = p.ep_step[t] + 1;
     const bool done = term || step >= p.max_episode_length;
     if (done) {  // Env.reset()
         const int ep = p.episode[t] + 1;
         const u32x4 r = rng_block(__ldg(p.seedp), p.tree_id0 + t, 3, ep, 0);
-        const double pi = 3.141592653589793;
-        nth = -pi + (pi - -pi) * u32_to_unit_f64(r.x);
-        nthdot = -1.0 + (1.0 - -1.0) * u32_to_unit_f64(r.y);
+        ENV::reset(u32_to_unit_f64(r.x), u32_to_unit_f64(r.y), nth, nthdot);
         p.episode[t] = ep;
     }
     p.ep_step[t] = done ? 0 : step;

@@ -228,13 +228,15 @@ __device__ __forceinline__ CHot fresh_hot(double r, float V, float action, uint3
     return h;
 }
 
-// MCTSContinuous.initialize_search (mcts.py:589-600): new root row, network input = obs(root)
+// MCTSContinuous.initialize_search (mcts.py:589-600): new root row, network input = obs(root).  ENV: env.cuh Pendulum |
+// MountainCarContinuous (the root is never terminal, even at the goal)
+template <class ENV>
 __device__ __forceinline__ void c_init(const TreeParams& p, int t) {
     const double th = p.root_state[(size_t)t * 2], thdot = p.root_state[(size_t)t * 2 + 1];
     CRow* root = p.crows + (size_t)t * p.R;
     store_hot(root, fresh_hot(0.0, p.use_tape ? p.tapeV[(size_t)t * p.R] : 0.0f, 0.0f, CROW_EXPANDED));
     store_sec1_new(root, th, thdot);
-    p.X[t] = env::pendulum_obs(th, thdot);
+    p.X[t] = ENV::obs(th, thdot);
     CCtl c;
     memset(&c, 0, sizeof c);
     c.n_rows = 1;
@@ -247,9 +249,10 @@ __device__ __forceinline__ void c_init(const TreeParams& p, int t) {
         tmt_seed_dev(p.tmt + (size_t)t * TMT_WORDS, s);
     }
 }
+template <class ENV>
 __global__ void k_init_continuous(const TreeParams p) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t < p.B) c_init(p, t);
+    if (t < p.B) c_init<ENV>(p, t);
 }
 
 // the add_pw_action(root) that precedes the rollout loop (mcts.py:673); runs after the root evaluation
@@ -343,7 +346,7 @@ __device__ __forceinline__ int uct_select(const TreeParams& p, const Tabs& tb, i
 // Shared by k_step_continuous (one launch per simulation) and the whole-search kernel k_search_fused (fused.cuh).
 // MT: AZG_FLAG_RNG_MT19937 (CPython's and torch's generators, 5 KB of state per tree in HBM: a compatibility mode that the one-launch-
 // per-simulation kernel alone instantiates; the whole-search kernels are built without it)
-template <bool MT = false>
+template <class ENV, bool MT = false>
 __device__ __forceinline__ void c_step(const TreeParams& p, const Tabs& tb, int t, const bool BACKUP, const bool SELECT) {
     CRow* rows = p.crows + (size_t)t * p.R;
     CHot* et = p.et + t;  // root child j: et[j * BS]
@@ -441,8 +444,8 @@ __device__ __forceinline__ void c_step(const TreeParams& p, const Tabs& tb, int 
                 cur_th = s0.th; cur_thdot = s0.thdot;
             }
             double nth, nthdot, rew;
-            const bool term = env::pendulum_step(cur_th, cur_thdot, sel_action, nth, nthdot, rew);
-            const double r = rew / AZG_PENDULUM_R_SCALE;  // mcts.py:687
+            const bool term = ENV::step(cur_th, cur_thdot, sel_action, nth, nthdot, rew);
+            const double r = rew / AZG_PENDULUM_R_SCALE;  // mcts.py:687: Pendulum's scale, whatever the env
             const uint32_t fl = CROW_EXPANDED | (term ? CROW_TERMINAL : 0u);
             float V = 0.0f;
             if (p.use_tape && !term) V = p.tapeV[(size_t)t * p.R + sel];
@@ -454,7 +457,7 @@ __device__ __forceinline__ void c_step(const TreeParams& p, const Tabs& tb, int 
                 h->r = r; h->V = V; h->nn_flags = fl;
             }
             store_sec1_new(rows + sel, nth, nthdot);
-            p.X[t] = env::pendulum_obs(nth, nthdot);
+            p.X[t] = ENV::obs(nth, nthdot);
             c.leaf = sel | LEAF_EVAL | (term ? LEAF_TERMINAL : 0) | (parent_is_root ? (LEAF_ROOTCHILD | (jsel << LEAF_J_SHIFT)) : 0);
             // first backup step R = r + gamma*V: with tapes V is known here, otherwise the evaluation kernel adds it
             c.leafR = p.use_tape ? r + (double)__fmul_rn(p.gamma_f32, V) : r;
@@ -478,13 +481,13 @@ __device__ __forceinline__ void c_step(const TreeParams& p, const Tabs& tb, int 
     store_ctl(p.ctl, p.BS, t, c);
     TP_STAMP(4);
 }
-template <bool BACKUP, bool SELECT>
+template <class ENV, bool BACKUP, bool SELECT>
 __global__ void __launch_bounds__(128) k_step_continuous(const TreeParams p) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     const Tabs tb = {p.pw_table, p.rcp_tab, p.sqrt_tab, AZG_TAB};
     if (t >= p.B) return;
-    if (p.rng_mt) c_step<true>(p, tb, t, BACKUP, SELECT);
-    else c_step<false>(p, tb, t, BACKUP, SELECT);
+    if (p.rng_mt) c_step<ENV, true>(p, tb, t, BACKUP, SELECT);
+    else c_step<ENV, false>(p, tb, t, BACKUP, SELECT);
 }
 
 // numpy pairwise summation for n <= 128 (np.sum in get_on_policy_value_target, mcts.py:111)

@@ -15,6 +15,9 @@ import torch
 from . import _cabi
 from ._cabi import ACT_ELU, ACT_RELU, CONTINUOUS, DISCRETE, VT, AzgConfig, check
 
+# the envs the engine steps (gym ids); the continuous search steps Pendulum-v0 unless told otherwise
+CARTPOLE, PENDULUM, MOUNTAIN_CAR_CONTINUOUS = "CartPole-v0", "Pendulum-v0", "MountainCarContinuous-v0"
+
 
 @dataclass
 class EngineConfig:
@@ -48,6 +51,9 @@ class EngineConfig:
     eval_q8: Optional[bool] = None
     rng_mt19937: bool = False  # AZG_FLAG_RNG_MT19937: CPython's generator for the discrete search's selection draws (include/azg.h)
     fused: Optional[bool] = None  # AZG_FLAG_FUSED: whole search in one persistent kernel; None = on where supported (eval_q8)
+    # the env the search steps: None = the variant's own (CartPole-v0 / Pendulum-v0); MOUNTAIN_CAR_CONTINUOUS (continuous variant,
+    # state_dim 2) sets AZG_FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS
+    env: Optional[str] = None
 
     def c(self) -> AzgConfig:
         return AzgConfig(self.variant, self.max_rollouts, self.max_trees, self.num_actions, self.num_components,
@@ -55,7 +61,15 @@ class EngineConfig:
                          self.puct_f32, self.device, self.c_uct, float(self.gamma), self.epsilon, self.c_pw, self.kappa,
                          self.action_bound, self.log_std_min, self.log_std_max,
                          (0 if self.use_graph else _cabi.FLAG_NO_GRAPH) | (_cabi.FLAG_EVAL_Q8 if self.is_q8() else 0)
-                         | (_cabi.FLAG_FUSED if self.is_fused() else 0) | (_cabi.FLAG_RNG_MT19937 if self.rng_mt19937 else 0), self.seed)
+                         | (_cabi.FLAG_FUSED if self.is_fused() else 0) | (_cabi.FLAG_RNG_MT19937 if self.rng_mt19937 else 0)
+                         | (_cabi.FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS if self.env_name() == MOUNTAIN_CAR_CONTINUOUS else 0), self.seed)
+
+    def env_name(self) -> str:
+        if self.env is None:
+            return CARTPOLE if self.variant == DISCRETE else PENDULUM
+        if self.env not in (CARTPOLE, PENDULUM, MOUNTAIN_CAR_CONTINUOUS):
+            raise ValueError(f"unknown env {self.env!r}: the engine steps {CARTPOLE}, {PENDULUM} and {MOUNTAIN_CAR_CONTINUOUS}")
+        return self.env
 
     def q8_supported(self) -> bool:
         head = self.num_actions if self.variant == DISCRETE else (3 * self.num_components if self.num_components > 1 else 2)
@@ -65,7 +79,8 @@ class EngineConfig:
         return self.q8_supported() if self.eval_q8 is None else bool(self.eval_q8)
 
     def is_fused(self) -> bool:
-        supported = (self.is_q8() and self.state_dim == (3 if self.variant == CONTINUOUS else 4)
+        env_dim = {CARTPOLE: 4, PENDULUM: 3, MOUNTAIN_CAR_CONTINUOUS: 2}[self.env_name()]
+        supported = (self.is_q8() and self.state_dim == env_dim
                      and not (self.rng_mt19937 and self.variant == CONTINUOUS))  # the torch-generator mode runs one launch per simulation
         return supported if self.fused is None else bool(self.fused)
 

@@ -7,8 +7,8 @@ upstream call form `search(n_mcts, c, Env, mcts_env)` named in BASELINE.json is 
 
 What changes underneath: the tree lives in HBM tables and the whole search -- select, env step, network
 evaluation, backup -- runs in the CUDA engine (csrc/, C ABI include/azg.h).  `model` is only read for its
-weights and shape; `Env` only for its hidden state (`Env.unwrapped.state`).  Envs other than CartPole /
-Pendulum raise: there is no CPU fallback.  Tie-break / epsilon-greedy / action-noise randomness comes from
+weights and shape; `Env` only for its hidden state (`Env.unwrapped.state`) and its class name.  Envs other than
+CartPole (MCTSDiscrete), Pendulum and MountainCarContinuous (MCTSContinuous) raise: there is no CPU fallback.  Tie-break / epsilon-greedy / action-noise randomness comes from
 the engine's counter-based Philox streams keyed by (`seed`, search counter) instead of Python's `random` and
 torch's global generator.
 
@@ -22,7 +22,7 @@ from typing import Any, Dict, Optional, Tuple
 import numpy as np
 
 from .._cabi import CONTINUOUS, DISCRETE
-from ..engine import EngineConfig, SearchEngine, flatten_state_dict
+from ..engine import MOUNTAIN_CAR_CONTINUOUS, PENDULUM, EngineConfig, SearchEngine, flatten_state_dict
 from ..network import describe_model, weights_version
 
 PENDULUM_R_SCALE = 16.2736044  # reference mcts.py:20 (applied inside the engine)
@@ -61,7 +61,9 @@ def _unwrap(env):
 def reward_model(env, variant: int):
     """(reward_step, reward_terminal) of the env's reward wrappers, innermost applied first, each with the wrapper's own Python
     expression (rl/wrappers.py:58-105) so that the constants are the reference's bit for bit."""
-    _, names = _wrapper_chain(env)
+    base, names = _wrapper_chain(env)
+    if names and variant != DISCRETE and _is_mountain_car_continuous(base):
+        raise NotImplementedError(f"{names[0]} around MountainCarContinuous-v0: the CUDA engine steps the plain env only")
     step, terminal = 1.0, 1.0  # gym CartPole-v0 pays 1.0 for every step, the terminating one included
     for name in reversed(names):
         if name == "ReparametrizeWrapper":
@@ -75,17 +77,30 @@ def reward_model(env, variant: int):
     return float(step), float(terminal)
 
 
+def _is_mountain_car_continuous(base) -> bool:
+    return type(base).__name__ == "Continuous_MountainCarEnv"  # gym's class (classic_control/continuous_mountain_car.py)
+
+
+def continuous_env(env) -> str:
+    """The env MCTSContinuous has the engine step for `env`: MountainCarContinuous-v0 for gym's Continuous_MountainCarEnv (by class
+    name, under any wrappers), Pendulum-v0 otherwise (env_hidden_state refuses the envs that are neither)."""
+    return MOUNTAIN_CAR_CONTINUOUS if _is_mountain_car_continuous(_unwrap(env)) else PENDULUM
+
+
 def env_hidden_state(env, variant: int) -> np.ndarray:
     """Root of the search = hidden state of the gym env (replaces copy.deepcopy(Env), mcts.py:443, :680)."""
     base = _unwrap(env)
     if not hasattr(base, "state") or base.state is None:
-        raise TypeError("Env has no hidden `.state`; only gym CartPole-v0 / Pendulum-v0 style envs are supported")
+        raise TypeError("Env has no hidden `.state`; only gym CartPole-v0 / Pendulum-v0 / MountainCarContinuous-v0 style envs are supported")
     s = np.asarray(base.state, dtype=np.float64).reshape(-1)
     name = type(base).__name__.lower()
     want = 4 if variant == DISCRETE else 2
-    if s.size != want or ("cartpole" in name and variant != DISCRETE) or ("pendulum" in name and variant != CONTINUOUS):
+    mcc = _is_mountain_car_continuous(base)
+    if (s.size != want or ("cartpole" in name and variant != DISCRETE) or ("pendulum" in name and variant != CONTINUOUS)
+            or ("mountaincar" in name and not (mcc and variant == CONTINUOUS))):
         raise TypeError(f"unsupported environment {type(base).__name__} for this search class: the CUDA engine implements "
-                        "CartPole-v0 (MCTSDiscrete) and Pendulum-v0 (MCTSContinuous) dynamics and has no CPU fallback")
+                        "CartPole-v0 (MCTSDiscrete), Pendulum-v0 and MountainCarContinuous-v0 (MCTSContinuous) dynamics and has no "
+                        "CPU fallback")
     return s
 
 
@@ -246,7 +261,9 @@ class MCTSDiscrete(MCTS):
 
 
 class MCTSContinuous(MCTS):
-    """A0C search with progressive widening for Pendulum-v0 (reference mcts.py:529-741)."""
+    """A0C search with progressive widening for Pendulum-v0 and MountainCarContinuous-v0 (reference mcts.py:529-741).  The env
+    is taken from the Env each search() is handed (continuous_env); search_batch steps the env of the last search(), or the
+    engine keyword `env` (engine.PENDULUM by default)."""
 
     variant = CONTINUOUS
 
@@ -256,6 +273,7 @@ class MCTSContinuous(MCTS):
                          V_target_policy=V_target_policy, root_state=root_state, seed=seed, **engine_kw)
         self.c_pw = c_pw
         self.kappa = kappa
+        self._env = self._engine_kw.pop("env", None) or PENDULUM
 
     def _engine_config(self, max_trees: int) -> EngineConfig:
         d = describe_model(self.model)
@@ -264,7 +282,7 @@ class MCTSContinuous(MCTS):
                             activation=d["activation"], V_target_policy=self.V_target_policy, c_uct=self.c_uct, c_pw=self.c_pw,
                             kappa=self.kappa, gamma=float(self.gamma), epsilon=self.epsilon, action_bound=d["action_bound"],
                             log_std_min=d["log_std_min"], log_std_max=d["log_std_max"], device=self._cuda_index(), seed=self.seed,
-                            **self._engine_kw)
+                            env=self._env, **self._engine_kw)
 
     def search(self, *args, **kwargs) -> None:
         Env, n_mcts, c = self._env_from_args(args, kwargs)
@@ -272,8 +290,17 @@ class MCTSContinuous(MCTS):
             self.close()
             self.n_rollouts, self.c_uct = n_mcts, c
         hidden = env_hidden_state(Env, CONTINUOUS)
+        env = continuous_env(Env)
+        if env != self._env:  # the engines are built for one env
+            self.close()
+            self._env = env
         # initialize_search (mcts.py:589-600): always a new root; the tree is never reused
-        obs = self.root_state if self.root_state is not None else np.array([np.cos(hidden[0]), np.sin(hidden[0]), hidden[1]])
+        if self.root_state is not None:
+            obs = self.root_state
+        elif env == MOUNTAIN_CAR_CONTINUOUS:
+            obs = hidden.copy()  # the observation is the state itself
+        else:
+            obs = np.array([np.cos(hidden[0]), np.sin(hidden[0]), hidden[1]])
         self.root_node = RootNode(np.asarray(obs), n=0, hidden=hidden)
         eng = self._engine(1)
         eng.set_reward_model(*reward_model(Env, CONTINUOUS))

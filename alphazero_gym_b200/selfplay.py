@@ -17,15 +17,16 @@ import torch
 
 from . import _cabi
 from ._cabi import CONTINUOUS, DISCRETE, check
-from .engine import SearchEngine
+from .engine import MOUNTAIN_CAR_CONTINUOUS, SearchEngine
 from .parallel import PackedRows, allgather_results, broadcast_weights
 
 ROW_KEYS = ("obs", "actions", "counts", "Q", "V_target")  # buffer.store((s, actions, counts, Qs, V)), buffers.py:61
 
 
-def initial_states(variant: int, B: int, seed: int = 34, tree_id0: int = 0, total: Optional[int] = None) -> np.ndarray:
+def initial_states(variant: int, B: int, seed: int = 34, tree_id0: int = 0, total: Optional[int] = None,
+                   env: Optional[str] = None) -> np.ndarray:
     """Env.reset() for every environment: the same rule as SURVEY 8d configs 3/4 (numpy default_rng(seed) over the GLOBAL
-    batch, this shard's slice)."""
+    batch, this shard's slice).  env (engine.EngineConfig.env): MOUNTAIN_CAR_CONTINUOUS draws position ~ U(-0.6, -0.4), velocity 0."""
     if total is None:
         # the draw below runs over the GLOBAL batch, so every rank must use the same `total`: tree_id0 + B is only right for a
         # single shard (or the last one)
@@ -35,6 +36,8 @@ def initial_states(variant: int, B: int, seed: int = 34, tree_id0: int = 0, tota
     rng = np.random.default_rng(seed)
     if variant == DISCRETE:
         s = rng.uniform(-0.05, 0.05, size=(total, 4))
+    elif env == MOUNTAIN_CAR_CONTINUOUS:
+        s = np.stack([rng.uniform(-0.6, -0.4, total), np.zeros(total)], 1)
     else:
         s = np.stack([rng.uniform(-np.pi, np.pi, total), rng.uniform(-1.0, 1.0, total)], 1)
     return np.ascontiguousarray(s[tree_id0:tree_id0 + B])
@@ -134,7 +137,7 @@ class SelfPlayDriver:
         sd, S, cm = engine.state_cols, cfg.state_dim, engine.cmax
         self.variant = cfg.variant
         z = lambda shape, dt: torch.zeros(shape, dtype=dt, device=dev)
-        self.env_state = torch.from_numpy(initial_states(cfg.variant, B, seed, tree_id0, self.total)).to(dev)
+        self.env_state = torch.from_numpy(initial_states(cfg.variant, B, seed, tree_id0, self.total, cfg.env_name())).to(dev)
         # the replay row of a step (ROW_KEYS) lives in ONE byte buffer, so that its all-gather is a single collective (parallel.PackedRows)
         self.packed = PackedRows([("Q", (cm,), torch.float64), ("V_target", (), torch.float64), ("obs", (S,), torch.float32),
                                   ("actions", (cm,), torch.float32), ("counts", (cm,), torch.int32)], B, dev)

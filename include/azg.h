@@ -31,7 +31,8 @@ extern "C" {
 #define AZG_ECAPACITY -5   /* tree arena / child fan-out capacity exceeded */
 
 #define AZG_DISCRETE 0   /* MCTSDiscrete  + CartPole-v0 dynamics + DiscretePolicy   */
-#define AZG_CONTINUOUS 1 /* MCTSContinuous + Pendulum-v0 dynamics + DiagonalNormal/GMM policy */
+#define AZG_CONTINUOUS 1 /* MCTSContinuous + Pendulum-v0 (or, with AZG_FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS, MountainCarContinuous-v0)
+                           dynamics + DiagonalNormal/GMM policy */
 
 #define AZG_ACT_RELU 0
 #define AZG_ACT_ELU 1
@@ -53,7 +54,7 @@ typedef struct azg_config {
     int32_t max_trees;      /* capacity: largest batch B */
     int32_t num_actions;    /* discrete: 2 (CartPole) */
     int32_t num_components; /* continuous: K mixture components (1 = DiagonalNormalPolicy) */
-    int32_t state_dim;      /* network input width: 4 CartPole, 3 Pendulum */
+    int32_t state_dim;      /* network input width: 4 CartPole, 3 Pendulum, 2 MountainCarContinuous */
     int32_t hidden;         /* hidden width (all hidden layers equal; 128 in both shipped configs) */
     int32_t n_hidden;       /* hidden layers: 2 (DiscretePolicy.yaml) / 3 (ContinuousPolicy.yaml) */
     int32_t activation;     /* AZG_ACT_* */
@@ -93,6 +94,13 @@ typedef struct azg_config {
                                    reproduced (goldens tests/golden/cartpole_mt_*, pendulum_mt_*).  The continuous variant runs
                                    this mode with one launch per simulation (no AZG_FLAG_FUSED). */
 
+#define AZG_FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS 16u /* continuous variant only, with state_dim 2: the search steps MountainCarContinuous-v0
+                                   (gym 0.17-0.19 continuous_mountain_car.py) instead of Pendulum-v0.  Hidden state (position,
+                                   velocity), network input (float)position, (float)velocity; an episode ends at the goal, so
+                                   expanded nodes can be terminal (V = 0).  The search reward is r / 16.2736044 as for every
+                                   continuous search (mcts.py:687).  Every schedule, every other flag and the row, control-block and
+                                   result layouts are those of the Pendulum search. */
+
 typedef struct azg_engine azg_engine;
 
 int azg_create(const azg_config* cfg, azg_engine** out);
@@ -115,7 +123,8 @@ int azg_set_weights(azg_engine* e, const float* flat, int64_t n, void* stream);
 int azg_search_discrete(azg_engine* e, int32_t B, const double* d_root_state, const int32_t* d_root_n_init,
                         int32_t n_rollouts, int64_t tree_id0, void* stream);
 
-/* Batched MCTSContinuous.search (mcts.py:656-702) over B Pendulum roots; d_root_state [B][2] (th, thdot). */
+/* Batched MCTSContinuous.search (mcts.py:656-702) over B Pendulum roots; d_root_state [B][2] (th, thdot)
+ * (MountainCarContinuous: (position, velocity)). */
 int azg_search_continuous(azg_engine* e, int32_t B, const double* d_root_state, int32_t n_rollouts, int64_t tree_id0,
                           void* stream);
 
@@ -170,7 +179,8 @@ int azg_set_reward_model(azg_engine* e, double reward_step, double reward_termin
  *   (reset_mcts), else discrete tree reuse: d_root_n = visit count of the chosen child (mcts.py:495-526).
  * All pointers are device pointers owned by the caller; in/out arrays carry the state from step to step. */
 typedef struct azg_selfplay_io {
-    double* d_env_state;   /* in/out [B][4|2] hidden env state (CartPole x, x_dot, theta, theta_dot | Pendulum th, thdot) */
+    double* d_env_state;   /* in/out [B][4|2] hidden env state (CartPole x, x_dot, theta, theta_dot | Pendulum th, thdot |
+                              MountainCarContinuous position, velocity) */
     int32_t* d_ep_step;    /* in/out [B] steps taken in the current episode */
     int32_t* d_episode;    /* in/out [B] episode counter (indexes the reset stream) */
     int32_t* d_root_n;     /* in/out [B] discrete only: root visit count carried into the next search; NULL for continuous */
@@ -254,7 +264,7 @@ int azg_profile_search(azg_engine* e, int32_t B, const double* d_root_state, con
 int32_t azg_head_dim(const azg_engine* e);
 int azg_mlp_forward(azg_engine* e, int32_t n, const float* d_x, float* d_V, float* d_head, void* stream);
 
-/* Batched env.step on its own (known-answer tests): d_state [n][4|2], d_action [n] (index as float for
+/* Batched env.step of the engine's env on its own (known-answer tests): d_state [n][4|2], d_action [n] (index as float for
  * CartPole) -> d_next [n][4|2], d_reward [n] (raw env reward), d_terminal [n], d_obs [n][state_dim]. */
 int azg_env_step(azg_engine* e, int32_t n, const double* d_state, const float* d_action, double* d_next, double* d_reward,
                  int32_t* d_terminal, float* d_obs, void* stream);
