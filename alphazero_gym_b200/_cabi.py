@@ -22,6 +22,7 @@ FLAG_EVAL_Q8 = 2
 FLAG_FUSED = 4
 FLAG_RNG_MT19937 = 8
 FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS = 16
+FLAG_ENV_MOUNTAIN_CAR = 32
 
 EXPORTS = [
     "azg_create", "azg_destroy", "azg_last_error", "azg_version", "azg_num_weights", "azg_set_weights",

@@ -36,6 +36,28 @@ struct __align__(16) DRow {  // NodeDiscrete + its ActionDiscrete[2]   (states.p
 static_assert(sizeof(DRow) == 64, "discrete row must be two 32 B sectors");
 #define DROW_NONE 0xFFFFu
 
+// The three-action row (MountainCar-v0): two aligned 64 B lines.  Line 0 holds everything the descent reads at a node, so a level
+// still costs one 64 B burst; line 1 holds what only the backup (r) and the tree dump (parent links) read.
+struct __align__(16) D3Row {  // NodeDiscrete + its ActionDiscrete[3]
+    // line 0
+    double W[3];             // Action.W
+    int32_t n_e[3];          // Action.n
+    float prior[3];          // Node.priors
+    float V;                 // Node.V (0 for terminal nodes)
+    int32_t node_n;          // Node.n
+    uint16_t child[3];       // Action.child_node (DROW_NONE if absent)
+    uint8_t flags;           // ROW_TERMINAL
+    uint8_t pad0;
+    // line 1
+    double r;                // Node.r
+    uint16_t parent;         // Node.parent_action.parent_node
+    uint8_t paction;         // Node.parent_action.action
+    uint8_t pad1[53];
+};
+static_assert(sizeof(D3Row) == 128, "three-action row must be two 64 B lines");
+static_assert(offsetof(D3Row, n_e) == 24 && offsetof(D3Row, prior) == 36 && offsetof(D3Row, V) == 48 && offsetof(D3Row, node_n) == 52 &&
+              offsetof(D3Row, child) == 56 && offsetof(D3Row, flags) == 62 && offsetof(D3Row, r) == 64, "line 0 = what the descent reads");
+
 struct __align__(16) CRow {  // ActionContinuous + the NodeContinuous it leads to (states.py:194-289, :365-433)
     // sector 0 ("hot" sector, struct CHot) -- read for every child scanned by UCT and rewritten by backup.
     // For children of the ROOT this sector is not used: their hot sectors live contiguously in the root edge
@@ -106,8 +128,8 @@ struct TreeParams {
     int32_t tree_word;      // launches captured into a CUDA graph: the global id of tree 0 is seedp[1] (and tree_id0 is 0), so that one
                             // graph serves every tree_id0 (the drop-in classes search with a new id every call)
     // discrete tables
-    DRow* drows;      // [B][R]
-    double* dstate;   // [B][R][4]
+    DRow* drows;      // [B][R]  (MountainCar-v0: D3Row [B][R], same pointer)
+    double* dstate;   // [B][R][4]  (MountainCar-v0: the first 2 of each 4)
     // continuous tables
     CRow* crows;      // [B][R]
     float* chead;     // [B][R][HS]  mu[K], sigma[K], prob[K]
@@ -129,7 +151,8 @@ struct TreeParams {
     uint32_t* mt;     // [B][625] AZG_FLAG_RNG_MT19937: per-tree MT19937 state + index word of CPython's generator (see mt19937 below)
     uint32_t* tmt;    // [B][628] AZG_FLAG_RNG_MT19937, continuous: torch's CPU generator (state, index, cached normal lo / hi / valid)
     int32_t rng_mt;
-    uint16_t* dpath;  // [B][R] discrete: the current simulation's path, (row << 1 | action) per level, root first (read by the backup)
+    uint16_t* dpath;  // [B][R] discrete: the current simulation's path, (row << 1 | action) per level (three actions: row << 2 | action),
+                      // root first (read by the backup)
     int32_t* ddepth;  // [B]    discrete: its length
     uint32_t* ctr;    // [4][B]: levels, children scanned, terminal-leaf sims, evals
     float4* X;        // [B] network input of the leaf

@@ -94,6 +94,7 @@ struct azg_engine {
     int l2_on = 0;
     bool fused = false;  // AZG_FLAG_FUSED: the whole continuous search in one persistent kernel (qmlp2.cuh)
     bool mcc = false;    // AZG_FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS: the continuous kernels are instantiated for env::MountainCarContinuous
+    bool mc = false;     // AZG_FLAG_ENV_MOUNTAIN_CAR: the discrete kernels are instantiated for env::MountainCar (three-action rows)
     // results staging (device) + pinned host staging for the *_host entry point
     float* r_actions = nullptr;
     int32_t* r_counts = nullptr;
@@ -128,6 +129,9 @@ static int head_dim_of(const azg_config& c) {
     if (c.variant == AZG_DISCRETE) return c.num_actions;
     return c.num_components > 1 ? 3 * c.num_components : 2;
 }
+
+// width of the hidden-state arrays the host hands in and gets back: CartPole 4, MountainCar and the continuous envs 2
+static int state_width(const azg_engine* e) { return e->cfg.variant == AZG_DISCRETE && !e->mc ? 4 : 2; }
 
 static int pw_limit(double c_pw, double kappa, int n) { return (int)std::ceil(c_pw * std::pow((double)(n + 1), kappa)); }
 
@@ -177,10 +181,17 @@ extern "C" int azg_create(const azg_config* cfg, azg_engine** out) {
     const bool mcc = (c.flags & AZG_FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS) != 0;
     if (mcc && (c.variant != AZG_CONTINUOUS || c.state_dim != 2))
         return fail(AZG_EINVAL, "AZG_FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS needs the continuous variant and state_dim 2");
+    const bool mc = (c.flags & AZG_FLAG_ENV_MOUNTAIN_CAR) != 0;
+    if (mc && mcc) return fail(AZG_EINVAL, "AZG_FLAG_ENV_MOUNTAIN_CAR and AZG_FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS exclude each other");
+    if (mc && (c.variant != AZG_DISCRETE || c.num_actions != 3 || c.state_dim != 2))
+        return fail(AZG_EINVAL, "AZG_FLAG_ENV_MOUNTAIN_CAR needs the discrete variant, num_actions 3 and state_dim 2");
     if (c.variant == AZG_DISCRETE) {
-        if (c.num_actions != 2 || c.state_dim != 4)
-            return fail(AZG_EINVAL, "discrete variant is CartPole: num_actions must be 2 and state_dim 4");
+        if (!mc && (c.num_actions != 2 || c.state_dim != 4))
+            return fail(AZG_EINVAL, "discrete variant is CartPole (num_actions 2, state_dim 4) or, with AZG_FLAG_ENV_MOUNTAIN_CAR, MountainCar-v0 "
+                                    "(num_actions 3, state_dim 2)");
         if (c.max_rollouts + 2 > 65534) return fail(AZG_EINVAL, "max_rollouts too large for 16-bit child links");
+        if (mc && c.max_rollouts + 2 > 16384)
+            return fail(AZG_EINVAL, "MountainCar-v0 supports max_rollouts <= 16382 (a path entry holds row << 2 | action in 16 bits)");
     } else {
         if (!mcc && c.state_dim != 3) return fail(AZG_EINVAL, "continuous variant is Pendulum: state_dim must be 3");
         if (c.num_components < 1 || c.num_components > AZG_MAX_K) return fail(AZG_EINVAL, "num_components must be in 1..8");
@@ -194,6 +205,7 @@ extern "C" int azg_create(const azg_config* cfg, azg_engine** out) {
     azg_engine* e = new azg_engine();
     e->cfg = c;
     e->mcc = mcc;
+    e->mc = mc;
     e->R = c.max_rollouts + 2;
     e->P = head_dim_of(c);
     e->PO_PAD = ((1 + e->P) + 3) / 4 * 4;
@@ -234,9 +246,10 @@ extern "C" int azg_create(const azg_config* cfg, azg_engine** out) {
         delete e;
         return fail(AZG_EINVAL, "AZG_FLAG_RNG_MT19937 with the continuous search runs one launch per simulation (no AZG_FLAG_FUSED)");
     }
-    if (e->fused && !(e->q8 && c.state_dim == (c.variant == AZG_CONTINUOUS ? (mcc ? 2 : 3) : 4))) {
+    if (e->fused && !(e->q8 && c.state_dim == (c.variant == AZG_CONTINUOUS ? (mcc ? 2 : 3) : (mc ? 2 : 4)))) {
         delete e;
-        return fail(AZG_EINVAL, "AZG_FLAG_FUSED needs AZG_FLAG_EVAL_Q8 and the shipped envs (state_dim 3 Pendulum / 2 MountainCarContinuous / 4 CartPole)");
+        return fail(AZG_EINVAL, "AZG_FLAG_FUSED needs AZG_FLAG_EVAL_Q8 and the shipped envs (state_dim 3 Pendulum / 2 MountainCarContinuous / 4 CartPole / "
+                                "2 MountainCar)");
     }
     const size_t B = c.max_trees, R = e->R;
     std::vector<int32_t> pwt;
@@ -264,7 +277,7 @@ extern "C" int azg_create(const azg_config* cfg, azg_engine** out) {
         }                                               \
     } while (0)
     if (c.variant == AZG_DISCRETE) {
-        ALLOC(drows, B * R);
+        ALLOC(drows, B * R * (mc ? sizeof(D3Row) / sizeof(DRow) : 1));  // MountainCar: D3Row [B][R]
         ALLOC(dstate, B * R * 4);
         ALLOC(dpath, B * R);
         ALLOC(ddepth, B);
@@ -569,7 +582,7 @@ static cudaError_t launch_qmlp_t(const azg_engine* e, const MlpParams& m, cudaSt
         if (ce != cudaSuccess) return ce;
         ce = cudaFuncSetAttribute(k_qmlp2<ENV, ACT, NL, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)e->qmlp_smem);
         if (ce != cudaSuccess) return ce;
-        if constexpr (ENV::DISCRETE) {  // trees in shared memory: everything the SM has beyond the kernel's static allocation
+        if constexpr (env::actions_of<ENV>() == 2) {  // trees in shared memory (CartPole): everything the SM has beyond the kernel's static allocation
             cudaFuncAttributes fa;
             ce = cudaFuncGetAttributes(&fa, k_qmlp2<ENV, ACT, NL, true, true>);
             if (ce != cudaSuccess) return ce;
@@ -595,8 +608,8 @@ static cudaError_t launch_qmlp_t(const azg_engine* e, const MlpParams& m, cudaSt
 template <class ENV, int ACT, int NL>
 static cudaError_t launch_fused_t(const azg_engine* e, const MlpParams& m, const TreeParams& p, int N, cudaStream_t st, int* launches) {
     int chunk = e->sm_count * Q2_MAX_TILES * 128;
-    if constexpr (ENV::DISCRETE) {
-        // Discrete search: up to two full waves of shared-memory-resident trees (cap per SM x SMs each) beat the two-phase kernel on
+    if constexpr (env::actions_of<ENV>() == 2) {
+        // CartPole search: up to two full waves of shared-memory-resident trees (cap per SM x SMs each) beat the two-phase kernel on
         // rows in HBM, whose simulation takes 32 us whatever the batch (measured, profiles/README.md r2p: 8192 trees 248 M sims/s
         // there against 2 x 4096 at 337 M) -- so such a batch is cut into equal chunks, one launch each
         int cap = 0;
@@ -617,7 +630,7 @@ static cudaError_t launch_fused_t(const azg_engine* e, const MlpParams& m, const
         // Discrete search, thin batch: when the rows of ceil(trees / SMs) trees fit in an SM's shared memory next to the evaluation's
         // operands, the CTA keeps its trees there for the whole search (tree_discrete.cuh ds_step; BASELINE config 3: 28 trees per SM)
         int tsm_per = 0;
-        if constexpr (ENV::DISCRETE) {
+        if constexpr (env::actions_of<ENV>() == 2) {  // (not built for three-action rows: MountainCar's thin batches run the two-phase kernel)
             const int per = (hi - lo + e->sm_count - 1) / e->sm_count;
             if (two_phase && !p.rng_mt && !getenv("AZG_NO_TSM") && per <= 128 &&
                 qmlp2_tsm_smem_bytes(NL, e->qfl_count, per, p.R, e->PO_PAD) <= e->tsm_smem_max)
@@ -625,7 +638,7 @@ static cudaError_t launch_fused_t(const azg_engine* e, const MlpParams& m, const
         }
         const_cast<azg_engine*>(e)->last_fused_kind = tsm_per ? 3 : (two_phase ? 1 : 2);
         if (tsm_per) {
-            if constexpr (ENV::DISCRETE) {
+            if constexpr (env::actions_of<ENV>() == 2) {
                 const int grid = (hi - lo + tsm_per - 1) / tsm_per;
                 ce = launch_ex(e, k_qmlp2<ENV, ACT, NL, true, true>, grid, Q2_THREADS, qmlp2_tsm_smem_bytes(NL, e->qfl_count, tsm_per, p.R, e->PO_PAD), st, m, p, N, lo, hi);
             }
@@ -651,6 +664,13 @@ using ShippedEnv = std::conditional_t<S == 4, env::CartPole, env::Pendulum>;
 
 static cudaError_t launch_fused(const azg_engine* e, const MlpParams& m, const TreeParams& p, int N, cudaStream_t st, int* launches) {
     const int S = e->cfg.state_dim, A = e->cfg.activation, NL = e->cfg.n_hidden - 1;
+    if (e->mc) {
+#define FUSED_MC_CASE(a, nl) \
+    if (A == a && NL == nl) return launch_fused_t<env::MountainCar, a, nl>(e, m, p, N, st, launches);
+        FUSED_MC_CASE(0, 1) FUSED_MC_CASE(1, 1) FUSED_MC_CASE(0, 2) FUSED_MC_CASE(1, 2)
+#undef FUSED_MC_CASE
+        return cudaErrorInvalidValue;
+    }
     if (e->mcc) {
 #define FUSED_MCC_CASE(a, nl) \
     if (A == a && NL == nl) return launch_fused_t<env::MountainCarContinuous, a, nl>(e, m, p, N, st, launches);
@@ -670,6 +690,13 @@ static cudaError_t launch_mlp(const azg_engine* e, const MlpParams& m, cudaStrea
     const int H = e->cfg.hidden, S = e->cfg.state_dim, A = e->cfg.activation;
     if (e->q8) {
         const int NL = e->cfg.n_hidden - 1;
+        if (e->mc) {
+#define QMLP_MC_CASE(a, nl) \
+    if (A == a && NL == nl) return launch_qmlp_t<env::MountainCar, a, nl>(e, m, st, set_attr);
+            QMLP_MC_CASE(0, 1) QMLP_MC_CASE(1, 1) QMLP_MC_CASE(0, 2) QMLP_MC_CASE(1, 2)
+#undef QMLP_MC_CASE
+            return cudaErrorInvalidValue;
+        }
         if (e->mcc) {
 #define QMLP_MCC_CASE(a, nl) \
     if (A == a && NL == nl) return launch_qmlp_t<env::MountainCarContinuous, a, nl>(e, m, st, set_attr);
@@ -684,7 +711,7 @@ static cudaError_t launch_mlp(const azg_engine* e, const MlpParams& m, cudaStrea
 #undef QMLP_CASE
         return cudaErrorInvalidValue;
     }
-    if (e->mcc) {  // layer 0 with two inputs
+    if (e->mcc || e->mc) {  // layer 0 with two inputs (both MountainCar envs; k_mlp reads the row layout at run time)
 #define MLP_MCC_CASE(h, a) \
     if (H == h && A == a) return launch_mlp_t<h, 2, a>(e, m, st, set_attr);
         MLP_MCC_CASE(128, 0) MLP_MCC_CASE(128, 1) MLP_MCC_CASE(128, 2) MLP_MCC_CASE(128, 3) MLP_MCC_CASE(128, 4) MLP_MCC_CASE(128, 5)
@@ -702,6 +729,12 @@ static cudaError_t launch_mlp(const azg_engine* e, const MlpParams& m, cudaStrea
     MLP_CASE(64, 3, 2) MLP_CASE(64, 3, 3) MLP_CASE(64, 3, 4) MLP_CASE(64, 3, 5)
 #undef MLP_CASE
     return cudaErrorInvalidValue;
+}
+
+template <bool BK, bool SEL>
+static cudaError_t launch_step_discrete(const azg_engine* e, const TreeParams& p, cudaStream_t st) {
+    if (e->mc) return launch_ex(e, k_step_discrete<env::MountainCar, BK, SEL>, (p.B + 127) / 128, 128, 0, st, p);
+    return launch_ex(e, k_step_discrete<env::CartPole, BK, SEL>, (p.B + 127) / 128, 128, 0, st, p);
 }
 
 template <bool BK, bool SEL>
@@ -752,14 +785,15 @@ static int enqueue_search(azg_engine* e, int B, int N, int64_t tree_id0, cudaStr
         return launches;
     }
     if (e->cfg.variant == AZG_DISCRETE) {
-        LK(2, (k_init_discrete<<<tg, tb, 0, st>>>(p)));
+        if (e->mc) LK(2, (k_init_discrete<env::MountainCar><<<tg, tb, 0, st>>>(p)));
+        else LK(2, (k_init_discrete<env::CartPole><<<tg, tb, 0, st>>>(p)));
         if (!tape) LK(1, ce = launch_mlp(e, m, st, false));
         for (int it = 0; it < N; ++it) {
-            if (it == 0) LK(0, (k_step_discrete<false, true><<<tg, tb, 0, st>>>(p)));
-            else LK(0, (k_step_discrete<true, true><<<tg, tb, 0, st>>>(p)));
+            if (it == 0) LK(0, ce = (launch_step_discrete<false, true>(e, p, st)));
+            else LK(0, ce = (launch_step_discrete<true, true>(e, p, st)));
             if (!tape) LK(1, ce = launch_mlp(e, m, st, false));
         }
-        LK(0, (k_step_discrete<true, false><<<tg, tb, 0, st>>>(p)));
+        LK(0, ce = (launch_step_discrete<true, false>(e, p, st)));
     } else {
         if (e->mcc) LK(2, (k_init_continuous<env::MountainCarContinuous><<<tg, tb, 0, st>>>(p)));
         else LK(2, (k_init_continuous<env::Pendulum><<<tg, tb, 0, st>>>(p)));
@@ -785,7 +819,7 @@ static int run_search(azg_engine* e, int B, const double* d_root_state, const in
     if (!d_root_state) return fail(AZG_EINVAL, "null root state");
     if (!e->weights_set && !e->tapeV) return fail(AZG_EINVAL, "azg_set_weights has not been called");
     CK(cudaSetDevice(e->cfg.device));
-    const int sd = e->cfg.variant == AZG_DISCRETE ? 4 : 2;
+    const int sd = state_width(e);
     // stage the roots in engine-owned buffers so the captured graph has fixed addresses
     if (d_root_state != e->root_state)
         CK(cudaMemcpyAsync(e->root_state, d_root_state, (size_t)B * sd * sizeof(double), cudaMemcpyDeviceToDevice, st));
@@ -863,7 +897,7 @@ extern "C" int azg_profile_search(azg_engine* e, int32_t B, const double* d_root
     if (!e->weights_set && !e->tapeV) return fail(AZG_EINVAL, "azg_set_weights has not been called");
     CK(cudaSetDevice(e->cfg.device));
     cudaStream_t st = (cudaStream_t)stream;
-    const int sd = e->cfg.variant == AZG_DISCRETE ? 4 : 2;
+    const int sd = state_width(e);
     if (d_root_state != e->root_state)
         CK(cudaMemcpyAsync(e->root_state, d_root_state, (size_t)B * sd * sizeof(double), cudaMemcpyDeviceToDevice, st));
     if (e->cfg.variant == AZG_DISCRETE) {
@@ -898,7 +932,8 @@ extern "C" int azg_root_results(azg_engine* e, int32_t B, float* d_actions, int3
     cudaStream_t st = (cudaStream_t)stream;
     const TreeParams p = make_params(e, B, 0);
     const int tb = 128, tg = (B + tb - 1) / tb;
-    if (e->cfg.variant == AZG_DISCRETE) k_results_discrete<<<tg, tb, 0, st>>>(p, e->cmax, d_actions, d_counts, d_Q, d_V_target, d_n_children);
+    if (e->cfg.variant == AZG_DISCRETE && e->mc) k_results_discrete<env::MountainCar><<<tg, tb, 0, st>>>(p, e->cmax, d_actions, d_counts, d_Q, d_V_target, d_n_children);
+    else if (e->cfg.variant == AZG_DISCRETE) k_results_discrete<env::CartPole><<<tg, tb, 0, st>>>(p, e->cmax, d_actions, d_counts, d_Q, d_V_target, d_n_children);
     else k_results_continuous<<<tg, tb, 0, st>>>(p, e->cmax, d_actions, d_counts, d_Q, d_V_target, d_n_children);
     CK(cudaGetLastError());
     return AZG_OK;
@@ -924,7 +959,7 @@ extern "C" int azg_search_host(azg_engine* e, int32_t B, const double* h_root_st
     if (e->cfg.variant == AZG_CONTINUOUS && h_root_n_init) return fail(AZG_EINVAL, "root_n_init is a discrete-only argument");
     CK(cudaSetDevice(e->cfg.device));
     cudaStream_t st = e->own_stream;
-    const int sd = e->cfg.variant == AZG_DISCRETE ? 4 : 2;
+    const int sd = state_width(e);
     const size_t cm = e->cmax;
     // carve the pinned staging buffer
     char* hp = (char*)e->h_pinned;
@@ -1018,7 +1053,7 @@ extern "C" int azg_search_host_begin(azg_engine* e, int32_t slot, int32_t B, con
     double* rv = slot ? e->r2_Vt : e->r_Vt;
     int32_t* rn = slot ? e->r2_nchild : e->r_nchild;
     cudaStream_t st = e->own_stream;
-    const int sd = e->cfg.variant == AZG_DISCRETE ? 4 : 2;
+    const int sd = state_width(e);
     CK(cudaMemcpyAsync(e->root_state, h_root_state, (size_t)B * sd * sizeof(double), cudaMemcpyHostToDevice, st));
     const int32_t* d_rn = nullptr;
     if (h_root_n_init) {
@@ -1150,8 +1185,8 @@ extern "C" int azg_set_reward_model(azg_engine* e, double reward_step, double re
     if (!e) return fail(AZG_EINVAL, "null engine");
     if (!(reward_step == reward_step) || !(reward_terminal == reward_terminal) || std::isinf(reward_step) || std::isinf(reward_terminal))
         return fail(AZG_EINVAL, "rewards must be finite");
-    if (e->cfg.variant != AZG_DISCRETE && (reward_step != 1.0 || reward_terminal != 1.0))
-        return fail(AZG_EINVAL, "the reward model applies to the discrete (CartPole) search");
+    if ((e->cfg.variant != AZG_DISCRETE || e->mc) && (reward_step != 1.0 || reward_terminal != 1.0))
+        return fail(AZG_EINVAL, "the reward model applies to the CartPole search (the other envs' searches take the env's own reward)");
     if (reward_step == e->reward_step && reward_terminal == e->reward_terminal) return AZG_OK;
     CK(cudaSetDevice(e->cfg.device));
     CK(cudaDeviceSynchronize());
@@ -1192,7 +1227,8 @@ extern "C" int azg_selfplay_step(azg_engine* e, int32_t B, const azg_selfplay_io
     sp.obs = io->d_obs; sp.action_taken = io->d_action_taken; sp.reward = io->d_reward; sp.done = io->d_done;
     sp.drows = e->drows; sp.R = e->R;
     const int tb = 128, tg = (B + tb - 1) / tb;
-    if (disc) k_selfplay_discrete<<<tg, tb, 0, st>>>(sp);
+    if (disc && e->mc) k_selfplay_discrete<env::MountainCar><<<tg, tb, 0, st>>>(sp);
+    else if (disc) k_selfplay_discrete<env::CartPole><<<tg, tb, 0, st>>>(sp);
     else if (e->mcc) k_selfplay_continuous<env::MountainCarContinuous><<<tg, tb, 0, st>>>(sp);
     else k_selfplay_continuous<env::Pendulum><<<tg, tb, 0, st>>>(sp);
     CK(cudaGetLastError());
@@ -1200,17 +1236,14 @@ extern "C" int azg_selfplay_step(azg_engine* e, int32_t B, const azg_selfplay_io
 }
 
 // ---- tree dump (host side unpacking of the device tables) ------------------------------------------------
-extern "C" int azg_dump_tree_discrete(azg_engine* e, int32_t B, const azg_dump_discrete* o) {
-    if (!e || !o) return fail(AZG_EINVAL, "null argument");
-    if (e->cfg.variant != AZG_DISCRETE) return fail(AZG_EINVAL, "engine is not discrete");
-    if (B < 1 || B > e->cfg.max_trees) return fail(AZG_EINVAL, "B out of range");
-    CK(cudaSetDevice(e->cfg.device));
-    CK(cudaDeviceSynchronize());
-    const size_t R = e->R, A = 2;
-    std::vector<DRow> rows((size_t)B * R);
+// ROW = DRow (CartPole: A = 2, state 4 wide) or D3Row (MountainCar: A = 3, state 2 wide)
+template <class ROW>
+static int dump_discrete(azg_engine* e, int32_t B, const azg_dump_discrete* o, size_t A, size_t SW) {
+    const size_t R = e->R;
+    std::vector<ROW> rows((size_t)B * R);
     std::vector<double> st((size_t)B * R * 4);
     std::vector<int32_t> nr(B);
-    CK(cudaMemcpy(rows.data(), e->drows, rows.size() * sizeof(DRow), cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(rows.data(), e->drows, rows.size() * sizeof(ROW), cudaMemcpyDeviceToHost));
     CK(cudaMemcpy(st.data(), e->dstate, st.size() * sizeof(double), cudaMemcpyDeviceToHost));
     CK(cudaMemcpy(nr.data(), e->n_rows, (size_t)B * sizeof(int32_t), cudaMemcpyDeviceToHost));
     for (size_t t = 0; t < (size_t)B; ++t) {
@@ -1218,14 +1251,14 @@ extern "C" int azg_dump_tree_discrete(azg_engine* e, int32_t B, const azg_dump_d
         for (size_t i = 0; i < R; ++i) {
             const size_t q = t * R + i;
             const bool live = (int)i < nr[t];
-            const DRow& r = rows[q];
+            const ROW& r = rows[q];
             o->parent[q] = live ? (r.parent == DROW_NONE ? -1 : r.parent) : 0;
             o->paction[q] = live ? (r.parent == DROW_NONE ? -1 : r.paction) : 0;
             o->node_n[q] = live ? r.node_n : 0;
             o->terminal[q] = live ? (r.flags & ROW_TERMINAL) : 0;
             o->V[q] = live ? r.V : 0.0f;
             o->r[q] = live ? r.r : 0.0;
-            for (size_t k = 0; k < 4; ++k) o->state[q * 4 + k] = live ? st[q * 4 + k] : 0.0;
+            for (size_t k = 0; k < SW; ++k) o->state[q * SW + k] = live ? st[q * 4 + k] : 0.0;
             for (size_t a = 0; a < A; ++a) {
                 o->prior[q * A + a] = live ? r.prior[a] : 0.0f;
                 o->eW[q * A + a] = live ? r.W[a] : 0.0;
@@ -1235,6 +1268,16 @@ extern "C" int azg_dump_tree_discrete(azg_engine* e, int32_t B, const azg_dump_d
         }
     }
     return AZG_OK;
+}
+
+extern "C" int azg_dump_tree_discrete(azg_engine* e, int32_t B, const azg_dump_discrete* o) {
+    if (!e || !o) return fail(AZG_EINVAL, "null argument");
+    if (e->cfg.variant != AZG_DISCRETE) return fail(AZG_EINVAL, "engine is not discrete");
+    if (B < 1 || B > e->cfg.max_trees) return fail(AZG_EINVAL, "B out of range");
+    CK(cudaSetDevice(e->cfg.device));
+    CK(cudaDeviceSynchronize());
+    if (e->mc) return dump_discrete<D3Row>(e, B, o, 3, 2);
+    return dump_discrete<DRow>(e, B, o, 2, 4);
 }
 
 extern "C" int azg_dump_tree_continuous(azg_engine* e, int32_t B, const azg_dump_continuous* o) {
@@ -1316,10 +1359,18 @@ __device__ __forceinline__ void env_step_continuous(int i, const double* s, cons
     term[i] = t;
 }
 
-__global__ void k_env_step(int variant, bool mcc, int n, const double* s, const float* a, double* o, double* rew, int32_t* term, float* obs) {
+__global__ void k_env_step(int variant, bool mcc, bool mc, int n, const double* s, const float* a, double* o, double* rew, int32_t* term,
+                           float* obs) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    if (variant == AZG_DISCRETE) {
+    if (variant == AZG_DISCRETE && mc) {  // the action is an index 0, 1, 2
+        double n0, n1, r;
+        const bool t = env::MountainCar::step(s[i * 2], s[i * 2 + 1], (int)a[i], n0, n1, r);
+        o[i * 2] = n0; o[i * 2 + 1] = n1;
+        obs[i * 2] = (float)n0; obs[i * 2 + 1] = (float)n1;
+        rew[i] = r;
+        term[i] = t;
+    } else if (variant == AZG_DISCRETE) {
         const double in[4] = {s[i * 4], s[i * 4 + 1], s[i * 4 + 2], s[i * 4 + 3]};
         double out[4], r;
         const bool t = env::cartpole_step(in, (int)a[i], out, r);
@@ -1338,7 +1389,7 @@ extern "C" int azg_env_step(azg_engine* e, int32_t n, const double* d_state, con
     if (!e || !d_state || !d_action || !d_next || !d_reward || !d_terminal || !d_obs) return fail(AZG_EINVAL, "null argument");
     if (n < 1) return fail(AZG_EINVAL, "n must be >= 1");
     CK(cudaSetDevice(e->cfg.device));
-    k_env_step<<<(n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(e->cfg.variant, e->mcc, n, d_state, d_action, d_next, d_reward, d_terminal, d_obs);
+    k_env_step<<<(n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(e->cfg.variant, e->mcc, e->mc, n, d_state, d_action, d_next, d_reward, d_terminal, d_obs);
     CK(cudaGetLastError());
     return AZG_OK;
 }

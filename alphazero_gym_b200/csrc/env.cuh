@@ -85,11 +85,41 @@ __device__ __forceinline__ bool mountain_car_step(double pos, double vel, float 
     return done;
 }
 
-// The env of a continuous search as a compile-time type: the hidden state is two doubles (CRow sector 1), the network input the
-// first S lanes of a float4.  CartPole names the discrete tree in the kernels that serve both variants.
+// MountainCar-v0 (gym 0.17-0.19 classic_control/mountain_car.py); returns done.  The right-hand side of `velocity +=` is summed
+// first; (action - 1) * force is an int times a float (-0.001, +0.0 or 0.001); np.clip passes a NaN and keeps -0; the left wall stores
+// the int 0 (+0 from then on); done is false for a NaN state; the reward is -1.0 on every step, the terminating one included.
+__device__ __forceinline__ bool mountain_car_step(double pos, double vel, int action, double& newpos, double& newvel, double& reward) {
+    const double min_position = -1.2, max_position = 0.6, max_speed = 0.07, goal_position = 0.5, force = 0.001, gravity = 0.0025;
+    vel = vel + ((double)(action - 1) * force + det::cos_(3 * pos) * -gravity);
+    vel = vel < -max_speed ? -max_speed : (vel > max_speed ? max_speed : vel);
+    pos = pos + vel;
+    pos = pos < min_position ? min_position : (pos > max_position ? max_position : pos);
+    if (pos == min_position && vel < 0) vel = 0.0;
+    newpos = pos;
+    newvel = vel;
+    reward = -1.0;
+    return pos >= goal_position && vel >= 0.0;
+}
+
+// The env of a search as a compile-time type.  Continuous: the hidden state is two doubles (CRow sector 1), the network input the
+// first S lanes of a float4.  Discrete: A actions, the row layout follows (DRow for 2, D3Row for 3).  CartPole names the discrete tree
+// in the kernels that serve both variants.
 struct CartPole {
-    static constexpr int S = 4;
+    static constexpr int S = 4, A = 2;
     static constexpr bool DISCRETE = true;
+};
+struct MountainCar {
+    static constexpr int S = 2, A = 3;
+    static constexpr bool DISCRETE = true;
+    static __device__ __forceinline__ bool step(double pos, double vel, int a, double& npos, double& nvel, double& r) {
+        return mountain_car_step(pos, vel, a, npos, nvel, r);
+    }
+    static __device__ __forceinline__ float4 obs(double pos, double vel) { return make_float4((float)pos, (float)vel, 0.0f, 0.0f); }
+    // Env.reset: position ~ U(-0.6, -0.4), velocity +0 (the same formula as MountainCarContinuous)
+    static __device__ __forceinline__ void reset(double u0, double, double& pos, double& vel) {
+        pos = -0.6 + (-0.4 - -0.6) * u0;
+        vel = 0.0;
+    }
 };
 struct Pendulum {
     static constexpr int S = 3;
@@ -118,5 +148,15 @@ struct MountainCarContinuous {
         vel = 0.0;
     }
 };
+
+// actions of a discrete env, 0 for a continuous one
+template <class ENV>
+__host__ __device__ constexpr int actions_of() {
+    if constexpr (ENV::DISCRETE) return ENV::A;
+    else return 0;
+}
+// whether an env's search writes three-action rows (D3Row)
+template <class ENV>
+__host__ __device__ constexpr bool row3() { return actions_of<ENV>() == 3; }
 
 }  // namespace env

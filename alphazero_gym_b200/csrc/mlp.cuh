@@ -212,7 +212,10 @@ __device__ __forceinline__ void finish_row_continuous(const MlpParams& p, int gr
 }
 
 // post-processing + write-back of one evaluated row: V and the raw policy-head outputs -> softmax priors / GMM parameters ->
-// the tree tables (mode 0) or dense outputs (mode 1).  Shared by k_mlp and k_qmlp2; the caller counts the evaluation.
+// the tree tables (mode 0) or dense outputs (mode 1).  Shared by k_mlp, k_qmlp2 and k_search_wg; the caller counts the evaluation.
+// ROW3: the discrete tree may hold three-action rows (D3Row, MountainCar-v0), told apart by p.A at run time.  k_mlp serves every env
+// and passes true; the k_qmlp2 / k_search_wg instantiations know their env and pass whether it is MountainCar.
+template <bool ROW3>
 __device__ __forceinline__ void mlp_finish_row(const MlpParams& p, int gr, int leafw, double lr, float V, const float* raw) {
     if (p.mode == 0 && p.variant == 0 && p.A == 2) {  // CartPole: softmax_seq over two logits, written out (registers only)
         const float m = raw[1] > raw[0] ? raw[1] : raw[0];
@@ -222,6 +225,16 @@ __device__ __forceinline__ void mlp_finish_row(const MlpParams& p, int gr, int l
         d->V = (leafw & LEAF_TERMINAL) ? 0.0f : V;  // mcts.py:406-410
         *reinterpret_cast<float2*>(d->prior) = make_float2(__fdiv_rn(e0, sum), __fdiv_rn(e1, sum));
         return;
+    }
+    if constexpr (ROW3) {
+        if (p.mode == 0 && p.variant == 0 && p.A == 3) {  // MountainCar: softmax_seq over three logits into line 0 of the D3Row
+            float pr[3];
+            softmax_seq(raw, 3, pr);
+            D3Row* d = reinterpret_cast<D3Row*>(p.drows) + (size_t)gr * p.R + (leafw & LEAF_ROW_MASK);
+            d->V = (leafw & LEAF_TERMINAL) ? 0.0f : V;
+            d->prior[0] = pr[0]; d->prior[1] = pr[1]; d->prior[2] = pr[2];
+            return;
+        }
     }
     if (p.mode == 0 && p.variant == 1) {
         switch (p.K) {
@@ -425,7 +438,7 @@ __device__ __forceinline__ void mlp_unit(const MlpParams& p, const float* w, flo
     if (q == 0 && need) {
         float raw[3 * AZG_MAX_K];
         for (int i = 0; i < p.P; ++i) raw[i] = outg[(1 + i) * TU + row];
-        mlp_finish_row(p, gr, leafw, lr, outg[row], raw);
+        mlp_finish_row<true>(p, gr, leafw, lr, outg[row], raw);  // k_mlp serves every env: the row layout is known at run time
         if (p.mode == 0) p.evals[gr] += 1;
     }
 }

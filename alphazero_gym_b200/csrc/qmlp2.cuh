@@ -237,7 +237,8 @@ __device__ __forceinline__ void q2_heads_tsm(const Q2Ctx& c, const MlpParams& p,
     }
 }
 
-// post-processing warp of row group lg: one thread per row of the tile in slot T
+// post-processing warp of row group lg: one thread per row of the tile in slot T (ROW3: mlp_finish_row)
+template <bool ROW3>
 __device__ __forceinline__ void q2_finish_tile(const MlpParams& p, uint32_t tb, const float* bh, int lg, int T, bool need, int gr, int leafw,
                                                double lr, uint64_t* hfree, uint32_t& nev, int& ev_row) {
     const uint32_t lane_base = tb + ((uint32_t)(lg * 32) << 16) + Q2_SCRATCH_COL + T * 64;
@@ -262,7 +263,7 @@ __device__ __forceinline__ void q2_finish_tile(const MlpParams& p, uint32_t tb, 
     tc_fence_before();
     mbar_arrive(hfree + T);  // the scratch columns may be reused (half-0 activations of the next tile in this slot)
     if (need) {
-        mlp_finish_row(p, gr, leafw, lr, out[0], out + 1);
+        mlp_finish_row<ROW3>(p, gr, leafw, lr, out[0], out + 1);
         ++nev;
         ev_row = gr;
     }
@@ -420,7 +421,7 @@ template <class ENV, int ACT, int NL, bool FUSED, bool TSM = false>
 __global__ void __launch_bounds__(Q2_THREADS, 1)
 k_qmlp2(const MlpParams p_in, const TreeParams tp, const int n_sims, const int chunk_begin, const int chunk_end) {
     constexpr int S = ENV::S;
-    static_assert(!TSM || (FUSED && ENV::DISCRETE), "trees in shared memory: whole-search kernel of the discrete tree");
+    static_assert(!TSM || (FUSED && env::actions_of<ENV>() == 2), "trees in shared memory: whole-search kernel of the two-action discrete tree");
     extern __shared__ __align__(1024) uint8_t qsm_raw[];
     __shared__ __align__(8) uint64_t wbar, full[2], ready[2], freeb[2], hfull[2], hfree[2], phase_bar;
     __shared__ uint32_t tmem_base_s;
@@ -569,7 +570,7 @@ k_qmlp2(const MlpParams p_in, const TreeParams tp, const int n_sims, const int c
             mbar_wait(&hfull[T], (hph >> T) & 1u);
             hph ^= 1u << T;
             tc_fence_after();
-            if (lg * 32 < nv) q2_finish_tile(p, tb, bh, lg, T, need, gr, leafw, lr, hfree, nev, ev_row);
+            if (lg * 32 < nv) q2_finish_tile<env::row3<ENV>()>(p, tb, bh, lg, T, need, gr, leafw, lr, hfree, nev, ev_row);
             else mbar_arrive(&hfree[T]);
         }
         if (FUSED) {
@@ -641,7 +642,7 @@ k_qmlp2(const MlpParams p_in, const TreeParams tp, const int n_sims, const int c
         if (FUSED) {  // MCTSContinuous.initialize_search for every tree of the CTA
             for (int i = tid; i < nrows; i += Q2_EPI_THREADS) {
                 if (TSM) ds_init(tp, smt, i, row_begin + i);
-                else if constexpr (ENV::DISCRETE) d_init(tp, row_begin + i);
+                else if constexpr (ENV::DISCRETE) d_init<ENV>(tp, row_begin + i);
                 else c_init<ENV>(tp, row_begin + i);
             }
             phase_sync(&phase_bar, pph);
@@ -767,7 +768,7 @@ k_qmlp2(const MlpParams p_in, const TreeParams tp, const int n_sims, const int c
             for (int i = tid; i < nrows; i += Q2_EPI_THREADS) {
                 const int gr = row_begin + i;
                 if constexpr (ENV::DISCRETE) {
-                    d_step(tp, tabs, gr, s > 0, s + 1 < n_evals);
+                    d_step<ENV>(tp, tabs, gr, s > 0, s + 1 < n_evals);
                 } else {
                     if (s == 0) c_root_insert(tp, gr);                // the add_pw_action(root) before the loop (mcts.py:673)
                     c_step<ENV>(tp, tabs, gr, s > 0, s + 1 < n_evals);  // backup of simulation s, descent + expansion of simulation s + 1

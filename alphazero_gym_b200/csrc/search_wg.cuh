@@ -375,7 +375,7 @@ k_search_wg(const MlpParams p, const TreeParams tp, const int n_sims, const int 
         for (int rd = 0; rd < rounds; ++rd) {
             const int tile = 4 * rd + g, row0 = row_begin + tile * th;
             if (tile < ntiles && row0 + r < min(row0 + th, row_end)) {
-                if constexpr (ENV::DISCRETE) d_init(tp, row0 + r);
+                if constexpr (ENV::DISCRETE) d_init<ENV>(tp, row0 + r);
                 else c_init<ENV>(tp, row0 + r);
             }
         }
@@ -419,12 +419,12 @@ k_search_wg(const MlpParams p, const TreeParams tp, const int n_sims, const int 
                     leafw = p.leaf[gr];
                 }
                 if (leafw & LEAF_EVAL) {
-                    mlp_finish_row(p, gr, leafw, lr, out[0], out + 1);
+                    mlp_finish_row<env::row3<ENV>()>(p, gr, leafw, lr, out[0], out + 1);
                     ++nev;
                     ev_row = gr;
                 }
                 if constexpr (ENV::DISCRETE) {
-                    d_step(tp, tabs, gr, s > 0, s + 1 < n_evals);
+                    d_step<ENV>(tp, tabs, gr, s > 0, s + 1 < n_evals);
                 } else {
                     if (s == 0) c_root_insert(tp, gr);             // the add_pw_action(root) before the loop (mcts.py:673)
                     c_step<ENV>(tp, tabs, gr, s > 0, s + 1 < n_evals);  // backup of simulation s, descent + expansion of simulation s + 1

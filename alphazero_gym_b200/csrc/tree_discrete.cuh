@@ -19,46 +19,84 @@ __device__ __forceinline__ DRow load_drow(const DRow* p) {
     d[0] = s[0]; d[1] = s[1]; d[2] = s[2]; d[3] = s[3];
     return r;
 }
+__device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
+// line 0 of a three-action row: everything the descent reads
+__device__ __forceinline__ void load_line0(D3Row* r, const D3Row* p) {
+    const uint4* s = reinterpret_cast<const uint4*>(p);
+    uint4* d = reinterpret_cast<uint4*>(r);
+    d[0] = s[0]; d[1] = s[1]; d[2] = s[2]; d[3] = s[3];
+}
+
+// a fresh three-action row: no edges visited, no children
+__device__ __forceinline__ D3Row d3_row(uint16_t parent, int paction, double r, bool term) {
+    D3Row nr;
+    memset(&nr, 0, sizeof nr);
+    nr.child[0] = nr.child[1] = nr.child[2] = DROW_NONE;
+    nr.flags = term ? ROW_TERMINAL : 0;
+    nr.r = r;
+    nr.parent = parent;
+    nr.paction = (uint8_t)paction;
+    return nr;
+}
 
 // root row + first network input (MCTSDiscrete.initialize_search, mcts.py:364-383)
+template <class ENV>
 __device__ __forceinline__ void d_init(const TreeParams& p, int t) {
-    const double* s = p.root_state + (size_t)t * 4;
+    const double* s = p.root_state + (size_t)t * ENV::S;  // the root's hidden state (MountainCar: the observation is the state)
     double* st = p.dstate + (size_t)t * p.R * 4;
-    DRow row;
-    row.W[0] = row.W[1] = 0.0;
-    row.r = 0.0;
-    row.n_e[0] = row.n_e[1] = 0;
-    row.prior[0] = row.prior[1] = 0.0f;
-    row.V = 0.0f;
-    row.node_n = p.root_n_init ? p.root_n_init[t] : 0;
-    row.child[0] = row.child[1] = DROW_NONE;
-    row.parent = DROW_NONE;
-    row.paction = 0;
-    row.flags = 0;
-    row.pad[0] = row.pad[1] = 0;
-    if (p.use_tape) {
-        row.V = p.tapeV[(size_t)t * p.R];
-        row.prior[0] = p.tapeP[(size_t)t * p.R * 2];
-        row.prior[1] = p.tapeP[(size_t)t * p.R * 2 + 1];
+    if constexpr (ENV::A == 2) {
+        DRow row;
+        row.W[0] = row.W[1] = 0.0;
+        row.r = 0.0;
+        row.n_e[0] = row.n_e[1] = 0;
+        row.prior[0] = row.prior[1] = 0.0f;
+        row.V = 0.0f;
+        row.node_n = p.root_n_init ? p.root_n_init[t] : 0;
+        row.child[0] = row.child[1] = DROW_NONE;
+        row.parent = DROW_NONE;
+        row.paction = 0;
+        row.flags = 0;
+        row.pad[0] = row.pad[1] = 0;
+        if (p.use_tape) {
+            row.V = p.tapeV[(size_t)t * p.R];
+            row.prior[0] = p.tapeP[(size_t)t * p.R * 2];
+            row.prior[1] = p.tapeP[(size_t)t * p.R * 2 + 1];
+        }
+        p.drows[(size_t)t * p.R] = row;
+        st[0] = s[0]; st[1] = s[1]; st[2] = s[2]; st[3] = s[3];
+        p.X[t] = make_float4((float)s[0], (float)s[1], (float)s[2], (float)s[3]);
+    } else {
+        D3Row row = d3_row(DROW_NONE, 0, 0.0, false);
+        row.node_n = p.root_n_init ? p.root_n_init[t] : 0;
+        if (p.use_tape) {
+            row.V = p.tapeV[(size_t)t * p.R];
+            for (int k = 0; k < 3; ++k) row.prior[k] = p.tapeP[(size_t)t * p.R * 3 + k];
+        }
+        reinterpret_cast<D3Row*>(p.drows)[(size_t)t * p.R] = row;
+        st[0] = s[0]; st[1] = s[1];
+        p.X[t] = ENV::obs(s[0], s[1]);
     }
-    p.drows[(size_t)t * p.R] = row;
-    st[0] = s[0]; st[1] = s[1]; st[2] = s[2]; st[3] = s[3];
-    p.X[t] = make_float4((float)s[0], (float)s[1], (float)s[2], (float)s[3]);
     p.leaf[t] = 0 | LEAF_EVAL;
     p.n_rows[t] = 1;
     p.draws[t] = 0;
     if (p.rng_mt) mt_seed_dev(p.mt + (size_t)t * (MT_N + 1), __ldg(p.seedp) + (uint64_t)(tree_base(p) + t));  // random.seed(seed + tree)
     for (int k = 0; k < 4; ++k) p.ctr[(size_t)k * p.B + t] = 0;
 }
+template <class ENV>
 __global__ void k_init_discrete(const TreeParams p) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t < p.B) d_init(p, t);
+    if (t < p.B) d_init<ENV>(p, t);
 }
 
 // one simulation step of tree t: backup of the previous simulation (BACKUP), then descent + expansion of the next (SELECT).
-// Shared by k_step_discrete (one launch per simulation) and the whole-search kernel (qmlp2.cuh, FUSED).
+// Shared by k_step_discrete (one launch per simulation) and the whole-search kernels (qmlp2.cuh, search_wg.cuh).
+// ENV::A = 2 (CartPole): DRow, path entries (row << 1 | action).  ENV::A = 3 (MountainCar): D3Row, path entries (row << 2 | action);
+// the descent reads line 0 of a row, the backup also reads r from line 1.
+template <class ENV>
 __device__ __forceinline__ void d_step(const TreeParams& p, const Tabs& tb, int t, const bool BACKUP, const bool SELECT) {
+    constexpr int A = ENV::A, PSH = A == 2 ? 1 : 2;  // path entry: row << PSH | action
     DRow* rows = p.drows + (size_t)t * p.R;
+    D3Row* rows3 = reinterpret_cast<D3Row*>(p.drows) + (size_t)t * p.R;
 
     uint16_t* path = p.dpath + (size_t)t * p.R;
     TP_BEGIN();
@@ -70,30 +108,60 @@ __device__ __forceinline__ void d_step(const TreeParams& p, const Tabs& tb, int 
         const int leaf = p.leaf[t] & LEAF_ROW_MASK;
         const int d = p.ddepth[t];
         double Rv, r;
-        {
+        if constexpr (A == 2) {
             const DRow lr = load_drow(rows + leaf);
             Rv = (double)lr.V;
             r = lr.r;
+        } else {
+            Rv = (double)rows3[leaf].V;
+            r = rows3[leaf].r;
         }
 #pragma unroll 1
         for (int base = d - 1; base >= 0; base -= 4) {
-            DRow q[4];
-            int pe[4];
+            if constexpr (A == 2) {
+                DRow q[4];
+                int pe[4];
 #pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                pe[k] = base - k >= 0 ? (int)path[base - k] : 0;
-                q[k] = load_drow(rows + (pe[k] >> 1));
-            }
+                for (int k = 0; k < 4; ++k) {
+                    pe[k] = base - k >= 0 ? (int)path[base - k] : 0;
+                    q[k] = load_drow(rows + (pe[k] >> 1));
+                }
 #pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                if (base - k >= 0) {
-                    DRow* pr = rows + (pe[k] >> 1);
-                    const int pa = pe[k] & 1;
-                    Rv = r + p.gamma * Rv;
-                    pr->W[pa] = (pa ? q[k].W[1] : q[k].W[0]) + Rv;
-                    pr->n_e[pa] = (pa ? q[k].n_e[1] : q[k].n_e[0]) + 1;
-                    pr->node_n = q[k].node_n + 1;
-                    r = q[k].r;
+                for (int k = 0; k < 4; ++k) {
+                    if (base - k >= 0) {
+                        DRow* pr = rows + (pe[k] >> 1);
+                        const int pa = pe[k] & 1;
+                        Rv = r + p.gamma * Rv;
+                        pr->W[pa] = (pa ? q[k].W[1] : q[k].W[0]) + Rv;
+                        pr->n_e[pa] = (pa ? q[k].n_e[1] : q[k].n_e[0]) + 1;
+                        pr->node_n = q[k].node_n + 1;
+                        r = q[k].r;
+                    }
+                }
+            } else {  // only the four words the backup touches per level: the edge's W and n, node.n (line 0) and r (line 1)
+                double qW[4], qr[4];
+                int qn[4], qnn[4], pe[4];
+#pragma unroll
+                for (int k = 0; k < 4; ++k) {
+                    pe[k] = base - k >= 0 ? (int)path[base - k] : 0;
+                    const D3Row* q = rows3 + (pe[k] >> 2);
+                    const int pa = pe[k] & 3;
+                    qW[k] = q->W[pa];
+                    qn[k] = q->n_e[pa];
+                    qnn[k] = q->node_n;
+                    qr[k] = q->r;
+                }
+#pragma unroll
+                for (int k = 0; k < 4; ++k) {
+                    if (base - k >= 0) {
+                        D3Row* pr = rows3 + (pe[k] >> 2);
+                        const int pa = pe[k] & 3;
+                        Rv = r + p.gamma * Rv;
+                        pr->W[pa] = qW[k] + Rv;
+                        pr->n_e[pa] = qn[k] + 1;
+                        pr->node_n = qnn[k] + 1;
+                        r = qr[k];
+                    }
                 }
             }
         }
@@ -104,7 +172,11 @@ __device__ __forceinline__ void d_step(const TreeParams& p, const Tabs& tb, int 
         const int64_t tree = tree_base(p) + t;
         int draws = p.draws[t];
         int cur = 0;
-        DRow row = load_drow(rows);
+        // the node being descended: a DRow, or line 0 of a D3Row
+        DRow row;
+        D3Row row3;
+        if constexpr (A == 2) row = load_drow(rows);
+        else load_line0(&row3, rows3);
         int a = -1;
         uint32_t levels = 0;
         uint32_t xr[4] = {0, 0, 0, 0};
@@ -112,27 +184,37 @@ __device__ __forceinline__ void d_step(const TreeParams& p, const Tabs& tb, int 
         int mti = p.rng_mt ? (int)mt[MT_N] : 0;
         bool nan = false;
         while (true) {
-            // both children are LOADED while the scores are computed (32 registers): the level costs max(round trip, arithmetic)
-            // instead of their sum, and the next level's children are requested the moment the choice is made
-            const int c0 = row.child[0], c1 = row.child[1];
+            // CartPole: both children are LOADED while the scores are computed (32 registers): the level costs max(round trip,
+            // arithmetic) instead of their sum, and the next level's children are requested the moment the choice is made.
+            // MountainCar: holding line 0 of three children (48 registers) spilled in the warpgroup kernel (search_wg.cuh), so the
+            // three lines are prefetched into L2 instead and only the chosen one is loaded
             uint4 k0[4], k1[4];
-            {
+            int c0, c1, c2 = DROW_NONE;
+            if constexpr (A == 2) {
+                c0 = row.child[0], c1 = row.child[1];
                 const uint4* s0 = reinterpret_cast<const uint4*>(rows + (c0 != DROW_NONE ? c0 : cur));
                 const uint4* s1 = reinterpret_cast<const uint4*>(rows + (c1 != DROW_NONE ? c1 : cur));
 #pragma unroll
                 for (int q = 0; q < 4; ++q) { k0[q] = s0[q]; k1[q] = s1[q]; }
+            } else {
+                c0 = row3.child[0], c1 = row3.child[1], c2 = row3.child[2];
+                if (c0 != DROW_NONE) prefetch_l2(rows3 + c0);
+                if (c1 != DROW_NONE) prefetch_l2(rows3 + c1);
+                if (c2 != DROW_NONE) prefetch_l2(rows3 + c2);
             }
             // UCT_a = Q_a + prior_a*c_uct*(sqrt(node.n+1)/(n_a+1))   (mcts.py:483-484)
-            const double sq = sqrt_small(row.node_n + 1, tb.sq, tb.n);
-            double u[2];
+            const double sq = sqrt_small((A == 2 ? row.node_n : row3.node_n) + 1, tb.sq, tb.n);
+            double u[A];
 #pragma unroll
-            for (int i = 0; i < 2; ++i) {
-                const int n = row.n_e[i];
-                const double Q = n > 0 ? div_small(row.W[i], n, tb.rcp, tb.n) : (double)row.V;
-                const double pc = p.puct_f32 ? (double)__fmul_rn(row.prior[i], (float)p.c_uct) : (double)row.prior[i] * p.c_uct;
+            for (int i = 0; i < A; ++i) {
+                const int n = A == 2 ? row.n_e[i] : row3.n_e[i];
+                const double Q = n > 0 ? div_small(A == 2 ? row.W[i] : row3.W[i], n, tb.rcp, tb.n) : (double)(A == 2 ? row.V : row3.V);
+                const float pr = A == 2 ? row.prior[i] : row3.prior[i];
+                const double pc = p.puct_f32 ? (double)__fmul_rn(pr, (float)p.c_uct) : (double)pr * p.c_uct;
                 u[i] = Q + pc * div_small(sq, n + 1, tb.rcp, tb.n);
             }
-            nan |= (u[0] != u[0]) || (u[1] != u[1]);
+            if constexpr (A == 2) nan |= (u[0] != u[0]) || (u[1] != u[1]);
+            else nan |= (u[0] != u[0]) || (u[1] != u[1]) || (u[2] != u[2]);
 #ifdef AZG_TREE_PROF
             if (u[0] + u[1] == 12345.678) atomicOr(p.err, 0);  // (profiling builds: the scores are complete before the stamp)
             TP_STAMP(5);
@@ -150,36 +232,59 @@ __device__ __forceinline__ void d_step(const TreeParams& p, const Tabs& tb, int 
                 const double x = (double)u32_to_unit(xk);
                 random_pick = x < p.epsilon;
             }
-            if (p.rng_mt) {  // randint(0, 1), or choice over the 1 or 2 winners (which also draws for a single winner)
-                if (random_pick) a = mt_below_dev(mt, mti, draws, 2);
-                else if (u[0] == u[1]) a = mt_below_dev(mt, mti, draws, 2);
-                else { (void)mt_below_dev(mt, mti, draws, 1); a = u[1] > u[0] ? 1 : 0; }
-            } else if (random_pick) {
-                a = u32_to_index(rng_select_u32(p, tree, draws++), 2);
+            if constexpr (A == 2) {
+                if (p.rng_mt) {  // randint(0, 1), or choice over the 1 or 2 winners (which also draws for a single winner)
+                    if (random_pick) a = mt_below_dev(mt, mti, draws, 2);
+                    else if (u[0] == u[1]) a = mt_below_dev(mt, mti, draws, 2);
+                    else { (void)mt_below_dev(mt, mti, draws, 1); a = u[1] > u[0] ? 1 : 0; }
+                } else if (random_pick) {
+                    a = u32_to_index(rng_select_u32(p, tree, draws++), 2);
+                } else {
+                    // argmax with random tie-break: one draw is consumed even for a single winner
+                    if (u[0] == u[1]) a = u32_to_index(rng_select_u32(p, tree, draws), 2);
+                    else a = u[1] > u[0] ? 1 : 0;
+                    ++draws;
+                }
             } else {
-                // argmax with random tie-break: one draw is consumed even for a single winner
-                if (u[0] == u[1]) a = u32_to_index(rng_select_u32(p, tree, draws), 2);
-                else a = u[1] > u[0] ? 1 : 0;
-                ++draws;
+                // helpers.argmax: winners = the indices of max(u) in ascending order; random.choice(winners), one draw even for a
+                // single winner (a NaN score leaves no winner: ERR_NAN is raised and the pick is immaterial)
+                double m = u[0];
+                m = u[1] > m ? u[1] : m;
+                m = u[2] > m ? u[2] : m;
+                const int w0 = u[0] == m, w1 = u[1] == m, nw = w0 + w1 + (u[2] == m);
+                int pick = 0;
+                if (p.rng_mt) {  // randint(0, 2) / CPython's _randbelow(n_winners)
+                    if (random_pick) a = mt_below_dev(mt, mti, draws, 3);
+                    else pick = mt_below_dev(mt, mti, draws, nw > 0 ? nw : 1);
+                } else if (random_pick) {
+                    a = u32_to_index(rng_select_u32(p, tree, draws++), 3);
+                } else {
+                    if (nw > 1) pick = u32_to_index(rng_select_u32(p, tree, draws), nw);
+                    ++draws;
+                }
+                if (!random_pick) a = (w0 && pick == 0) ? 0 : ((w1 && pick == w0) ? 1 : 2);
             }
 #ifdef AZG_TREE_PROF
             if (a == 77) atomicOr(p.err, 0);
             TP_STAMP(6);
             if ((threadIdx.x & 31) == 0 && p.prof) atomicAdd(p.prof + 7, 1ull);
 #endif
-            path[levels] = (uint16_t)((cur << 1) | a);
+            path[levels] = (uint16_t)((cur << PSH) | a);
             ++levels;
-            const int child = a ? c1 : c0;
+            const int child = A == 2 ? (a ? c1 : c0) : (a == 0 ? c0 : (a == 1 ? c1 : c2));
             if (child == DROW_NONE) break;  // expansion
             cur = child;
-            {
+            if constexpr (A == 2) {
                 uint4* d = reinterpret_cast<uint4*>(&row);
 #pragma unroll
                 for (int q = 0; q < 4; ++q) d[q] = a ? k1[q] : k0[q];
+                if (row.flags & ROW_TERMINAL) { a = -1; break; }  // trace ends on an existing terminal node
+            } else {
+                load_line0(&row3, rows3 + child);
+                if (row3.flags & ROW_TERMINAL) { a = -1; break; }
             }
-            if (row.flags & ROW_TERMINAL) { a = -1; break; }  // trace ends on an existing terminal node
 #ifdef AZG_TREE_PROF
-            if (row.node_n == -77) atomicOr(p.err, 0);  // (the next row has arrived)
+            if ((A == 2 ? row.node_n : row3.node_n) == -77) atomicOr(p.err, 0);  // (the next row has arrived)
             TP_STAMP(3);
 #endif
         }
@@ -189,39 +294,56 @@ __device__ __forceinline__ void d_step(const TreeParams& p, const Tabs& tb, int 
         p.ddepth[t] = (int)levels;  // edges between the root and the leaf (the new node, or the existing terminal node the trace ended on)
         p.draws[t] = draws;
         p.ctr[t] += levels;
-        p.ctr[(size_t)p.B + t] += levels * 2;
+        p.ctr[(size_t)p.B + t] += levels * A;
         if (a >= 0) {
             const int child = p.n_rows[t];
             if (child >= p.R) { atomicOr(p.err, ERR_CAPACITY); p.leaf[t] = cur; return; }
             p.n_rows[t] = child + 1;
             double* st = p.dstate + ((size_t)t * p.R + cur) * 4;
-            const double s[4] = {st[0], st[1], st[2], st[3]};
-            double o[4], rew;
-            const bool term = env::cartpole_step(s, a, o, rew);
-            rew = term ? p.reward_terminal : p.reward_step;  // rl/wrappers.py (1.0 / 1.0 without wrappers)
-            double* so = p.dstate + ((size_t)t * p.R + child) * 4;
-            so[0] = o[0]; so[1] = o[1]; so[2] = o[2]; so[3] = o[3];
-            DRow nr;
-            nr.W[0] = nr.W[1] = 0.0;
-            nr.r = rew;
-            nr.n_e[0] = nr.n_e[1] = 0;
-            nr.prior[0] = nr.prior[1] = 0.0f;
-            nr.V = 0.0f;
-            nr.node_n = 0;
-            nr.child[0] = nr.child[1] = DROW_NONE;
-            nr.parent = (uint16_t)cur;
-            nr.paction = (uint8_t)a;
-            nr.flags = term ? ROW_TERMINAL : 0;
-            nr.pad[0] = nr.pad[1] = 0;
-            if (p.use_tape) {
-                const size_t ti = (size_t)t * p.R + child;
-                nr.V = term ? 0.0f : p.tapeV[ti];
-                nr.prior[0] = p.tapeP[ti * 2];
-                nr.prior[1] = p.tapeP[ti * 2 + 1];
+            bool term;
+            if constexpr (A == 2) {
+                const double s[4] = {st[0], st[1], st[2], st[3]};
+                double o[4], rew;
+                term = env::cartpole_step(s, a, o, rew);
+                rew = term ? p.reward_terminal : p.reward_step;  // rl/wrappers.py (1.0 / 1.0 without wrappers)
+                double* so = p.dstate + ((size_t)t * p.R + child) * 4;
+                so[0] = o[0]; so[1] = o[1]; so[2] = o[2]; so[3] = o[3];
+                DRow nr;
+                nr.W[0] = nr.W[1] = 0.0;
+                nr.r = rew;
+                nr.n_e[0] = nr.n_e[1] = 0;
+                nr.prior[0] = nr.prior[1] = 0.0f;
+                nr.V = 0.0f;
+                nr.node_n = 0;
+                nr.child[0] = nr.child[1] = DROW_NONE;
+                nr.parent = (uint16_t)cur;
+                nr.paction = (uint8_t)a;
+                nr.flags = term ? ROW_TERMINAL : 0;
+                nr.pad[0] = nr.pad[1] = 0;
+                if (p.use_tape) {
+                    const size_t ti = (size_t)t * p.R + child;
+                    nr.V = term ? 0.0f : p.tapeV[ti];
+                    nr.prior[0] = p.tapeP[ti * 2];
+                    nr.prior[1] = p.tapeP[ti * 2 + 1];
+                }
+                rows[child] = nr;
+                rows[cur].child[a] = (uint16_t)child;
+                p.X[t] = make_float4((float)o[0], (float)o[1], (float)o[2], (float)o[3]);
+            } else {
+                double o0, o1, rew;
+                term = ENV::step(st[0], st[1], a, o0, o1, rew);  // Node.r = the env's reward
+                double* so = p.dstate + ((size_t)t * p.R + child) * 4;
+                so[0] = o0; so[1] = o1;
+                D3Row nr = d3_row((uint16_t)cur, a, rew, term);
+                if (p.use_tape) {
+                    const size_t ti = (size_t)t * p.R + child;
+                    nr.V = term ? 0.0f : p.tapeV[ti];
+                    for (int k = 0; k < 3; ++k) nr.prior[k] = p.tapeP[ti * 3 + k];
+                }
+                rows3[child] = nr;
+                rows3[cur].child[a] = (uint16_t)child;
+                p.X[t] = ENV::obs(o0, o1);
             }
-            rows[child] = nr;
-            rows[cur].child[a] = (uint16_t)child;
-            p.X[t] = make_float4((float)o[0], (float)o[1], (float)o[2], (float)o[3]);
             p.leaf[t] = child | LEAF_EVAL | (term ? LEAF_TERMINAL : 0);
         } else {
             p.leaf[t] = cur;
@@ -231,11 +353,11 @@ __device__ __forceinline__ void d_step(const TreeParams& p, const Tabs& tb, int 
     }
 }
 
-template <bool BACKUP, bool SELECT>
+template <class ENV, bool BACKUP, bool SELECT>
 __global__ void __launch_bounds__(128) k_step_discrete(const TreeParams p) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     const Tabs tb = {p.pw_table, p.rcp_tab, p.sqrt_tab, AZG_TAB};
-    if (t < p.B) d_step(p, tb, t, BACKUP, SELECT);
+    if (t < p.B) d_step<ENV>(p, tb, t, BACKUP, SELECT);
 }
 
 // ---- shared-memory-resident trees (whole-search kernel, thin batches: qmlp2.cuh TSM) -----------------------------------------------
@@ -634,28 +756,55 @@ __device__ __forceinline__ void ds_writeback(const TreeParams& p, const SmTrees&
 }
 
 // MCTS.return_results (mcts.py:269-307) for the discrete root
+template <class ENV>
 __global__ void k_results_discrete(const TreeParams p, int cmax, float* actions, int32_t* counts, double* Q, double* Vt,
                                    int32_t* nchild) {
+    constexpr int A = ENV::A;
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= p.B) return;
-    const DRow row = load_drow(p.drows + (size_t)t * p.R);
-    double q[2];
-    for (int a = 0; a < 2; ++a) {
-        const int n = row.n_e[a];
-        q[a] = n > 0 ? row.W[a] / (double)n : (double)row.V;
-        actions[(size_t)t * cmax + a] = (float)a;
-        counts[(size_t)t * cmax + a] = n;
-        Q[(size_t)t * cmax + a] = q[a];
-    }
-    nchild[t] = 2;
-    double v;
-    if (p.v_target == 1) {  // on_policy: np.sum((counts / np.sum(counts)) * Q), n < 8 -> sequential sum from 0.
-        const double tot = (double)(row.n_e[0] + row.n_e[1]);
-        v = 0.0;
-        v += ((double)row.n_e[0] / tot) * q[0];
-        v += ((double)row.n_e[1] / tot) * q[1];
+    if constexpr (A == 2) {
+        const DRow row = load_drow(p.drows + (size_t)t * p.R);
+        double q[2];
+        for (int a = 0; a < 2; ++a) {
+            const int n = row.n_e[a];
+            q[a] = n > 0 ? row.W[a] / (double)n : (double)row.V;
+            actions[(size_t)t * cmax + a] = (float)a;
+            counts[(size_t)t * cmax + a] = n;
+            Q[(size_t)t * cmax + a] = q[a];
+        }
+        nchild[t] = 2;
+        double v;
+        if (p.v_target == 1) {  // on_policy: np.sum((counts / np.sum(counts)) * Q), n < 8 -> sequential sum from 0.
+            const double tot = (double)(row.n_e[0] + row.n_e[1]);
+            v = 0.0;
+            v += ((double)row.n_e[0] / tot) * q[0];
+            v += ((double)row.n_e[1] / tot) * q[1];
+        } else {
+            v = q[1] > q[0] ? q[1] : q[0];
+        }
+        Vt[t] = v;
     } else {
-        v = q[1] > q[0] ? q[1] : q[0];
+        D3Row row;
+        load_line0(&row, reinterpret_cast<const D3Row*>(p.drows) + (size_t)t * p.R);
+        double q[A];
+        for (int a = 0; a < A; ++a) {
+            const int n = row.n_e[a];
+            q[a] = n > 0 ? row.W[a] / (double)n : (double)row.V;
+            actions[(size_t)t * cmax + a] = (float)a;
+            counts[(size_t)t * cmax + a] = n;
+            Q[(size_t)t * cmax + a] = q[a];
+        }
+        nchild[t] = A;
+        double v;
+        if (p.v_target == 1) {  // on_policy: np.sum((counts / np.sum(counts)) * Q), n < 8 -> sequential sum from 0.
+            int tot = 0;
+            for (int a = 0; a < A; ++a) tot += row.n_e[a];
+            v = 0.0;
+            for (int a = 0; a < A; ++a) v += ((double)row.n_e[a] / (double)tot) * q[a];
+        } else {  // Q.max()
+            v = q[0];
+            for (int a = 1; a < A; ++a) v = q[a] > v ? q[a] : v;
+        }
+        Vt[t] = v;
     }
-    Vt[t] = v;
 }

@@ -15,8 +15,9 @@ import torch
 from . import _cabi
 from ._cabi import ACT_ELU, ACT_RELU, CONTINUOUS, DISCRETE, VT, AzgConfig, check
 
-# the envs the engine steps (gym ids); the continuous search steps Pendulum-v0 unless told otherwise
+# the envs the engine steps (gym ids); the discrete search steps CartPole-v0 and the continuous search Pendulum-v0 unless told otherwise
 CARTPOLE, PENDULUM, MOUNTAIN_CAR_CONTINUOUS = "CartPole-v0", "Pendulum-v0", "MountainCarContinuous-v0"
+MOUNTAIN_CAR = "MountainCar-v0"
 
 
 @dataclass
@@ -52,7 +53,8 @@ class EngineConfig:
     rng_mt19937: bool = False  # AZG_FLAG_RNG_MT19937: CPython's generator for the discrete search's selection draws (include/azg.h)
     fused: Optional[bool] = None  # AZG_FLAG_FUSED: whole search in one persistent kernel; None = on where supported (eval_q8)
     # the env the search steps: None = the variant's own (CartPole-v0 / Pendulum-v0); MOUNTAIN_CAR_CONTINUOUS (continuous variant,
-    # state_dim 2) sets AZG_FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS
+    # state_dim 2) sets AZG_FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS; MOUNTAIN_CAR (discrete variant, num_actions 3, state_dim 2) sets
+    # AZG_FLAG_ENV_MOUNTAIN_CAR
     env: Optional[str] = None
 
     def c(self) -> AzgConfig:
@@ -62,13 +64,17 @@ class EngineConfig:
                          self.action_bound, self.log_std_min, self.log_std_max,
                          (0 if self.use_graph else _cabi.FLAG_NO_GRAPH) | (_cabi.FLAG_EVAL_Q8 if self.is_q8() else 0)
                          | (_cabi.FLAG_FUSED if self.is_fused() else 0) | (_cabi.FLAG_RNG_MT19937 if self.rng_mt19937 else 0)
-                         | (_cabi.FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS if self.env_name() == MOUNTAIN_CAR_CONTINUOUS else 0), self.seed)
+                         | (_cabi.FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS if self.env_name() == MOUNTAIN_CAR_CONTINUOUS else 0)
+                         | (_cabi.FLAG_ENV_MOUNTAIN_CAR if self.env_name() == MOUNTAIN_CAR else 0), self.seed)
 
     def env_name(self) -> str:
         if self.env is None:
             return CARTPOLE if self.variant == DISCRETE else PENDULUM
-        if self.env not in (CARTPOLE, PENDULUM, MOUNTAIN_CAR_CONTINUOUS):
-            raise ValueError(f"unknown env {self.env!r}: the engine steps {CARTPOLE}, {PENDULUM} and {MOUNTAIN_CAR_CONTINUOUS}")
+        if self.env not in (CARTPOLE, PENDULUM, MOUNTAIN_CAR_CONTINUOUS, MOUNTAIN_CAR):
+            raise ValueError(f"unknown env {self.env!r}: the engine steps {CARTPOLE}, {MOUNTAIN_CAR}, {PENDULUM} and "
+                             f"{MOUNTAIN_CAR_CONTINUOUS}")
+        if self.env == MOUNTAIN_CAR and self.variant != DISCRETE:
+            raise ValueError(f"{MOUNTAIN_CAR} has discrete actions: it is searched by the discrete variant")
         return self.env
 
     def q8_supported(self) -> bool:
@@ -79,7 +85,7 @@ class EngineConfig:
         return self.q8_supported() if self.eval_q8 is None else bool(self.eval_q8)
 
     def is_fused(self) -> bool:
-        env_dim = {CARTPOLE: 4, PENDULUM: 3, MOUNTAIN_CAR_CONTINUOUS: 2}[self.env_name()]
+        env_dim = {CARTPOLE: 4, PENDULUM: 3, MOUNTAIN_CAR_CONTINUOUS: 2, MOUNTAIN_CAR: 2}[self.env_name()]
         supported = (self.is_q8() and self.state_dim == env_dim
                      and not (self.rng_mt19937 and self.variant == CONTINUOUS))  # the torch-generator mode runs one launch per simulation
         return supported if self.fused is None else bool(self.fused)
@@ -115,7 +121,7 @@ class SearchEngine:
         self.cmax = self._lib.azg_cmax(h)
         self.head_dim = self._lib.azg_head_dim(h)
         self.num_weights = self._lib.azg_num_weights(h)
-        self.state_cols = 4 if cfg.variant == DISCRETE else 2
+        self.state_cols = 4 if cfg.variant == DISCRETE and cfg.env_name() == CARTPOLE else 2  # hidden-state width
         self._keep = {}
         self.last_B = 0
 
@@ -151,7 +157,7 @@ class SearchEngine:
     # ---- device-resident path ------------------------------------------------------------------------
     def search(self, root_state: torch.Tensor, n_rollouts: int, root_n_init: Optional[torch.Tensor] = None,
                tree_id0: int = 0) -> None:
-        """Batched search; root_state is a CUDA f64 tensor [B, 4|2].  Asynchronous on the current stream."""
+        """Batched search; root_state is a CUDA f64 tensor [B, 4|2] (CartPole 4, the other envs 2).  Asynchronous on the current stream."""
         assert root_state.is_cuda and root_state.dtype == torch.float64 and root_state.is_contiguous()
         B = root_state.shape[0]
         assert root_state.shape[1] == self.state_cols
@@ -265,7 +271,7 @@ class SearchEngine:
         if self.cfg.variant == DISCRETE:
             d = dict(n_nodes=np.zeros(B, np.int32), parent=np.zeros((B, R), np.int32), paction=np.zeros((B, R), np.int32),
                      node_n=np.zeros((B, R), np.int32), terminal=np.zeros((B, R), np.int32), V=np.zeros((B, R), np.float32),
-                     r=np.zeros((B, R), np.float64), state=np.zeros((B, R, 4), np.float64),
+                     r=np.zeros((B, R), np.float64), state=np.zeros((B, R, self.state_cols), np.float64),
                      prior=np.zeros((B, R, A), np.float32), eW=np.zeros((B, R, A), np.float64),
                      en=np.zeros((B, R, A), np.int32), echild=np.zeros((B, R, A), np.int32))
             s = _cabi.DumpDiscrete(*[d[n].ctypes.data for n in _cabi.DumpDiscrete.FIELDS])

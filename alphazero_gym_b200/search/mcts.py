@@ -8,7 +8,7 @@ upstream call form `search(n_mcts, c, Env, mcts_env)` named in BASELINE.json is 
 What changes underneath: the tree lives in HBM tables and the whole search -- select, env step, network
 evaluation, backup -- runs in the CUDA engine (csrc/, C ABI include/azg.h).  `model` is only read for its
 weights and shape; `Env` only for its hidden state (`Env.unwrapped.state`) and its class name.  Envs other than
-CartPole (MCTSDiscrete), Pendulum and MountainCarContinuous (MCTSContinuous) raise: there is no CPU fallback.  Tie-break / epsilon-greedy / action-noise randomness comes from
+CartPole and MountainCar (MCTSDiscrete), Pendulum and MountainCarContinuous (MCTSContinuous) raise: there is no CPU fallback.  Tie-break / epsilon-greedy / action-noise randomness comes from
 the engine's counter-based Philox streams keyed by (`seed`, search counter) instead of Python's `random` and
 torch's global generator.
 
@@ -22,7 +22,7 @@ from typing import Any, Dict, Optional, Tuple
 import numpy as np
 
 from .._cabi import CONTINUOUS, DISCRETE
-from ..engine import MOUNTAIN_CAR_CONTINUOUS, PENDULUM, EngineConfig, SearchEngine, flatten_state_dict
+from ..engine import CARTPOLE, MOUNTAIN_CAR, MOUNTAIN_CAR_CONTINUOUS, PENDULUM, EngineConfig, SearchEngine, flatten_state_dict
 from ..network import describe_model, weights_version
 
 PENDULUM_R_SCALE = 16.2736044  # reference mcts.py:20 (applied inside the engine)
@@ -64,6 +64,8 @@ def reward_model(env, variant: int):
     base, names = _wrapper_chain(env)
     if names and variant != DISCRETE and _is_mountain_car_continuous(base):
         raise NotImplementedError(f"{names[0]} around MountainCarContinuous-v0: the CUDA engine steps the plain env only")
+    if names and variant == DISCRETE and _is_mountain_car(base):
+        raise NotImplementedError(f"{names[0]} around MountainCar-v0: the CUDA engine steps the plain env only")
     step, terminal = 1.0, 1.0  # gym CartPole-v0 pays 1.0 for every step, the terminating one included
     for name in reversed(names):
         if name == "ReparametrizeWrapper":
@@ -81,18 +83,35 @@ def _is_mountain_car_continuous(base) -> bool:
     return type(base).__name__ == "Continuous_MountainCarEnv"  # gym's class (classic_control/continuous_mountain_car.py)
 
 
+def _is_mountain_car(base) -> bool:
+    return type(base).__name__ == "MountainCarEnv"  # gym's class (classic_control/mountain_car.py)
+
+
+def discrete_env(env) -> str:
+    """The env MCTSDiscrete has the engine step for `env`: MountainCar-v0 for gym's MountainCarEnv (by class name, under any
+    wrappers), CartPole-v0 otherwise (env_hidden_state refuses the envs that are neither)."""
+    return MOUNTAIN_CAR if _is_mountain_car(_unwrap(env)) else CARTPOLE
+
+
 def continuous_env(env) -> str:
     """The env MCTSContinuous has the engine step for `env`: MountainCarContinuous-v0 for gym's Continuous_MountainCarEnv (by class
     name, under any wrappers), Pendulum-v0 otherwise (env_hidden_state refuses the envs that are neither)."""
     return MOUNTAIN_CAR_CONTINUOUS if _is_mountain_car_continuous(_unwrap(env)) else PENDULUM
 
 
-def env_hidden_state(env, variant: int) -> np.ndarray:
-    """Root of the search = hidden state of the gym env (replaces copy.deepcopy(Env), mcts.py:443, :680)."""
+def env_hidden_state(env, variant: int, env_id: Optional[str] = None) -> np.ndarray:
+    """Root of the search = hidden state of the gym env (replaces copy.deepcopy(Env), mcts.py:443, :680).  env_id = MOUNTAIN_CAR
+    accepts gym's MountainCarEnv for the discrete variant (a 2-wide state); without it the search classes' original envs only."""
     base = _unwrap(env)
     if not hasattr(base, "state") or base.state is None:
-        raise TypeError("Env has no hidden `.state`; only gym CartPole-v0 / Pendulum-v0 / MountainCarContinuous-v0 style envs are supported")
+        raise TypeError("Env has no hidden `.state`; only gym CartPole-v0 / MountainCar-v0 / Pendulum-v0 / MountainCarContinuous-v0 style "
+                        "envs are supported")
     s = np.asarray(base.state, dtype=np.float64).reshape(-1)
+    if env_id == MOUNTAIN_CAR:
+        if variant != DISCRETE or not _is_mountain_car(base) or s.size != 2:
+            raise TypeError(f"unsupported environment {type(base).__name__} for MountainCar-v0: the discrete search steps gym's "
+                            "MountainCarEnv (a 2-wide state)")
+        return s
     name = type(base).__name__.lower()
     want = 4 if variant == DISCRETE else 2
     mcc = _is_mountain_car_continuous(base)
@@ -204,7 +223,9 @@ class MCTS:
 
 
 class MCTSDiscrete(MCTS):
-    """AlphaZero search for CartPole-v0 (reference mcts.py:310-526)."""
+    """AlphaZero search for CartPole-v0 and MountainCar-v0 (reference mcts.py:310-526).  The env is taken from the Env each search()
+    is handed (discrete_env); search_batch steps the env of the last search(), or the engine keyword `env` (engine.CARTPOLE by
+    default)."""
 
     variant = DISCRETE
 
@@ -213,20 +234,30 @@ class MCTSDiscrete(MCTS):
         super().__init__(model=model, n_rollouts=n_rollouts, c_uct=c_uct, gamma=gamma, epsilon=epsilon, device=device,
                          V_target_policy=V_target_policy, root_state=root_state, seed=seed, **engine_kw)
         self.num_actions = num_actions
+        self._env = self._engine_kw.pop("env", None) or CARTPOLE
 
     def _engine_config(self, max_trees: int) -> EngineConfig:
         d = describe_model(self.model)
         return EngineConfig(variant=DISCRETE, max_rollouts=self.n_rollouts, max_trees=max_trees, num_actions=self.num_actions,
                             state_dim=d["state_dim"], hidden=d["hidden"], n_hidden=d["n_hidden"], activation=d["activation"],
                             V_target_policy=self.V_target_policy, c_uct=self.c_uct, gamma=float(self.gamma), epsilon=self.epsilon,
-                            device=self._cuda_index(), seed=self.seed, **self._engine_kw)
+                            device=self._cuda_index(), seed=self.seed, env=self._env, **self._engine_kw)
 
     def search(self, *args, **kwargs) -> None:
         Env, n_mcts, c = self._env_from_args(args, kwargs)
         if n_mcts is not None and (n_mcts != self.n_rollouts or c != self.c_uct):
             self.close()
             self.n_rollouts, self.c_uct = n_mcts, c
-        hidden = env_hidden_state(Env, DISCRETE)
+        env = discrete_env(Env)
+        if env == MOUNTAIN_CAR:
+            if self.num_actions != 3:
+                raise ValueError(f"MountainCar-v0 has 3 actions, the search was built with num_actions={self.num_actions}")
+            hidden = env_hidden_state(Env, DISCRETE, env_id=MOUNTAIN_CAR)
+        else:
+            hidden = env_hidden_state(Env, DISCRETE)
+        if env != self._env:  # the engines are built for one env
+            self.close()
+            self._env = env
         # initialize_search (mcts.py:364-383): new root, or continue from the node forward() selected
         if self.root_node is None:
             self.root_node = RootNode(np.asarray(self.root_state if self.root_state is not None else hidden), n=0, hidden=hidden)

@@ -17,7 +17,7 @@ import torch
 
 from . import _cabi
 from ._cabi import CONTINUOUS, DISCRETE, check
-from .engine import MOUNTAIN_CAR_CONTINUOUS, SearchEngine
+from .engine import MOUNTAIN_CAR, MOUNTAIN_CAR_CONTINUOUS, SearchEngine
 from .parallel import PackedRows, allgather_results, broadcast_weights
 
 ROW_KEYS = ("obs", "actions", "counts", "Q", "V_target")  # buffer.store((s, actions, counts, Qs, V)), buffers.py:61
@@ -26,7 +26,8 @@ ROW_KEYS = ("obs", "actions", "counts", "Q", "V_target")  # buffer.store((s, act
 def initial_states(variant: int, B: int, seed: int = 34, tree_id0: int = 0, total: Optional[int] = None,
                    env: Optional[str] = None) -> np.ndarray:
     """Env.reset() for every environment: the same rule as SURVEY 8d configs 3/4 (numpy default_rng(seed) over the GLOBAL
-    batch, this shard's slice).  env (engine.EngineConfig.env): MOUNTAIN_CAR_CONTINUOUS draws position ~ U(-0.6, -0.4), velocity 0."""
+    batch, this shard's slice).  env (engine.EngineConfig.env): MOUNTAIN_CAR (discrete) and MOUNTAIN_CAR_CONTINUOUS draw
+    position ~ U(-0.6, -0.4), velocity 0."""
     if total is None:
         # the draw below runs over the GLOBAL batch, so every rank must use the same `total`: tree_id0 + B is only right for a
         # single shard (or the last one)
@@ -34,9 +35,9 @@ def initial_states(variant: int, B: int, seed: int = 34, tree_id0: int = 0, tota
             raise ValueError("initial_states: pass total (the global number of environments) when torch.distributed is initialised")
         total = tree_id0 + B
     rng = np.random.default_rng(seed)
-    if variant == DISCRETE:
+    if variant == DISCRETE and env != MOUNTAIN_CAR:
         s = rng.uniform(-0.05, 0.05, size=(total, 4))
-    elif env == MOUNTAIN_CAR_CONTINUOUS:
+    elif env in (MOUNTAIN_CAR, MOUNTAIN_CAR_CONTINUOUS):
         s = np.stack([rng.uniform(-0.6, -0.4, total), np.zeros(total)], 1)
     else:
         s = np.stack([rng.uniform(-np.pi, np.pi, total), rng.uniform(-1.0, 1.0, total)], 1)

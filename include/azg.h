@@ -30,7 +30,7 @@ extern "C" {
 #define AZG_ENAN -4        /* NaN met in a UCT vector (helpers.py:47-48 only warns; we refuse) */
 #define AZG_ECAPACITY -5   /* tree arena / child fan-out capacity exceeded */
 
-#define AZG_DISCRETE 0   /* MCTSDiscrete  + CartPole-v0 dynamics + DiscretePolicy   */
+#define AZG_DISCRETE 0   /* MCTSDiscrete  + CartPole-v0 dynamics (or, with AZG_FLAG_ENV_MOUNTAIN_CAR, MountainCar-v0) + DiscretePolicy */
 #define AZG_CONTINUOUS 1 /* MCTSContinuous + Pendulum-v0 (or, with AZG_FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS, MountainCarContinuous-v0)
                            dynamics + DiagonalNormal/GMM policy */
 
@@ -52,9 +52,9 @@ typedef struct azg_config {
     int32_t variant;        /* AZG_DISCRETE | AZG_CONTINUOUS */
     int32_t max_rollouts;   /* capacity: largest n_rollouts a search call may ask for */
     int32_t max_trees;      /* capacity: largest batch B */
-    int32_t num_actions;    /* discrete: 2 (CartPole) */
+    int32_t num_actions;    /* discrete: 2 (CartPole), 3 (MountainCar-v0) */
     int32_t num_components; /* continuous: K mixture components (1 = DiagonalNormalPolicy) */
-    int32_t state_dim;      /* network input width: 4 CartPole, 3 Pendulum, 2 MountainCarContinuous */
+    int32_t state_dim;      /* network input width: 4 CartPole, 3 Pendulum, 2 MountainCarContinuous and MountainCar */
     int32_t hidden;         /* hidden width (all hidden layers equal; 128 in both shipped configs) */
     int32_t n_hidden;       /* hidden layers: 2 (DiscretePolicy.yaml) / 3 (ContinuousPolicy.yaml) */
     int32_t activation;     /* AZG_ACT_* */
@@ -100,6 +100,15 @@ typedef struct azg_config {
                                    expanded nodes can be terminal (V = 0).  The search reward is r / 16.2736044 as for every
                                    continuous search (mcts.py:687).  Every schedule, every other flag and the row, control-block and
                                    result layouts are those of the Pendulum search. */
+#define AZG_FLAG_ENV_MOUNTAIN_CAR 32u /* discrete variant only, with num_actions 3 and state_dim 2 (not with
+                                   AZG_FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS): the search steps MountainCar-v0 (gym 0.17-0.19 mountain_car.py)
+                                   instead of CartPole-v0.  Hidden state (position, velocity), network input (float)position,
+                                   (float)velocity; actions 0 (push left), 1 (none), 2 (push right); Node.r is the env's reward, -1.0;
+                                   an episode ends at the goal.  The tree holds 128-byte three-action rows, so max_rollouts <= 16382.
+                                   Every schedule and every other flag apply, except the trees-in-shared-memory whole-search kernel
+                                   (thin batches run the two-phase kernel).  Hidden-state arrays (search roots, d_env_state, the dump's
+                                   state, azg_env_step) are 2 wide; results and dump arrays carry 3 actions.  The reward model
+                                   (azg_set_reward_model) stays the identity. */
 
 typedef struct azg_engine azg_engine;
 
@@ -115,8 +124,8 @@ const char* azg_version(void);
 int64_t azg_num_weights(const azg_engine* e);
 int azg_set_weights(azg_engine* e, const float* flat, int64_t n, void* stream);
 
-/* Batched MCTSDiscrete.search (mcts.py:418-462) over B CartPole roots.
- * d_root_state [B][4] f64 hidden env state (x, x_dot, theta, theta_dot);
+/* Batched MCTSDiscrete.search (mcts.py:418-462) over B CartPole (or MountainCar-v0) roots.
+ * d_root_state [B][4] f64 hidden env state (x, x_dot, theta, theta_dot); MountainCar [B][2] (position, velocity);
  * d_root_n_init [B] carried-over root visit count after forward() (mcts.py:495-526) or NULL;
  * tree_id0: global id of tree 0 -- tree i's RNG streams are keyed by tree_id0+i, which makes results
  * independent of batch composition and of how trees are sharded over GPUs. */
@@ -164,7 +173,8 @@ int azg_set_seed(azg_engine* e, uint64_t seed, void* stream);
  * ReparametrizeWrapper, each / 250.0 with ScaleRewardWrapper (the host computes the constants with the wrappers' own Python
  * expressions).  Takes effect for searches enqueued after the call (synchronises the device and drops captured graphs when something
  * changes).  Not implemented, and refused by the drop-in classes: NormalizeWrapper (sklearn scaler), PILCOWrapper (scipy pdf),
- * ScaleRewardWrapper around Pendulum (it returns np.float32, whose promotion through the backup depends on the numpy version). */
+ * ScaleRewardWrapper around Pendulum (it returns np.float32, whose promotion through the backup depends on the numpy version).  An
+ * engine for any other env (the continuous ones, MountainCar-v0) accepts only the identity (1.0, 1.0). */
 int azg_set_reward_model(azg_engine* e, double reward_step, double reward_terminal);
 
 /* ---- self-play step (SURVEY 8f rank 1; BASELINE config 5) -------------------------------------------------------------
@@ -179,7 +189,7 @@ int azg_set_reward_model(azg_engine* e, double reward_step, double reward_termin
  *   (reset_mcts), else discrete tree reuse: d_root_n = visit count of the chosen child (mcts.py:495-526).
  * All pointers are device pointers owned by the caller; in/out arrays carry the state from step to step. */
 typedef struct azg_selfplay_io {
-    double* d_env_state;   /* in/out [B][4|2] hidden env state (CartPole x, x_dot, theta, theta_dot | Pendulum th, thdot |
+    double* d_env_state;   /* in/out [B][4|2] hidden env state (CartPole x, x_dot, theta, theta_dot | MountainCar position, velocity | Pendulum th, thdot |
                               MountainCarContinuous position, velocity) */
     int32_t* d_ep_step;    /* in/out [B] steps taken in the current episode */
     int32_t* d_episode;    /* in/out [B] episode counter (indexes the reset stream) */
@@ -215,7 +225,7 @@ typedef struct azg_dump_discrete { /* host arrays, R = azg_rows(e), A = num_acti
     int32_t* terminal; /* [B][R] */
     float* V;          /* [B][R] */
     double* r;         /* [B][R] */
-    double* state;     /* [B][R][4] */
+    double* state;     /* [B][R][4]; MountainCar [B][R][2] */
     float* prior;      /* [B][R][A] */
     double* eW;        /* [B][R][A] Action.W */
     int32_t* en;       /* [B][R][A] Action.n */
@@ -264,8 +274,8 @@ int azg_profile_search(azg_engine* e, int32_t B, const double* d_root_state, con
 int32_t azg_head_dim(const azg_engine* e);
 int azg_mlp_forward(azg_engine* e, int32_t n, const float* d_x, float* d_V, float* d_head, void* stream);
 
-/* Batched env.step of the engine's env on its own (known-answer tests): d_state [n][4|2], d_action [n] (index as float for
- * CartPole) -> d_next [n][4|2], d_reward [n] (raw env reward), d_terminal [n], d_obs [n][state_dim]. */
+/* Batched env.step of the engine's env on its own (known-answer tests): d_state [n][4|2] (CartPole 4, MountainCar and the continuous
+ * envs 2), d_action [n] (index as float for CartPole and MountainCar) -> d_next [n][4|2], d_reward [n] (raw env reward), d_terminal [n], d_obs [n][state_dim]. */
 int azg_env_step(azg_engine* e, int32_t n, const double* d_state, const float* d_action, double* d_next, double* d_reward,
                  int32_t* d_terminal, float* d_obs, void* stream);
 
