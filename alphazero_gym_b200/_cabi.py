@@ -12,6 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("AZG_LIB_PATH") or os.path.join(HERE, "lib", "libazg.so")  # override: kernel experiments only
 
 AZG_OK, AZG_EINVAL, AZG_ECUDA, AZG_ETERMINAL, AZG_ENAN, AZG_ECAPACITY = 0, -1, -2, -3, -4, -5
+AZG_EWRAP = -6  # Acrobot-v1: an angle reached the wrap loop's cap (include/azg.h)
 DISCRETE, CONTINUOUS = 0, 1
 ACT_RELU, ACT_ELU, ACT_LEAKYRELU, ACT_RELU6, ACT_SILU, ACT_HARDSWISH = 0, 1, 2, 3, 4, 5
 # nonlinearity strings of config/policy/*.yaml (alphazero/network/utils.py:5-14) and torch module names -> AZG_ACT_*
@@ -23,6 +24,7 @@ FLAG_FUSED = 4
 FLAG_RNG_MT19937 = 8
 FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS = 16
 FLAG_ENV_MOUNTAIN_CAR = 32
+FLAG_ENV_ACROBOT = 64
 
 EXPORTS = [
     "azg_create", "azg_destroy", "azg_last_error", "azg_version", "azg_num_weights", "azg_set_weights",

@@ -116,6 +116,7 @@ static_assert(sizeof(CCtl) == 64, "control block must be one 64 B line");
 
 #define ERR_NAN 1
 #define ERR_CAPACITY 2
+#define ERR_WRAP 4  // Acrobot: an angle reached ACROBOT_WRAP_CAP iterations of wrap (env.cuh)
 
 struct TreeParams {
     int32_t B, R, A, K, HS;  // trees, rows per tree, actions, mixture components, head stride (floats)
@@ -128,8 +129,8 @@ struct TreeParams {
     int32_t tree_word;      // launches captured into a CUDA graph: the global id of tree 0 is seedp[1] (and tree_id0 is 0), so that one
                             // graph serves every tree_id0 (the drop-in classes search with a new id every call)
     // discrete tables
-    DRow* drows;      // [B][R]  (MountainCar-v0: D3Row [B][R], same pointer)
-    double* dstate;   // [B][R][4]  (MountainCar-v0: the first 2 of each 4)
+    DRow* drows;      // [B][R]  (MountainCar-v0, Acrobot-v1: D3Row [B][R], same pointer)
+    double* dstate;   // [B][R][4]  (MountainCar-v0: the first 2 of each 4; Acrobot-v1: all 4)
     // continuous tables
     CRow* crows;      // [B][R]
     float* chead;     // [B][R][HS]  mu[K], sigma[K], prob[K]
@@ -155,7 +156,7 @@ struct TreeParams {
                       // root first (read by the backup)
     int32_t* ddepth;  // [B]    discrete: its length
     uint32_t* ctr;    // [4][B]: levels, children scanned, terminal-leaf sims, evals
-    float4* X;        // [B] network input of the leaf
+    float4* X;        // [B][XW] network input of the leaf (XW = 2 for Acrobot's 6 inputs, 1 otherwise)
     const double* root_state;
     const int32_t* root_n_init;
     int32_t* err;

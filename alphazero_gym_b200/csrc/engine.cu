@@ -95,6 +95,7 @@ struct azg_engine {
     bool fused = false;  // AZG_FLAG_FUSED: the whole continuous search in one persistent kernel (qmlp2.cuh)
     bool mcc = false;    // AZG_FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS: the continuous kernels are instantiated for env::MountainCarContinuous
     bool mc = false;     // AZG_FLAG_ENV_MOUNTAIN_CAR: the discrete kernels are instantiated for env::MountainCar (three-action rows)
+    bool ac = false;     // AZG_FLAG_ENV_ACROBOT: the discrete kernels are instantiated for env::Acrobot (three-action rows, 6 inputs)
     // results staging (device) + pinned host staging for the *_host entry point
     float* r_actions = nullptr;
     int32_t* r_counts = nullptr;
@@ -130,7 +131,7 @@ static int head_dim_of(const azg_config& c) {
     return c.num_components > 1 ? 3 * c.num_components : 2;
 }
 
-// width of the hidden-state arrays the host hands in and gets back: CartPole 4, MountainCar and the continuous envs 2
+// width of the hidden-state arrays the host hands in and gets back: CartPole and Acrobot 4, MountainCar and the continuous envs 2
 static int state_width(const azg_engine* e) { return e->cfg.variant == AZG_DISCRETE && !e->mc ? 4 : 2; }
 
 static int pw_limit(double c_pw, double kappa, int n) { return (int)std::ceil(c_pw * std::pow((double)(n + 1), kappa)); }
@@ -185,13 +186,17 @@ extern "C" int azg_create(const azg_config* cfg, azg_engine** out) {
     if (mc && mcc) return fail(AZG_EINVAL, "AZG_FLAG_ENV_MOUNTAIN_CAR and AZG_FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS exclude each other");
     if (mc && (c.variant != AZG_DISCRETE || c.num_actions != 3 || c.state_dim != 2))
         return fail(AZG_EINVAL, "AZG_FLAG_ENV_MOUNTAIN_CAR needs the discrete variant, num_actions 3 and state_dim 2");
+    const bool ac = (c.flags & AZG_FLAG_ENV_ACROBOT) != 0;
+    if (ac && (mc || mcc)) return fail(AZG_EINVAL, "AZG_FLAG_ENV_ACROBOT excludes both MountainCar flags");
+    if (ac && (c.variant != AZG_DISCRETE || c.num_actions != 3 || c.state_dim != 6))
+        return fail(AZG_EINVAL, "AZG_FLAG_ENV_ACROBOT needs the discrete variant, num_actions 3 and state_dim 6");
     if (c.variant == AZG_DISCRETE) {
-        if (!mc && (c.num_actions != 2 || c.state_dim != 4))
+        if (!mc && !ac && (c.num_actions != 2 || c.state_dim != 4))
             return fail(AZG_EINVAL, "discrete variant is CartPole (num_actions 2, state_dim 4) or, with AZG_FLAG_ENV_MOUNTAIN_CAR, MountainCar-v0 "
-                                    "(num_actions 3, state_dim 2)");
+                                    "(num_actions 3, state_dim 2) or, with AZG_FLAG_ENV_ACROBOT, Acrobot-v1 (num_actions 3, state_dim 6)");
         if (c.max_rollouts + 2 > 65534) return fail(AZG_EINVAL, "max_rollouts too large for 16-bit child links");
-        if (mc && c.max_rollouts + 2 > 16384)
-            return fail(AZG_EINVAL, "MountainCar-v0 supports max_rollouts <= 16382 (a path entry holds row << 2 | action in 16 bits)");
+        if ((mc || ac) && c.max_rollouts + 2 > 16384)
+            return fail(AZG_EINVAL, "MountainCar-v0 and Acrobot-v1 support max_rollouts <= 16382 (a path entry holds row << 2 | action in 16 bits)");
     } else {
         if (!mcc && c.state_dim != 3) return fail(AZG_EINVAL, "continuous variant is Pendulum: state_dim must be 3");
         if (c.num_components < 1 || c.num_components > AZG_MAX_K) return fail(AZG_EINVAL, "num_components must be in 1..8");
@@ -206,6 +211,7 @@ extern "C" int azg_create(const azg_config* cfg, azg_engine** out) {
     e->cfg = c;
     e->mcc = mcc;
     e->mc = mc;
+    e->ac = ac;
     e->R = c.max_rollouts + 2;
     e->P = head_dim_of(c);
     e->PO_PAD = ((1 + e->P) + 3) / 4 * 4;
@@ -246,10 +252,10 @@ extern "C" int azg_create(const azg_config* cfg, azg_engine** out) {
         delete e;
         return fail(AZG_EINVAL, "AZG_FLAG_RNG_MT19937 with the continuous search runs one launch per simulation (no AZG_FLAG_FUSED)");
     }
-    if (e->fused && !(e->q8 && c.state_dim == (c.variant == AZG_CONTINUOUS ? (mcc ? 2 : 3) : (mc ? 2 : 4)))) {
+    if (e->fused && !(e->q8 && c.state_dim == (c.variant == AZG_CONTINUOUS ? (mcc ? 2 : 3) : (mc ? 2 : (ac ? 6 : 4))))) {
         delete e;
         return fail(AZG_EINVAL, "AZG_FLAG_FUSED needs AZG_FLAG_EVAL_Q8 and the shipped envs (state_dim 3 Pendulum / 2 MountainCarContinuous / 4 CartPole / "
-                                "2 MountainCar)");
+                                "2 MountainCar / 6 Acrobot)");
     }
     const size_t B = c.max_trees, R = e->R;
     std::vector<int32_t> pwt;
@@ -277,7 +283,7 @@ extern "C" int azg_create(const azg_config* cfg, azg_engine** out) {
         }                                               \
     } while (0)
     if (c.variant == AZG_DISCRETE) {
-        ALLOC(drows, B * R * (mc ? sizeof(D3Row) / sizeof(DRow) : 1));  // MountainCar: D3Row [B][R]
+        ALLOC(drows, B * R * (mc || ac ? sizeof(D3Row) / sizeof(DRow) : 1));  // MountainCar, Acrobot: D3Row [B][R]
         ALLOC(dstate, B * R * 4);
         ALLOC(dpath, B * R);
         ALLOC(ddepth, B);
@@ -327,7 +333,7 @@ extern "C" int azg_create(const azg_config* cfg, azg_engine** out) {
     }
     ALLOC(n_rows, B); ALLOC(draws, B); ALLOC(leaf, B);
     ALLOC(ctr, 4 * B);
-    ALLOC(X, B);
+    ALLOC(X, B * (ac ? env::Acrobot::XW : 1));  // Acrobot: 6 inputs in two float4 per tree
     ALLOC(root_state, B * 4);
     ALLOC(root_n_init, B);
     ALLOC(err, 1);
@@ -541,7 +547,7 @@ static MlpParams make_mlp_params(const azg_engine* e, int n) {
     memset(&m, 0, sizeof m);
     const azg_config& c = e->cfg;
     m.wpack = e->wpack; m.wcount = e->wcount; m.L = c.n_hidden; m.P = e->P; m.PO_PAD = e->PO_PAD;
-    m.n = n; m.X = reinterpret_cast<const float*>(e->X); m.xstride = 4; m.mode = 0;
+    m.n = n; m.X = reinterpret_cast<const float*>(e->X); m.xstride = e->ac ? 4 * env::Acrobot::XW : 4; m.mode = 0;
     m.variant = c.variant; m.A = c.num_actions; m.K = c.num_components; m.R = e->R; m.HS = e->HS;
     m.ls_min = c.log_std_min; m.ls_max = c.log_std_max;
     m.leaf = e->leaf; m.drows = e->drows; m.crows = e->crows; m.chead = e->chead; m.evals = e->ctr + (size_t)3 * n;
@@ -664,6 +670,13 @@ using ShippedEnv = std::conditional_t<S == 4, env::CartPole, env::Pendulum>;
 
 static cudaError_t launch_fused(const azg_engine* e, const MlpParams& m, const TreeParams& p, int N, cudaStream_t st, int* launches) {
     const int S = e->cfg.state_dim, A = e->cfg.activation, NL = e->cfg.n_hidden - 1;
+    if (e->ac) {
+#define FUSED_AC_CASE(a, nl) \
+    if (A == a && NL == nl) return launch_fused_t<env::Acrobot, a, nl>(e, m, p, N, st, launches);
+        FUSED_AC_CASE(0, 1) FUSED_AC_CASE(1, 1) FUSED_AC_CASE(0, 2) FUSED_AC_CASE(1, 2)
+#undef FUSED_AC_CASE
+        return cudaErrorInvalidValue;
+    }
     if (e->mc) {
 #define FUSED_MC_CASE(a, nl) \
     if (A == a && NL == nl) return launch_fused_t<env::MountainCar, a, nl>(e, m, p, N, st, launches);
@@ -690,6 +703,13 @@ static cudaError_t launch_mlp(const azg_engine* e, const MlpParams& m, cudaStrea
     const int H = e->cfg.hidden, S = e->cfg.state_dim, A = e->cfg.activation;
     if (e->q8) {
         const int NL = e->cfg.n_hidden - 1;
+        if (e->ac) {
+#define QMLP_AC_CASE(a, nl) \
+    if (A == a && NL == nl) return launch_qmlp_t<env::Acrobot, a, nl>(e, m, st, set_attr);
+            QMLP_AC_CASE(0, 1) QMLP_AC_CASE(1, 1) QMLP_AC_CASE(0, 2) QMLP_AC_CASE(1, 2)
+#undef QMLP_AC_CASE
+            return cudaErrorInvalidValue;
+        }
         if (e->mc) {
 #define QMLP_MC_CASE(a, nl) \
     if (A == a && NL == nl) return launch_qmlp_t<env::MountainCar, a, nl>(e, m, st, set_attr);
@@ -709,6 +729,14 @@ static cudaError_t launch_mlp(const azg_engine* e, const MlpParams& m, cudaStrea
         QMLP_CASE(4, 0, 1) QMLP_CASE(4, 1, 1) QMLP_CASE(3, 0, 1) QMLP_CASE(3, 1, 1)
         QMLP_CASE(4, 0, 2) QMLP_CASE(4, 1, 2) QMLP_CASE(3, 0, 2) QMLP_CASE(3, 1, 2)
 #undef QMLP_CASE
+        return cudaErrorInvalidValue;
+    }
+    if (e->ac) {  // layer 0 with six inputs (Acrobot)
+#define MLP_AC_CASE(h, a) \
+    if (H == h && A == a) return launch_mlp_t<h, 6, a>(e, m, st, set_attr);
+        MLP_AC_CASE(128, 0) MLP_AC_CASE(128, 1) MLP_AC_CASE(128, 2) MLP_AC_CASE(128, 3) MLP_AC_CASE(128, 4) MLP_AC_CASE(128, 5)
+        MLP_AC_CASE(64, 0) MLP_AC_CASE(64, 1) MLP_AC_CASE(64, 2) MLP_AC_CASE(64, 3) MLP_AC_CASE(64, 4) MLP_AC_CASE(64, 5)
+#undef MLP_AC_CASE
         return cudaErrorInvalidValue;
     }
     if (e->mcc || e->mc) {  // layer 0 with two inputs (both MountainCar envs; k_mlp reads the row layout at run time)
@@ -734,6 +762,7 @@ static cudaError_t launch_mlp(const azg_engine* e, const MlpParams& m, cudaStrea
 template <bool BK, bool SEL>
 static cudaError_t launch_step_discrete(const azg_engine* e, const TreeParams& p, cudaStream_t st) {
     if (e->mc) return launch_ex(e, k_step_discrete<env::MountainCar, BK, SEL>, (p.B + 127) / 128, 128, 0, st, p);
+    if (e->ac) return launch_ex(e, k_step_discrete<env::Acrobot, BK, SEL>, (p.B + 127) / 128, 128, 0, st, p);
     return launch_ex(e, k_step_discrete<env::CartPole, BK, SEL>, (p.B + 127) / 128, 128, 0, st, p);
 }
 
@@ -786,6 +815,7 @@ static int enqueue_search(azg_engine* e, int B, int N, int64_t tree_id0, cudaStr
     }
     if (e->cfg.variant == AZG_DISCRETE) {
         if (e->mc) LK(2, (k_init_discrete<env::MountainCar><<<tg, tb, 0, st>>>(p)));
+        else if (e->ac) LK(2, (k_init_discrete<env::Acrobot><<<tg, tb, 0, st>>>(p)));
         else LK(2, (k_init_discrete<env::CartPole><<<tg, tb, 0, st>>>(p)));
         if (!tape) LK(1, ce = launch_mlp(e, m, st, false));
         for (int it = 0; it < N; ++it) {
@@ -933,6 +963,7 @@ extern "C" int azg_root_results(azg_engine* e, int32_t B, float* d_actions, int3
     const TreeParams p = make_params(e, B, 0);
     const int tb = 128, tg = (B + tb - 1) / tb;
     if (e->cfg.variant == AZG_DISCRETE && e->mc) k_results_discrete<env::MountainCar><<<tg, tb, 0, st>>>(p, e->cmax, d_actions, d_counts, d_Q, d_V_target, d_n_children);
+    else if (e->cfg.variant == AZG_DISCRETE && e->ac) k_results_discrete<env::Acrobot><<<tg, tb, 0, st>>>(p, e->cmax, d_actions, d_counts, d_Q, d_V_target, d_n_children);
     else if (e->cfg.variant == AZG_DISCRETE) k_results_discrete<env::CartPole><<<tg, tb, 0, st>>>(p, e->cmax, d_actions, d_counts, d_Q, d_V_target, d_n_children);
     else k_results_continuous<<<tg, tb, 0, st>>>(p, e->cmax, d_actions, d_counts, d_Q, d_V_target, d_n_children);
     CK(cudaGetLastError());
@@ -948,6 +979,7 @@ extern "C" int azg_status(azg_engine* e, void* stream) {
     if (h) CK(cudaMemsetAsync(e->err, 0, sizeof h, (cudaStream_t)stream));
     if (h & ERR_NAN) return fail(AZG_ENAN, "NaN in a UCT vector (helpers.py:47-48)");
     if (h & ERR_CAPACITY) return fail(AZG_ECAPACITY, "tree arena or child fan-out capacity exceeded");
+    if (h & ERR_WRAP) return fail(AZG_EWRAP, "Acrobot-v1: an angle needed more than 64 iterations of wrap (gym would loop on)");
     return AZG_OK;
 }
 
@@ -1087,6 +1119,7 @@ extern "C" int azg_search_host_end(azg_engine* e, int32_t slot) {
     const int32_t h = e->h_err[slot];
     if (h & ERR_NAN) return fail(AZG_ENAN, "NaN in a UCT vector (helpers.py:47-48)");
     if (h & ERR_CAPACITY) return fail(AZG_ECAPACITY, "tree arena or child fan-out capacity exceeded");
+    if (h & ERR_WRAP) return fail(AZG_EWRAP, "Acrobot-v1: an angle needed more than 64 iterations of wrap (gym would loop on)");
     return AZG_OK;
 }
 
@@ -1185,7 +1218,7 @@ extern "C" int azg_set_reward_model(azg_engine* e, double reward_step, double re
     if (!e) return fail(AZG_EINVAL, "null engine");
     if (!(reward_step == reward_step) || !(reward_terminal == reward_terminal) || std::isinf(reward_step) || std::isinf(reward_terminal))
         return fail(AZG_EINVAL, "rewards must be finite");
-    if ((e->cfg.variant != AZG_DISCRETE || e->mc) && (reward_step != 1.0 || reward_terminal != 1.0))
+    if ((e->cfg.variant != AZG_DISCRETE || e->mc || e->ac) && (reward_step != 1.0 || reward_terminal != 1.0))
         return fail(AZG_EINVAL, "the reward model applies to the CartPole search (the other envs' searches take the env's own reward)");
     if (reward_step == e->reward_step && reward_terminal == e->reward_terminal) return AZG_OK;
     CK(cudaSetDevice(e->cfg.device));
@@ -1225,9 +1258,10 @@ extern "C" int azg_selfplay_step(azg_engine* e, int32_t B, const azg_selfplay_io
     sp.env_state = io->d_env_state; sp.ep_step = io->d_ep_step; sp.episode = io->d_episode; sp.root_n = io->d_root_n;
     sp.actions = io->d_actions; sp.counts = io->d_counts; sp.Q = io->d_Q; sp.n_children = io->d_n_children;
     sp.obs = io->d_obs; sp.action_taken = io->d_action_taken; sp.reward = io->d_reward; sp.done = io->d_done;
-    sp.drows = e->drows; sp.R = e->R;
+    sp.drows = e->drows; sp.R = e->R; sp.err = e->err;
     const int tb = 128, tg = (B + tb - 1) / tb;
     if (disc && e->mc) k_selfplay_discrete<env::MountainCar><<<tg, tb, 0, st>>>(sp);
+    else if (disc && e->ac) k_selfplay_discrete<env::Acrobot><<<tg, tb, 0, st>>>(sp);
     else if (disc) k_selfplay_discrete<env::CartPole><<<tg, tb, 0, st>>>(sp);
     else if (e->mcc) k_selfplay_continuous<env::MountainCarContinuous><<<tg, tb, 0, st>>>(sp);
     else k_selfplay_continuous<env::Pendulum><<<tg, tb, 0, st>>>(sp);
@@ -1236,7 +1270,7 @@ extern "C" int azg_selfplay_step(azg_engine* e, int32_t B, const azg_selfplay_io
 }
 
 // ---- tree dump (host side unpacking of the device tables) ------------------------------------------------
-// ROW = DRow (CartPole: A = 2, state 4 wide) or D3Row (MountainCar: A = 3, state 2 wide)
+// ROW = DRow (CartPole: A = 2, state 4 wide) or D3Row (MountainCar: A = 3, state 2 wide; Acrobot: A = 3, state 4 wide)
 template <class ROW>
 static int dump_discrete(azg_engine* e, int32_t B, const azg_dump_discrete* o, size_t A, size_t SW) {
     const size_t R = e->R;
@@ -1277,6 +1311,7 @@ extern "C" int azg_dump_tree_discrete(azg_engine* e, int32_t B, const azg_dump_d
     CK(cudaSetDevice(e->cfg.device));
     CK(cudaDeviceSynchronize());
     if (e->mc) return dump_discrete<D3Row>(e, B, o, 3, 2);
+    if (e->ac) return dump_discrete<D3Row>(e, B, o, 3, 4);
     return dump_discrete<DRow>(e, B, o, 2, 4);
 }
 
@@ -1359,11 +1394,23 @@ __device__ __forceinline__ void env_step_continuous(int i, const double* s, cons
     term[i] = t;
 }
 
-__global__ void k_env_step(int variant, bool mcc, bool mc, int n, const double* s, const float* a, double* o, double* rew, int32_t* term,
-                           float* obs) {
+__global__ void k_env_step(int variant, bool mcc, bool mc, bool ac, int n, const double* s, const float* a, double* o, double* rew,
+                           int32_t* term, float* obs, int32_t* err) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    if (variant == AZG_DISCRETE && mc) {  // the action is an index 0, 1, 2
+    if (variant == AZG_DISCRETE && ac) {  // the action is an index 0, 1, 2; the observation is 6 wide
+        const double in[4] = {s[i * 4], s[i * 4 + 1], s[i * 4 + 2], s[i * 4 + 3]};
+        double out[4], r;
+        bool capped = false;
+        const bool t = env::acrobot_step(in, (int)a[i], out, r, capped);
+        if (capped) atomicOr(err, ERR_WRAP);
+        float x[6];
+        env::acrobot_obs(out, x);
+        for (int k = 0; k < 4; ++k) o[i * 4 + k] = out[k];
+        for (int k = 0; k < 6; ++k) obs[i * 6 + k] = x[k];
+        rew[i] = r;
+        term[i] = t;
+    } else if (variant == AZG_DISCRETE && mc) {  // the action is an index 0, 1, 2
         double n0, n1, r;
         const bool t = env::MountainCar::step(s[i * 2], s[i * 2 + 1], (int)a[i], n0, n1, r);
         o[i * 2] = n0; o[i * 2 + 1] = n1;
@@ -1389,7 +1436,8 @@ extern "C" int azg_env_step(azg_engine* e, int32_t n, const double* d_state, con
     if (!e || !d_state || !d_action || !d_next || !d_reward || !d_terminal || !d_obs) return fail(AZG_EINVAL, "null argument");
     if (n < 1) return fail(AZG_EINVAL, "n must be >= 1");
     CK(cudaSetDevice(e->cfg.device));
-    k_env_step<<<(n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(e->cfg.variant, e->mcc, e->mc, n, d_state, d_action, d_next, d_reward, d_terminal, d_obs);
+    k_env_step<<<(n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(e->cfg.variant, e->mcc, e->mc, e->ac, n, d_state, d_action, d_next, d_reward,
+                                                                  d_terminal, d_obs, e->err);
     CK(cudaGetLastError());
     return AZG_OK;
 }

@@ -101,15 +101,92 @@ __device__ __forceinline__ bool mountain_car_step(double pos, double vel, int ac
     return pos >= goal_position && vel >= 0.0;
 }
 
-// The env of a search as a compile-time type.  Continuous: the hidden state is two doubles (CRow sector 1), the network input the
-// first S lanes of a float4.  Discrete: A actions, the row layout follows (DRow for 2, D3Row for 3).  CartPole names the discrete tree
-// in the kernels that serve both variants.
+// Acrobot-v1 (gym 0.17-0.19 classic_control/acrobot.py, book dynamics, no torque noise).  Every operation is f64 in the source's
+// left-to-right order; x ** 2 of a float is x * x; sin / cos are the deterministic ones, one sincos_ per distinct argument.
+//
+// wrap(x, -pi, pi) is gym's pair of unbounded while loops.  Each loop here stops after ACROBOT_WRAP_CAP iterations and sets `capped`
+// (the search then fails with ERR_WRAP) instead of spinning on an infinite or huge angle.  Stepped from inside gym's box (angles in
+// [-pi, pi], |dtheta1| <= 4 pi, |dtheta2| <= 9 pi) an angle needs at most 5 turns (DESIGN.md section 6), so the cap never changes
+// a result gym can produce.  A NaN passes through wrap and bound as it does in gym.
+#define ACROBOT_WRAP_CAP 64
+__device__ __forceinline__ void acrobot_dsdt(const double s[4], double a, double d[4]) {
+    const double m1 = 1.0, m2 = 1.0, l1 = 1.0, lc1 = 0.5, lc2 = 0.5, I1 = 1.0, I2 = 1.0, g = 9.8, pi = 3.141592653589793;
+    const double theta1 = s[0], theta2 = s[1], dtheta1 = s[2], dtheta2 = s[3];
+    double s2, c2;
+    det::sincos_(theta2, s2, c2);
+    const double d1 = m1 * (lc1 * lc1) + m2 * (l1 * l1 + lc2 * lc2 + 2 * l1 * lc2 * c2) + I1 + I2;
+    const double d2 = m2 * (lc2 * lc2 + l1 * lc2 * c2) + I2;
+    const double phi2 = m2 * lc2 * g * det::cos_(theta1 + theta2 - pi / 2.);
+    const double phi1 = -m2 * l1 * lc2 * (dtheta2 * dtheta2) * s2 - 2 * m2 * l1 * lc2 * dtheta2 * dtheta1 * s2 +
+                        (m1 * lc1 + m2 * l1) * g * det::cos_(theta1 - pi / 2) + phi2;
+    const double ddtheta2 = (a + d2 / d1 * phi1 - m2 * l1 * lc2 * (dtheta1 * dtheta1) * s2 - phi2) / (m2 * (lc2 * lc2) + I2 - (d2 * d2) / d1);
+    const double ddtheta1 = -(d2 * ddtheta2 + phi1) / d1;
+    d[0] = dtheta1; d[1] = dtheta2; d[2] = ddtheta1; d[3] = ddtheta2;
+}
+__device__ __forceinline__ double acrobot_wrap(double x, bool& capped) {
+    const double pi = 3.141592653589793, diff = pi - -pi;
+    for (int k = 0; x > pi; ++k) {
+        if (k == ACROBOT_WRAP_CAP) { capped = true; return x; }
+        x = x - diff;
+    }
+    for (int k = 0; x < -pi; ++k) {
+        if (k == ACROBOT_WRAP_CAP) { capped = true; return x; }
+        x = x + diff;
+    }
+    return x;
+}
+// bound(x, m, M) = min(max(x, m), M) with Python's builtins: a NaN passes, -0 stays -0
+__device__ __forceinline__ double acrobot_bound(double x, double m, double M) {
+    x = m > x ? m : x;
+    return M < x ? M : x;
+}
+// returns terminal; reward -1.0 before the goal, 0.0 at it.  The torque (the fifth RK4 component) has derivative 0, so it stays exact.
+__device__ __forceinline__ bool acrobot_step(const double s[4], int action, double o[4], double& reward, bool& capped) {
+    const double dt = .2, pi = 3.141592653589793, MAX_VEL_1 = 4 * pi, MAX_VEL_2 = 9 * pi;
+    const double torque = action == 0 ? -1.0 : (action == 1 ? 0.0 : 1.0);
+    const double dt2 = dt / 2.0;
+    double k1[4], k2[4], k3[4], k4[4], y[4];
+    acrobot_dsdt(s, torque, k1);
+#pragma unroll
+    for (int i = 0; i < 4; ++i) y[i] = s[i] + dt2 * k1[i];
+    acrobot_dsdt(y, torque, k2);
+#pragma unroll
+    for (int i = 0; i < 4; ++i) y[i] = s[i] + dt2 * k2[i];
+    acrobot_dsdt(y, torque, k3);
+#pragma unroll
+    for (int i = 0; i < 4; ++i) y[i] = s[i] + dt * k3[i];
+    acrobot_dsdt(y, torque, k4);
+#pragma unroll
+    for (int i = 0; i < 4; ++i) o[i] = s[i] + dt / 6.0 * (k1[i] + 2 * k2[i] + 2 * k3[i] + k4[i]);
+    o[0] = acrobot_wrap(o[0], capped);
+    o[1] = acrobot_wrap(o[1], capped);
+    o[2] = acrobot_bound(o[2], -MAX_VEL_1, MAX_VEL_1);
+    o[3] = acrobot_bound(o[3], -MAX_VEL_2, MAX_VEL_2);
+    const bool terminal = -det::cos_(o[0]) - det::cos_(o[1] + o[0]) > 1.;
+    reward = terminal ? 0.0 : -1.0;
+    return terminal;
+}
+// _get_ob: cos / sin of both angles and both velocities, computed in f64 and rounded to f32 per entry
+__device__ __forceinline__ void acrobot_obs(const double s[4], float x[6]) {
+    double s0, c0, s1, c1;
+    det::sincos_(s[0], s0, c0);
+    det::sincos_(s[1], s1, c1);
+    x[0] = (float)c0; x[1] = (float)s0; x[2] = (float)c1; x[3] = (float)s1; x[4] = (float)s[2]; x[5] = (float)s[3];
+}
+
+// The env of a search as a compile-time type.  S is the network input width, HS the width of the hidden state the tree keeps per node
+// (HS doubles; the discrete state table has room for 4).  Continuous: the hidden state is two doubles (CRow sector 1), the network input
+// the first S lanes of a float4.  Discrete: A actions, the row layout follows (DRow for 2, D3Row for 3).  CartPole names the discrete
+// tree in the kernels that serve both variants.
+//
+// The three-action envs also give the tree's view of the env on hidden-state arrays: expand (one env step; `capped`: a wrap loop reached
+// its cap) and input (the network input as XW = ceil(S / 4) float4, unused lanes 0); Acrobot's reset takes four uniforms.
 struct CartPole {
-    static constexpr int S = 4, A = 2;
+    static constexpr int S = 4, HS = 4, A = 2;
     static constexpr bool DISCRETE = true;
 };
 struct MountainCar {
-    static constexpr int S = 2, A = 3;
+    static constexpr int S = 2, HS = 2, A = 3, XW = 1;
     static constexpr bool DISCRETE = true;
     static __device__ __forceinline__ bool step(double pos, double vel, int a, double& npos, double& nvel, double& r) {
         return mountain_car_step(pos, vel, a, npos, nvel, r);
@@ -120,9 +197,30 @@ struct MountainCar {
         pos = -0.6 + (-0.4 - -0.6) * u0;
         vel = 0.0;
     }
+    static __device__ __forceinline__ bool expand(const double* s, int a, double* o, double& r, bool&) {
+        return step(s[0], s[1], a, o[0], o[1], r);
+    }
+    static __device__ __forceinline__ void input(const double* s, float4* x) { x[0] = obs(s[0], s[1]); }
+};
+struct Acrobot {
+    static constexpr int S = 6, HS = 4, A = 3, XW = 2;
+    static constexpr bool DISCRETE = true;
+    static __device__ __forceinline__ bool expand(const double* s, int a, double* o, double& r, bool& capped) {
+        return acrobot_step(s, a, o, r, capped);
+    }
+    static __device__ __forceinline__ void input(const double* s, float4* x) {
+        float v[6];
+        acrobot_obs(s, v);
+        x[0] = make_float4(v[0], v[1], v[2], v[3]);
+        x[1] = make_float4(v[4], v[5], 0.0f, 0.0f);
+    }
+    // Env.reset: the state ~ U(-0.1, 0.1)^4
+    static __device__ __forceinline__ void reset(const double* u, double* s) {
+        for (int k = 0; k < 4; ++k) s[k] = -0.1 + (0.1 - -0.1) * u[k];
+    }
 };
 struct Pendulum {
-    static constexpr int S = 3;
+    static constexpr int S = 3, HS = 2;
     static constexpr bool DISCRETE = false;
     static __device__ __forceinline__ bool step(double th, double thdot, float a, double& nth, double& nthdot, double& r) {
         return pendulum_step(th, thdot, a, nth, nthdot, r);
@@ -136,7 +234,7 @@ struct Pendulum {
     }
 };
 struct MountainCarContinuous {
-    static constexpr int S = 2;
+    static constexpr int S = 2, HS = 2;
     static constexpr bool DISCRETE = false;
     static __device__ __forceinline__ bool step(double pos, double vel, float a, double& npos, double& nvel, double& r) {
         return mountain_car_step(pos, vel, a, npos, nvel, r);

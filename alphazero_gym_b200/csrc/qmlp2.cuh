@@ -167,7 +167,15 @@ __device__ __forceinline__ float q2_layer0(const Q2Ctx& c, const MlpParams& p, i
 #pragma unroll
         for (int s = 0; s < S; ++s) x[s] = 0.0f;
         if (valid) {
-            if (p.xstride == 4) {
+            if constexpr (S > 4) {  // Acrobot: 6 inputs in two float4 per leaf (the tree writes xstride 8)
+                if (p.xstride == 8) {
+                    const float4 v = *reinterpret_cast<const float4*>(p.X + (size_t)gr * 8), w = *reinterpret_cast<const float4*>(p.X + (size_t)gr * 8 + 4);
+                    x[0] = v.x; x[1] = v.y; x[2] = v.z; x[3] = v.w; x[4] = w.x; x[5] = w.y;
+                } else {
+#pragma unroll
+                    for (int s = 0; s < S; ++s) x[s] = p.X[(size_t)gr * p.xstride + s];
+                }
+            } else if (p.xstride == 4) {
                 const float4 v = *reinterpret_cast<const float4*>(p.X + (size_t)gr * 4);
                 x[0] = v.x; x[1] = v.y;
                 if constexpr (S > 2) x[2] = v.z;
@@ -328,10 +336,15 @@ __device__ __forceinline__ void q2_eval_rep(const Q2Ctx& c, const MlpParams& p, 
 #pragma unroll
         for (int s = 0; s < S; ++s) x[s] = 0.0f;
         if (r < nv) {
-            const float4 v = *reinterpret_cast<const float4*>(p.X + (size_t)(row0 + r) * 4);  // xstride 4 in the whole-search kernel
-            x[0] = v.x; x[1] = v.y;
-            if constexpr (S > 2) x[2] = v.z;
-            if (S > 3) x[S - 1] = v.w;
+            if constexpr (S > 4) {  // Acrobot: xstride 8 in the whole-search kernel
+                const float4 v = *reinterpret_cast<const float4*>(p.X + (size_t)(row0 + r) * 8), w = *reinterpret_cast<const float4*>(p.X + (size_t)(row0 + r) * 8 + 4);
+                x[0] = v.x; x[1] = v.y; x[2] = v.z; x[3] = v.w; x[4] = w.x; x[5] = w.y;
+            } else {
+                const float4 v = *reinterpret_cast<const float4*>(p.X + (size_t)(row0 + r) * 4);  // xstride 4 in the whole-search kernel
+                x[0] = v.x; x[1] = v.y;
+                if constexpr (S > 2) x[2] = v.z;
+                if (S > 3) x[S - 1] = v.w;
+            }
         }
 #pragma unroll
         for (int k = 0; k < 8; k += 2) {

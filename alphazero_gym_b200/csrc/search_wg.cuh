@@ -130,10 +130,15 @@ __device__ __forceinline__ void wg_evaluate(const MlpParams& p, WgSlot& sl, cons
 #pragma unroll
         for (int s = 0; s < S; ++s) x[s] = 0.0f;
         if (valid) {
-            const float4 v = *reinterpret_cast<const float4*>(p.X + (size_t)gr * 4);
-            x[0] = v.x; x[1] = v.y;
-            if constexpr (S > 2) x[2] = v.z;
-            if (S > 3) x[S - 1] = v.w;
+            if constexpr (S > 4) {  // Acrobot: 6 inputs in two float4 per leaf
+                const float4 v = *reinterpret_cast<const float4*>(p.X + (size_t)gr * 8), w = *reinterpret_cast<const float4*>(p.X + (size_t)gr * 8 + 4);
+                x[0] = v.x; x[1] = v.y; x[2] = v.z; x[3] = v.w; x[4] = w.x; x[5] = w.y;
+            } else {
+                const float4 v = *reinterpret_cast<const float4*>(p.X + (size_t)gr * 4);
+                x[0] = v.x; x[1] = v.y;
+                if constexpr (S > 2) x[2] = v.z;
+                if (S > 3) x[S - 1] = v.w;
+            }
         }
 #pragma unroll 1
         for (int c = 0; c < 8; ++c) {

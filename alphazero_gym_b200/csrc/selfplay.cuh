@@ -12,7 +12,7 @@
 //                                                              the root's edges, so only root.n survives (SURVEY 7-7)
 // Randomness: the engine is re-keyed for every step (azg_selfplay_step); stream 2 = the discrete agent's action draw,
 // stream 3 = Env.reset (gym: CartPole U(-0.05, 0.05)^4, Pendulum th ~ U(-pi, pi), thdot ~ U(-1, 1), MountainCarContinuous and
-// MountainCar position ~ U(-0.6, -0.4), velocity 0).
+// MountainCar position ~ U(-0.6, -0.4), velocity 0, Acrobot U(-0.1, 0.1)^4).
 #pragma once
 #include "common.cuh"
 #include "env.cuh"
@@ -23,7 +23,7 @@ struct SelfPlayParams {
     int64_t tree_id0;
     const uint64_t* seedp;
     // state (in/out)
-    double* env_state;   // [B][4|2]  (CartPole 4; MountainCar and the continuous envs 2)
+    double* env_state;   // [B][HS]  (CartPole and Acrobot 4; MountainCar and the continuous envs 2)
     int32_t* ep_step;    // [B]
     int32_t* episode;    // [B]
     int32_t* root_n;     // [B] discrete
@@ -33,13 +33,14 @@ struct SelfPlayParams {
     const double* Q;
     const int32_t* n_children;
     // outputs
-    float* obs;          // [B][S] observation the search started from (S = 4 | 3 | 2)
+    float* obs;          // [B][S] observation the search started from (S = 6 | 4 | 3 | 2)
     float* action_taken; // [B]
     double* reward;      // [B]
     int32_t* done;       // [B]
     // discrete tree tables (root.n carry-over)
     const DRow* drows;
     int32_t R;
+    int32_t* err;        // ERR_WRAP (Acrobot's real env step)
 };
 
 __device__ __forceinline__ double u32_to_unit_f64(uint32_t x) { return ((double)x + 0.5) * 2.3283064365386963e-10; }
@@ -160,28 +161,63 @@ __global__ void k_selfplay_discrete(const SelfPlayParams p) {
             const double last = cdf[A - 1];
             for (int i = 0; i < A - 1; ++i) a += (u >= cdf[i] / last) ? 1 : 0;
         }
-        const double pos = p.env_state[(size_t)t * 2], vel = p.env_state[(size_t)t * 2 + 1];
-        const float4 ob = ENV::obs(pos, vel);
-        p.obs[(size_t)t * 2] = ob.x; p.obs[(size_t)t * 2 + 1] = ob.y;
-        double npos, nvel, rew;
-        const bool term = ENV::step(pos, vel, a, npos, nvel, rew);
-        const int step = p.ep_step[t] + 1;
-        const bool done = term || step >= p.max_episode_length;
+        // the env step, Env.reset() + reset_mcts when done, else mcts_forward: the chosen child keeps its visit count.  MountainCar's
+        // two-wide state stays in scalars as it always was (which keeps that kernel's code unchanged); wider hidden states in arrays.
+        double rew;
+        bool done;
         int root_n = 0;
-        if (done) {  // Env.reset() + reset_mcts
-            const int ep = p.episode[t] + 1;
-            const u32x4 r = rng_block(__ldg(p.seedp), p.tree_id0 + t, 3, ep, 0);
-            ENV::reset(u32_to_unit_f64(r.x), u32_to_unit_f64(r.y), npos, nvel);
-            p.episode[t] = ep;
-        } else {  // mcts_forward: the chosen child keeps its visit count
-            const D3Row* rows = reinterpret_cast<const D3Row*>(p.drows) + (size_t)t * p.R;
-            const uint16_t child = rows[0].child[a];
-            root_n = child == DROW_NONE ? 0 : rows[child].node_n;
+        if constexpr (ENV::HS == 2) {
+            const double pos = p.env_state[(size_t)t * 2], vel = p.env_state[(size_t)t * 2 + 1];
+            const float4 ob = ENV::obs(pos, vel);
+            p.obs[(size_t)t * 2] = ob.x; p.obs[(size_t)t * 2 + 1] = ob.y;
+            double npos, nvel;
+            const bool term = ENV::step(pos, vel, a, npos, nvel, rew);
+            const int step = p.ep_step[t] + 1;
+            done = term || step >= p.max_episode_length;
+            if (done) {
+                const int ep = p.episode[t] + 1;
+                const u32x4 r = rng_block(__ldg(p.seedp), p.tree_id0 + t, 3, ep, 0);
+                ENV::reset(u32_to_unit_f64(r.x), u32_to_unit_f64(r.y), npos, nvel);
+                p.episode[t] = ep;
+            } else {
+                const D3Row* rows = reinterpret_cast<const D3Row*>(p.drows) + (size_t)t * p.R;
+                const uint16_t child = rows[0].child[a];
+                root_n = child == DROW_NONE ? 0 : rows[child].node_n;
+            }
+            p.ep_step[t] = done ? 0 : step;
+            p.root_n[t] = root_n;
+            p.env_state[(size_t)t * 2] = npos;
+            p.env_state[(size_t)t * 2 + 1] = nvel;
+        } else {
+            constexpr int HS = ENV::HS, S = ENV::S;
+            double h[HS], o[HS];
+#pragma unroll
+            for (int k = 0; k < HS; ++k) h[k] = p.env_state[(size_t)t * HS + k];
+            float4 ob[ENV::XW];
+            ENV::input(h, ob);
+#pragma unroll
+            for (int k = 0; k < S; ++k) p.obs[(size_t)t * S + k] = reinterpret_cast<const float*>(ob)[k];
+            bool capped = false;
+            const bool term = ENV::expand(h, a, o, rew, capped);
+            if (capped) atomicOr(p.err, ERR_WRAP);
+            const int step = p.ep_step[t] + 1;
+            done = term || step >= p.max_episode_length;
+            if (done) {
+                const int ep = p.episode[t] + 1;
+                const u32x4 r = rng_block(__ldg(p.seedp), p.tree_id0 + t, 3, ep, 0);
+                const double u[4] = {u32_to_unit_f64(r.x), u32_to_unit_f64(r.y), u32_to_unit_f64(r.z), u32_to_unit_f64(r.w)};
+                ENV::reset(u, o);
+                p.episode[t] = ep;
+            } else {
+                const D3Row* rows = reinterpret_cast<const D3Row*>(p.drows) + (size_t)t * p.R;
+                const uint16_t child = rows[0].child[a];
+                root_n = child == DROW_NONE ? 0 : rows[child].node_n;
+            }
+            p.ep_step[t] = done ? 0 : step;
+            p.root_n[t] = root_n;
+#pragma unroll
+            for (int k = 0; k < HS; ++k) p.env_state[(size_t)t * HS + k] = o[k];
         }
-        p.ep_step[t] = done ? 0 : step;
-        p.root_n[t] = root_n;
-        p.env_state[(size_t)t * 2] = npos;
-        p.env_state[(size_t)t * 2 + 1] = nvel;
         p.action_taken[t] = (float)a;
         p.reward[t] = rew;
         p.done[t] = done ? 1 : 0;

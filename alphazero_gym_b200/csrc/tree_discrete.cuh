@@ -42,7 +42,7 @@ __device__ __forceinline__ D3Row d3_row(uint16_t parent, int paction, double r, 
 // root row + first network input (MCTSDiscrete.initialize_search, mcts.py:364-383)
 template <class ENV>
 __device__ __forceinline__ void d_init(const TreeParams& p, int t) {
-    const double* s = p.root_state + (size_t)t * ENV::S;  // the root's hidden state (MountainCar: the observation is the state)
+    const double* s = p.root_state + (size_t)t * ENV::HS;  // the root's hidden state
     double* st = p.dstate + (size_t)t * p.R * 4;
     if constexpr (ENV::A == 2) {
         DRow row;
@@ -73,8 +73,9 @@ __device__ __forceinline__ void d_init(const TreeParams& p, int t) {
             for (int k = 0; k < 3; ++k) row.prior[k] = p.tapeP[(size_t)t * p.R * 3 + k];
         }
         reinterpret_cast<D3Row*>(p.drows)[(size_t)t * p.R] = row;
-        st[0] = s[0]; st[1] = s[1];
-        p.X[t] = ENV::obs(s[0], s[1]);
+#pragma unroll
+        for (int k = 0; k < ENV::HS; ++k) st[k] = s[k];
+        ENV::input(s, p.X + (size_t)t * ENV::XW);  // the root's observation, from its hidden state
     }
     p.leaf[t] = 0 | LEAF_EVAL;
     p.n_rows[t] = 1;
@@ -90,8 +91,8 @@ __global__ void k_init_discrete(const TreeParams p) {
 
 // one simulation step of tree t: backup of the previous simulation (BACKUP), then descent + expansion of the next (SELECT).
 // Shared by k_step_discrete (one launch per simulation) and the whole-search kernels (qmlp2.cuh, search_wg.cuh).
-// ENV::A = 2 (CartPole): DRow, path entries (row << 1 | action).  ENV::A = 3 (MountainCar): D3Row, path entries (row << 2 | action);
-// the descent reads line 0 of a row, the backup also reads r from line 1.
+// ENV::A = 2 (CartPole): DRow, path entries (row << 1 | action).  ENV::A = 3 (MountainCar, Acrobot): D3Row, path entries
+// (row << 2 | action); the descent reads line 0 of a row, the backup also reads r from line 1.
 template <class ENV>
 __device__ __forceinline__ void d_step(const TreeParams& p, const Tabs& tb, int t, const bool BACKUP, const bool SELECT) {
     constexpr int A = ENV::A, PSH = A == 2 ? 1 : 2;  // path entry: row << PSH | action
@@ -330,10 +331,15 @@ __device__ __forceinline__ void d_step(const TreeParams& p, const Tabs& tb, int 
                 rows[cur].child[a] = (uint16_t)child;
                 p.X[t] = make_float4((float)o[0], (float)o[1], (float)o[2], (float)o[3]);
             } else {
-                double o0, o1, rew;
-                term = ENV::step(st[0], st[1], a, o0, o1, rew);  // Node.r = the env's reward
+                double h[ENV::HS], o[ENV::HS], rew;
+                bool capped = false;
+#pragma unroll
+                for (int k = 0; k < ENV::HS; ++k) h[k] = st[k];
+                term = ENV::expand(h, a, o, rew, capped);  // Node.r = the env's reward
+                if (capped) atomicOr(p.err, ERR_WRAP);
                 double* so = p.dstate + ((size_t)t * p.R + child) * 4;
-                so[0] = o0; so[1] = o1;
+#pragma unroll
+                for (int k = 0; k < ENV::HS; ++k) so[k] = o[k];
                 D3Row nr = d3_row((uint16_t)cur, a, rew, term);
                 if (p.use_tape) {
                     const size_t ti = (size_t)t * p.R + child;
@@ -342,7 +348,7 @@ __device__ __forceinline__ void d_step(const TreeParams& p, const Tabs& tb, int 
                 }
                 rows3[child] = nr;
                 rows3[cur].child[a] = (uint16_t)child;
-                p.X[t] = ENV::obs(o0, o1);
+                ENV::input(o, p.X + (size_t)t * ENV::XW);
             }
             p.leaf[t] = child | LEAF_EVAL | (term ? LEAF_TERMINAL : 0);
         } else {

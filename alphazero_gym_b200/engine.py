@@ -17,7 +17,7 @@ from ._cabi import ACT_ELU, ACT_RELU, CONTINUOUS, DISCRETE, VT, AzgConfig, check
 
 # the envs the engine steps (gym ids); the discrete search steps CartPole-v0 and the continuous search Pendulum-v0 unless told otherwise
 CARTPOLE, PENDULUM, MOUNTAIN_CAR_CONTINUOUS = "CartPole-v0", "Pendulum-v0", "MountainCarContinuous-v0"
-MOUNTAIN_CAR = "MountainCar-v0"
+MOUNTAIN_CAR, ACROBOT = "MountainCar-v0", "Acrobot-v1"
 
 
 @dataclass
@@ -54,7 +54,7 @@ class EngineConfig:
     fused: Optional[bool] = None  # AZG_FLAG_FUSED: whole search in one persistent kernel; None = on where supported (eval_q8)
     # the env the search steps: None = the variant's own (CartPole-v0 / Pendulum-v0); MOUNTAIN_CAR_CONTINUOUS (continuous variant,
     # state_dim 2) sets AZG_FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS; MOUNTAIN_CAR (discrete variant, num_actions 3, state_dim 2) sets
-    # AZG_FLAG_ENV_MOUNTAIN_CAR
+    # AZG_FLAG_ENV_MOUNTAIN_CAR; ACROBOT (discrete variant, num_actions 3, state_dim 6) sets AZG_FLAG_ENV_ACROBOT
     env: Optional[str] = None
 
     def c(self) -> AzgConfig:
@@ -65,16 +65,17 @@ class EngineConfig:
                          (0 if self.use_graph else _cabi.FLAG_NO_GRAPH) | (_cabi.FLAG_EVAL_Q8 if self.is_q8() else 0)
                          | (_cabi.FLAG_FUSED if self.is_fused() else 0) | (_cabi.FLAG_RNG_MT19937 if self.rng_mt19937 else 0)
                          | (_cabi.FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS if self.env_name() == MOUNTAIN_CAR_CONTINUOUS else 0)
-                         | (_cabi.FLAG_ENV_MOUNTAIN_CAR if self.env_name() == MOUNTAIN_CAR else 0), self.seed)
+                         | (_cabi.FLAG_ENV_MOUNTAIN_CAR if self.env_name() == MOUNTAIN_CAR else 0)
+                         | (_cabi.FLAG_ENV_ACROBOT if self.env_name() == ACROBOT else 0), self.seed)
 
     def env_name(self) -> str:
         if self.env is None:
             return CARTPOLE if self.variant == DISCRETE else PENDULUM
-        if self.env not in (CARTPOLE, PENDULUM, MOUNTAIN_CAR_CONTINUOUS, MOUNTAIN_CAR):
-            raise ValueError(f"unknown env {self.env!r}: the engine steps {CARTPOLE}, {MOUNTAIN_CAR}, {PENDULUM} and "
+        if self.env not in (CARTPOLE, PENDULUM, MOUNTAIN_CAR_CONTINUOUS, MOUNTAIN_CAR, ACROBOT):
+            raise ValueError(f"unknown env {self.env!r}: the engine steps {CARTPOLE}, {MOUNTAIN_CAR}, {ACROBOT}, {PENDULUM} and "
                              f"{MOUNTAIN_CAR_CONTINUOUS}")
-        if self.env == MOUNTAIN_CAR and self.variant != DISCRETE:
-            raise ValueError(f"{MOUNTAIN_CAR} has discrete actions: it is searched by the discrete variant")
+        if self.env in (MOUNTAIN_CAR, ACROBOT) and self.variant != DISCRETE:
+            raise ValueError(f"{self.env} has discrete actions: it is searched by the discrete variant")
         return self.env
 
     def q8_supported(self) -> bool:
@@ -85,7 +86,7 @@ class EngineConfig:
         return self.q8_supported() if self.eval_q8 is None else bool(self.eval_q8)
 
     def is_fused(self) -> bool:
-        env_dim = {CARTPOLE: 4, PENDULUM: 3, MOUNTAIN_CAR_CONTINUOUS: 2, MOUNTAIN_CAR: 2}[self.env_name()]
+        env_dim = {CARTPOLE: 4, PENDULUM: 3, MOUNTAIN_CAR_CONTINUOUS: 2, MOUNTAIN_CAR: 2, ACROBOT: 6}[self.env_name()]
         supported = (self.is_q8() and self.state_dim == env_dim
                      and not (self.rng_mt19937 and self.variant == CONTINUOUS))  # the torch-generator mode runs one launch per simulation
         return supported if self.fused is None else bool(self.fused)
@@ -121,7 +122,7 @@ class SearchEngine:
         self.cmax = self._lib.azg_cmax(h)
         self.head_dim = self._lib.azg_head_dim(h)
         self.num_weights = self._lib.azg_num_weights(h)
-        self.state_cols = 4 if cfg.variant == DISCRETE and cfg.env_name() == CARTPOLE else 2  # hidden-state width
+        self.state_cols = 4 if cfg.variant == DISCRETE and cfg.env_name() in (CARTPOLE, ACROBOT) else 2  # hidden-state width
         self._keep = {}
         self.last_B = 0
 
@@ -157,7 +158,7 @@ class SearchEngine:
     # ---- device-resident path ------------------------------------------------------------------------
     def search(self, root_state: torch.Tensor, n_rollouts: int, root_n_init: Optional[torch.Tensor] = None,
                tree_id0: int = 0) -> None:
-        """Batched search; root_state is a CUDA f64 tensor [B, 4|2] (CartPole 4, the other envs 2).  Asynchronous on the current stream."""
+        """Batched search; root_state is a CUDA f64 tensor [B, 4|2] (CartPole and Acrobot 4, the other envs 2).  Asynchronous on the current stream."""
         assert root_state.is_cuda and root_state.dtype == torch.float64 and root_state.is_contiguous()
         B = root_state.shape[0]
         assert root_state.shape[1] == self.state_cols

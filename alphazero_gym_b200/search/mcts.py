@@ -8,7 +8,7 @@ upstream call form `search(n_mcts, c, Env, mcts_env)` named in BASELINE.json is 
 What changes underneath: the tree lives in HBM tables and the whole search -- select, env step, network
 evaluation, backup -- runs in the CUDA engine (csrc/, C ABI include/azg.h).  `model` is only read for its
 weights and shape; `Env` only for its hidden state (`Env.unwrapped.state`) and its class name.  Envs other than
-CartPole and MountainCar (MCTSDiscrete), Pendulum and MountainCarContinuous (MCTSContinuous) raise: there is no CPU fallback.  Tie-break / epsilon-greedy / action-noise randomness comes from
+CartPole, MountainCar and Acrobot (MCTSDiscrete), Pendulum and MountainCarContinuous (MCTSContinuous) raise: there is no CPU fallback.  Tie-break / epsilon-greedy / action-noise randomness comes from
 the engine's counter-based Philox streams keyed by (`seed`, search counter) instead of Python's `random` and
 torch's global generator.
 
@@ -22,7 +22,7 @@ from typing import Any, Dict, Optional, Tuple
 import numpy as np
 
 from .._cabi import CONTINUOUS, DISCRETE
-from ..engine import CARTPOLE, MOUNTAIN_CAR, MOUNTAIN_CAR_CONTINUOUS, PENDULUM, EngineConfig, SearchEngine, flatten_state_dict
+from ..engine import ACROBOT, CARTPOLE, MOUNTAIN_CAR, MOUNTAIN_CAR_CONTINUOUS, PENDULUM, EngineConfig, SearchEngine, flatten_state_dict
 from ..network import describe_model, weights_version
 
 PENDULUM_R_SCALE = 16.2736044  # reference mcts.py:20 (applied inside the engine)
@@ -66,6 +66,8 @@ def reward_model(env, variant: int):
         raise NotImplementedError(f"{names[0]} around MountainCarContinuous-v0: the CUDA engine steps the plain env only")
     if names and variant == DISCRETE and _is_mountain_car(base):
         raise NotImplementedError(f"{names[0]} around MountainCar-v0: the CUDA engine steps the plain env only")
+    if names and variant == DISCRETE and _is_acrobot(base):
+        raise NotImplementedError(f"{names[0]} around Acrobot-v1: the CUDA engine steps the plain env only")
     step, terminal = 1.0, 1.0  # gym CartPole-v0 pays 1.0 for every step, the terminating one included
     for name in reversed(names):
         if name == "ReparametrizeWrapper":
@@ -87,10 +89,20 @@ def _is_mountain_car(base) -> bool:
     return type(base).__name__ == "MountainCarEnv"  # gym's class (classic_control/mountain_car.py)
 
 
+def _is_acrobot(base) -> bool:
+    return type(base).__name__ == "AcrobotEnv"  # gym's class (classic_control/acrobot.py)
+
+
+def acrobot_obs(s: np.ndarray) -> np.ndarray:
+    """AcrobotEnv._get_ob of the hidden state (theta1, theta2, dtheta1, dtheta2): what the network sees."""
+    return np.array([np.cos(s[0]), np.sin(s[0]), np.cos(s[1]), np.sin(s[1]), s[2], s[3]])
+
+
 def discrete_env(env) -> str:
-    """The env MCTSDiscrete has the engine step for `env`: MountainCar-v0 for gym's MountainCarEnv (by class name, under any
-    wrappers), CartPole-v0 otherwise (env_hidden_state refuses the envs that are neither)."""
-    return MOUNTAIN_CAR if _is_mountain_car(_unwrap(env)) else CARTPOLE
+    """The env MCTSDiscrete has the engine step for `env`: MountainCar-v0 for gym's MountainCarEnv and Acrobot-v1 for its AcrobotEnv
+    (by class name, under any wrappers), CartPole-v0 otherwise (env_hidden_state refuses the envs that are none of these)."""
+    base = _unwrap(env)
+    return MOUNTAIN_CAR if _is_mountain_car(base) else (ACROBOT if _is_acrobot(base) else CARTPOLE)
 
 
 def continuous_env(env) -> str:
@@ -101,16 +113,22 @@ def continuous_env(env) -> str:
 
 def env_hidden_state(env, variant: int, env_id: Optional[str] = None) -> np.ndarray:
     """Root of the search = hidden state of the gym env (replaces copy.deepcopy(Env), mcts.py:443, :680).  env_id = MOUNTAIN_CAR
-    accepts gym's MountainCarEnv for the discrete variant (a 2-wide state); without it the search classes' original envs only."""
+    accepts gym's MountainCarEnv for the discrete variant (a 2-wide state), env_id = ACROBOT its AcrobotEnv (a 4-wide state); without
+    it the search classes' original envs only."""
     base = _unwrap(env)
     if not hasattr(base, "state") or base.state is None:
-        raise TypeError("Env has no hidden `.state`; only gym CartPole-v0 / MountainCar-v0 / Pendulum-v0 / MountainCarContinuous-v0 style "
-                        "envs are supported")
+        raise TypeError("Env has no hidden `.state`; only gym CartPole-v0 / MountainCar-v0 / Acrobot-v1 / Pendulum-v0 / "
+                        "MountainCarContinuous-v0 style envs are supported")
     s = np.asarray(base.state, dtype=np.float64).reshape(-1)
     if env_id == MOUNTAIN_CAR:
         if variant != DISCRETE or not _is_mountain_car(base) or s.size != 2:
             raise TypeError(f"unsupported environment {type(base).__name__} for MountainCar-v0: the discrete search steps gym's "
                             "MountainCarEnv (a 2-wide state)")
+        return s
+    if env_id == ACROBOT:
+        if variant != DISCRETE or not _is_acrobot(base) or s.size != 4:
+            raise TypeError(f"unsupported environment {type(base).__name__} for Acrobot-v1: the discrete search steps gym's "
+                            "AcrobotEnv (a 4-wide state)")
         return s
     name = type(base).__name__.lower()
     want = 4 if variant == DISCRETE else 2
@@ -223,9 +241,10 @@ class MCTS:
 
 
 class MCTSDiscrete(MCTS):
-    """AlphaZero search for CartPole-v0 and MountainCar-v0 (reference mcts.py:310-526).  The env is taken from the Env each search()
-    is handed (discrete_env); search_batch steps the env of the last search(), or the engine keyword `env` (engine.CARTPOLE by
-    default)."""
+    """AlphaZero search for CartPole-v0, MountainCar-v0 and Acrobot-v1 (reference mcts.py:310-526).  The env is taken from the Env
+    each search() is handed (discrete_env); search_batch steps the env of the last search(), or the engine keyword `env`
+    (engine.CARTPOLE by default), from hidden states.  For Acrobot-v1 the root's state (return_results) and the state forward() takes
+    are the 6-wide observation (AcrobotEnv._get_ob), while the engine searches from the 4-wide hidden state."""
 
     variant = DISCRETE
 
@@ -249,10 +268,10 @@ class MCTSDiscrete(MCTS):
             self.close()
             self.n_rollouts, self.c_uct = n_mcts, c
         env = discrete_env(Env)
-        if env == MOUNTAIN_CAR:
+        if env in (MOUNTAIN_CAR, ACROBOT):
             if self.num_actions != 3:
-                raise ValueError(f"MountainCar-v0 has 3 actions, the search was built with num_actions={self.num_actions}")
-            hidden = env_hidden_state(Env, DISCRETE, env_id=MOUNTAIN_CAR)
+                raise ValueError(f"{env} has 3 actions, the search was built with num_actions={self.num_actions}")
+            hidden = env_hidden_state(Env, DISCRETE, env_id=env)
         else:
             hidden = env_hidden_state(Env, DISCRETE)
         if env != self._env:  # the engines are built for one env
@@ -260,7 +279,11 @@ class MCTSDiscrete(MCTS):
             self._env = env
         # initialize_search (mcts.py:364-383): new root, or continue from the node forward() selected
         if self.root_node is None:
-            self.root_node = RootNode(np.asarray(self.root_state if self.root_state is not None else hidden), n=0, hidden=hidden)
+            if self.root_state is not None:
+                obs = self.root_state
+            else:
+                obs = acrobot_obs(hidden) if env == ACROBOT else hidden
+            self.root_node = RootNode(np.asarray(obs), n=0, hidden=hidden)
         if self.root_node.terminal:
             raise ValueError("Can't do tree search from a terminal node")
         eng = self._engine(1)
@@ -281,7 +304,8 @@ class MCTSDiscrete(MCTS):
             self.root_node, self.root_state = None, state
             return
         child_state = t["state"][0, child]
-        if np.linalg.norm(child_state - np.asarray(state, np.float64).reshape(-1)) > 0.01:
+        child_obs = acrobot_obs(child_state) if self._env == ACROBOT else child_state  # what the agent's `state` is
+        if np.linalg.norm(child_obs - np.asarray(state, np.float64).reshape(-1)) > 0.01:
             print("Warning: this domain seems stochastic. Not re-using the subtree for next search. "
                   + "To deal with stochastic environments, implement progressive widening.")
             self.root_node, self.root_state = None, state

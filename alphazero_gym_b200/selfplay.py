@@ -17,7 +17,7 @@ import torch
 
 from . import _cabi
 from ._cabi import CONTINUOUS, DISCRETE, check
-from .engine import MOUNTAIN_CAR, MOUNTAIN_CAR_CONTINUOUS, SearchEngine
+from .engine import ACROBOT, MOUNTAIN_CAR, MOUNTAIN_CAR_CONTINUOUS, SearchEngine
 from .parallel import PackedRows, allgather_results, broadcast_weights
 
 ROW_KEYS = ("obs", "actions", "counts", "Q", "V_target")  # buffer.store((s, actions, counts, Qs, V)), buffers.py:61
@@ -27,7 +27,7 @@ def initial_states(variant: int, B: int, seed: int = 34, tree_id0: int = 0, tota
                    env: Optional[str] = None) -> np.ndarray:
     """Env.reset() for every environment: the same rule as SURVEY 8d configs 3/4 (numpy default_rng(seed) over the GLOBAL
     batch, this shard's slice).  env (engine.EngineConfig.env): MOUNTAIN_CAR (discrete) and MOUNTAIN_CAR_CONTINUOUS draw
-    position ~ U(-0.6, -0.4), velocity 0."""
+    position ~ U(-0.6, -0.4), velocity 0; ACROBOT draws the four state entries ~ U(-0.1, 0.1)."""
     if total is None:
         # the draw below runs over the GLOBAL batch, so every rank must use the same `total`: tree_id0 + B is only right for a
         # single shard (or the last one)
@@ -35,7 +35,9 @@ def initial_states(variant: int, B: int, seed: int = 34, tree_id0: int = 0, tota
             raise ValueError("initial_states: pass total (the global number of environments) when torch.distributed is initialised")
         total = tree_id0 + B
     rng = np.random.default_rng(seed)
-    if variant == DISCRETE and env != MOUNTAIN_CAR:
+    if variant == DISCRETE and env == ACROBOT:
+        s = rng.uniform(-0.1, 0.1, size=(total, 4))
+    elif variant == DISCRETE and env != MOUNTAIN_CAR:
         s = rng.uniform(-0.05, 0.05, size=(total, 4))
     elif env in (MOUNTAIN_CAR, MOUNTAIN_CAR_CONTINUOUS):
         s = np.stack([rng.uniform(-0.6, -0.4, total), np.zeros(total)], 1)

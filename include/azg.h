@@ -29,8 +29,11 @@ extern "C" {
 #define AZG_ETERMINAL -3   /* "Can't do tree search from a terminal node" (mcts.py:382-383, :599-600) */
 #define AZG_ENAN -4        /* NaN met in a UCT vector (helpers.py:47-48 only warns; we refuse) */
 #define AZG_ECAPACITY -5   /* tree arena / child fan-out capacity exceeded */
+#define AZG_EWRAP -6       /* Acrobot-v1: an angle needed more than 64 iterations of gym's wrap loop (an infinite or huge angle, on
+                              which gym would loop for that long or forever); the search's results are not gym's */
 
-#define AZG_DISCRETE 0   /* MCTSDiscrete  + CartPole-v0 dynamics (or, with AZG_FLAG_ENV_MOUNTAIN_CAR, MountainCar-v0) + DiscretePolicy */
+#define AZG_DISCRETE 0   /* MCTSDiscrete  + CartPole-v0 dynamics (or, with AZG_FLAG_ENV_MOUNTAIN_CAR, MountainCar-v0; with AZG_FLAG_ENV_ACROBOT,
+                            Acrobot-v1) + DiscretePolicy */
 #define AZG_CONTINUOUS 1 /* MCTSContinuous + Pendulum-v0 (or, with AZG_FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS, MountainCarContinuous-v0)
                            dynamics + DiagonalNormal/GMM policy */
 
@@ -52,9 +55,9 @@ typedef struct azg_config {
     int32_t variant;        /* AZG_DISCRETE | AZG_CONTINUOUS */
     int32_t max_rollouts;   /* capacity: largest n_rollouts a search call may ask for */
     int32_t max_trees;      /* capacity: largest batch B */
-    int32_t num_actions;    /* discrete: 2 (CartPole), 3 (MountainCar-v0) */
+    int32_t num_actions;    /* discrete: 2 (CartPole), 3 (MountainCar-v0, Acrobot-v1) */
     int32_t num_components; /* continuous: K mixture components (1 = DiagonalNormalPolicy) */
-    int32_t state_dim;      /* network input width: 4 CartPole, 3 Pendulum, 2 MountainCarContinuous and MountainCar */
+    int32_t state_dim;      /* network input width: 4 CartPole, 3 Pendulum, 2 MountainCarContinuous and MountainCar, 6 Acrobot */
     int32_t hidden;         /* hidden width (all hidden layers equal; 128 in both shipped configs) */
     int32_t n_hidden;       /* hidden layers: 2 (DiscretePolicy.yaml) / 3 (ContinuousPolicy.yaml) */
     int32_t activation;     /* AZG_ACT_* */
@@ -109,6 +112,17 @@ typedef struct azg_config {
                                    (thin batches run the two-phase kernel).  Hidden-state arrays (search roots, d_env_state, the dump's
                                    state, azg_env_step) are 2 wide; results and dump arrays carry 3 actions.  The reward model
                                    (azg_set_reward_model) stays the identity. */
+#define AZG_FLAG_ENV_ACROBOT 64u /* discrete variant only, with num_actions 3 and state_dim 6 (not with either MountainCar flag): the
+                                   search steps Acrobot-v1 (gym 0.17-0.19 acrobot.py: book dynamics, RK4 over dt = 0.2, no torque
+                                   noise) instead of CartPole-v0.  Hidden state (theta1, theta2, dtheta1, dtheta2); network input the
+                                   observation (float)cos theta1, sin theta1, cos theta2, sin theta2, dtheta1, dtheta2; actions 0, 1, 2
+                                   (torque -1, 0, +1); Node.r is the env's reward, -1.0 before the goal and 0.0 at it; an episode ends
+                                   at the goal.  gym's wrap loop is capped: a search or env step that reaches the cap fails with
+                                   AZG_EWRAP.  The tree holds 128-byte three-action rows, so max_rollouts <= 16382.  Every schedule and
+                                   every other flag apply, except the trees-in-shared-memory whole-search kernel (thin batches run the
+                                   two-phase kernel).  Hidden-state arrays (search roots, d_env_state, the dump's state, azg_env_step)
+                                   are 4 wide; observations (azg_env_step's d_obs, the self-play d_obs) are 6 wide; results and dump
+                                   arrays carry 3 actions.  The reward model (azg_set_reward_model) stays the identity. */
 
 typedef struct azg_engine azg_engine;
 
@@ -124,8 +138,9 @@ const char* azg_version(void);
 int64_t azg_num_weights(const azg_engine* e);
 int azg_set_weights(azg_engine* e, const float* flat, int64_t n, void* stream);
 
-/* Batched MCTSDiscrete.search (mcts.py:418-462) over B CartPole (or MountainCar-v0) roots.
- * d_root_state [B][4] f64 hidden env state (x, x_dot, theta, theta_dot); MountainCar [B][2] (position, velocity);
+/* Batched MCTSDiscrete.search (mcts.py:418-462) over B CartPole (or MountainCar-v0, Acrobot-v1) roots.
+ * d_root_state [B][4] f64 hidden env state (x, x_dot, theta, theta_dot); MountainCar [B][2] (position, velocity); Acrobot [B][4]
+ * (theta1, theta2, dtheta1, dtheta2);
  * d_root_n_init [B] carried-over root visit count after forward() (mcts.py:495-526) or NULL;
  * tree_id0: global id of tree 0 -- tree i's RNG streams are keyed by tree_id0+i, which makes results
  * independent of batch composition and of how trees are sharded over GPUs. */
@@ -159,7 +174,8 @@ int azg_search_host_begin(azg_engine* e, int32_t slot, int32_t B, const double* 
                           int32_t* h_n_children);
 int azg_search_host_end(azg_engine* e, int32_t slot);
 
-/* Device status of the last search(es): AZG_OK, AZG_ENAN or AZG_ECAPACITY.  Synchronises `stream`. */
+/* Device status of the last search(es), self-play steps and env steps: AZG_OK, AZG_ENAN, AZG_ECAPACITY or AZG_EWRAP.  Synchronises
+ * `stream`. */
 int azg_status(azg_engine* e, void* stream);
 
 /* Re-key the Philox streams (tie-break / eps-greedy / action noise / self-play draws).  Stream-ordered: searches enqueued
@@ -189,7 +205,8 @@ int azg_set_reward_model(azg_engine* e, double reward_step, double reward_termin
  *   (reset_mcts), else discrete tree reuse: d_root_n = visit count of the chosen child (mcts.py:495-526).
  * All pointers are device pointers owned by the caller; in/out arrays carry the state from step to step. */
 typedef struct azg_selfplay_io {
-    double* d_env_state;   /* in/out [B][4|2] hidden env state (CartPole x, x_dot, theta, theta_dot | MountainCar position, velocity | Pendulum th, thdot |
+    double* d_env_state;   /* in/out [B][4|2] hidden env state (CartPole x, x_dot, theta, theta_dot | Acrobot theta1, theta2, dtheta1, dtheta2 |
+                              MountainCar position, velocity | Pendulum th, thdot |
                               MountainCarContinuous position, velocity) */
     int32_t* d_ep_step;    /* in/out [B] steps taken in the current episode */
     int32_t* d_episode;    /* in/out [B] episode counter (indexes the reset stream) */
@@ -225,7 +242,7 @@ typedef struct azg_dump_discrete { /* host arrays, R = azg_rows(e), A = num_acti
     int32_t* terminal; /* [B][R] */
     float* V;          /* [B][R] */
     double* r;         /* [B][R] */
-    double* state;     /* [B][R][4]; MountainCar [B][R][2] */
+    double* state;     /* [B][R][4]; MountainCar [B][R][2] (Acrobot 4) */
     float* prior;      /* [B][R][A] */
     double* eW;        /* [B][R][A] Action.W */
     int32_t* en;       /* [B][R][A] Action.n */
@@ -275,7 +292,7 @@ int32_t azg_head_dim(const azg_engine* e);
 int azg_mlp_forward(azg_engine* e, int32_t n, const float* d_x, float* d_V, float* d_head, void* stream);
 
 /* Batched env.step of the engine's env on its own (known-answer tests): d_state [n][4|2] (CartPole 4, MountainCar and the continuous
- * envs 2), d_action [n] (index as float for CartPole and MountainCar) -> d_next [n][4|2], d_reward [n] (raw env reward), d_terminal [n], d_obs [n][state_dim]. */
+ * envs 2; Acrobot 4), d_action [n] (index as float for CartPole, MountainCar and Acrobot) -> d_next [n][4|2], d_reward [n] (raw env reward), d_terminal [n], d_obs [n][state_dim]. */
 int azg_env_step(azg_engine* e, int32_t n, const double* d_state, const float* d_action, double* d_next, double* d_reward,
                  int32_t* d_terminal, float* d_obs, void* stream);
 
