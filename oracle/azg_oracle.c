@@ -531,23 +531,146 @@ static void pendulum_obs(const azo_config* c, const double* s, float* obs) {
     obs[2] = (float)s[1];
 }
 
-int azo_env_step(const azo_config* c, const double* s_in, float action, double* s_out, double* reward, float* obs) {
-    int term;
-    if (c->variant == AZO_DISCRETE) {
-        term = cartpole_step(c, s_in, (int)action, s_out, reward);
-        if (obs) for (int i = 0; i < 4; ++i) obs[i] = (float)s_out[i];
-    } else {
-        term = pendulum_step(c, s_in, action, s_out, reward);
-        if (obs) pendulum_obs(c, s_out, obs);
+/* MountainCarContinuous-v0.  The f32 action enters f64 arithmetic exactly (numpy-1.x promotion); force = min(max(a, -1.0), 1.0) with
+ * Python's max / min (a NaN passes, -0 stays -0); velocity + ((force * power) - (0.0025 * cos(3 * position))); the left wall sets
+ * velocity to +0; done = position >= 0.45 and velocity >= 0; reward (done ? 100.0 : 0.0) - pow(a, 2) * 0.1 on the unclipped action
+ * (0 - x with the int 0 is 0.0 - x: +0 for a zero action; pow(a, 2) of an f32 is exact in f64). */
+static int mountain_car_continuous_step(const azo_config* c, const double* s, float action, double* o, double* reward) {
+    const double min_position = -1.2, max_position = 0.6, max_speed = 0.07, goal_position = 0.45, power = 0.0015;
+    double pos = s[0], vel = s[1];
+    const double a = (double)action;
+    double force = -1.0 > a ? -1.0 : a;
+    force = 1.0 < force ? 1.0 : force;
+    vel = vel + (force * power - 0.0025 * m_cos(c, 3 * pos));
+    if (vel > max_speed) vel = max_speed;
+    if (vel < -max_speed) vel = -max_speed;
+    pos = pos + vel;
+    if (pos > max_position) pos = max_position;
+    if (pos < min_position) pos = min_position;
+    if (pos == min_position && vel < 0) vel = 0.0;
+    const int done = pos >= goal_position && vel >= 0.0;
+    *reward = (done ? 100.0 : 0.0) - (a * a) * 0.1;
+    o[0] = pos; o[1] = vel;
+    return done;
+}
+
+/* MountainCar-v0.  velocity += (action - 1) * force + cos(3 * position) * (-gravity), the right-hand side summed first ((action - 1) *
+ * force is an int times a float); np.clip on velocity and position (a NaN passes, -0 stays -0); the left wall stores the int 0 (+0 from
+ * then on); done = position >= 0.5 and velocity >= 0 (false for a NaN); reward -1.0 on every step. */
+static int mountain_car_step(const azo_config* c, const double* s, int action, double* o, double* reward) {
+    const double min_position = -1.2, max_position = 0.6, max_speed = 0.07, goal_position = 0.5, force = 0.001, gravity = 0.0025;
+    double pos = s[0], vel = s[1];
+    vel = vel + ((double)(action - 1) * force + m_cos(c, 3 * pos) * -gravity);
+    vel = vel < -max_speed ? -max_speed : (vel > max_speed ? max_speed : vel);
+    pos = pos + vel;
+    pos = pos < min_position ? min_position : (pos > max_position ? max_position : pos);
+    if (pos == min_position && vel < 0) vel = 0.0;
+    *reward = -1.0;
+    o[0] = pos; o[1] = vel;
+    return pos >= goal_position && vel >= 0.0;
+}
+
+/* Acrobot-v1 (book dynamics, no torque noise) */
+#define ACROBOT_WRAP_CAP 64 /* iterations per wrap loop, as in the engine (env.cuh) */
+
+static void acrobot_dsdt(const azo_config* c, const double* s, double a, double* d) {
+    const double m1 = 1.0, m2 = 1.0, l1 = 1.0, lc1 = 0.5, lc2 = 0.5, I1 = 1.0, I2 = 1.0, g = 9.8, pi = 3.141592653589793;
+    const double theta1 = s[0], theta2 = s[1], dtheta1 = s[2], dtheta2 = s[3];
+    const double c2 = m_cos(c, theta2), s2 = m_sin(c, theta2);
+    const double d1 = m1 * (lc1 * lc1) + m2 * (l1 * l1 + lc2 * lc2 + 2 * l1 * lc2 * c2) + I1 + I2;
+    const double d2 = m2 * (lc2 * lc2 + l1 * lc2 * c2) + I2;
+    const double phi2 = m2 * lc2 * g * m_cos(c, theta1 + theta2 - pi / 2.);
+    const double phi1 = -m2 * l1 * lc2 * (dtheta2 * dtheta2) * s2 - 2 * m2 * l1 * lc2 * dtheta2 * dtheta1 * s2 +
+                        (m1 * lc1 + m2 * l1) * g * m_cos(c, theta1 - pi / 2) + phi2;
+    const double ddtheta2 = (a + d2 / d1 * phi1 - m2 * l1 * lc2 * (dtheta1 * dtheta1) * s2 - phi2) / (m2 * (lc2 * lc2) + I2 - (d2 * d2) / d1);
+    const double ddtheta1 = -(d2 * ddtheta2 + phi1) / d1;
+    d[0] = dtheta1; d[1] = dtheta2; d[2] = ddtheta1; d[3] = ddtheta2;
+}
+
+/* gym's wrap with each loop capped at ACROBOT_WRAP_CAP iterations (*capped = 1 when a loop would go on) */
+static double acrobot_wrap(double x, int* capped) {
+    const double pi = 3.141592653589793, diff = pi - -pi;
+    for (int k = 0; x > pi; ++k) {
+        if (k == ACROBOT_WRAP_CAP) { *capped = 1; return x; }
+        x = x - diff;
     }
+    for (int k = 0; x < -pi; ++k) {
+        if (k == ACROBOT_WRAP_CAP) { *capped = 1; return x; }
+        x = x + diff;
+    }
+    return x;
+}
+
+/* min(max(x, m), M) with Python's builtins: a NaN passes, -0 stays -0 */
+static double acrobot_bound(double x, double m, double M) {
+    x = m > x ? m : x;
+    return M < x ? M : x;
+}
+
+/* one step: RK4 over [0, dt] of the book dynamics, wrap, bound; returns terminal, or AZO_ERR_WRAP when a wrap loop reached its cap */
+static int acrobot_step(const azo_config* c, const double* s, int action, double* o, double* reward) {
+    const double dt = .2, pi = 3.141592653589793, MAX_VEL_1 = 4 * pi, MAX_VEL_2 = 9 * pi;
+    const double torque = action == 0 ? -1.0 : (action == 1 ? 0.0 : 1.0);
+    const double dt2 = dt / 2.0;
+    double k1[4], k2[4], k3[4], k4[4], y[4];
+    int capped = 0;
+    acrobot_dsdt(c, s, torque, k1);
+    for (int i = 0; i < 4; ++i) y[i] = s[i] + dt2 * k1[i];
+    acrobot_dsdt(c, y, torque, k2);
+    for (int i = 0; i < 4; ++i) y[i] = s[i] + dt2 * k2[i];
+    acrobot_dsdt(c, y, torque, k3);
+    for (int i = 0; i < 4; ++i) y[i] = s[i] + dt * k3[i];
+    acrobot_dsdt(c, y, torque, k4);
+    for (int i = 0; i < 4; ++i) o[i] = s[i] + dt / 6.0 * (k1[i] + 2 * k2[i] + 2 * k3[i] + k4[i]);
+    o[0] = acrobot_wrap(o[0], &capped);
+    o[1] = acrobot_wrap(o[1], &capped);
+    o[2] = acrobot_bound(o[2], -MAX_VEL_1, MAX_VEL_1);
+    o[3] = acrobot_bound(o[3], -MAX_VEL_2, MAX_VEL_2);
+    const int terminal = -m_cos(c, o[0]) - m_cos(c, o[1] + o[0]) > 1.;
+    *reward = terminal ? 0.0 : -1.0;
+    return capped ? AZO_ERR_WRAP : terminal;
+}
+
+/* _get_ob of a hidden state, each entry rounded to f32 */
+static void acrobot_obs(const azo_config* c, const double* s, float* x) {
+    x[0] = (float)m_cos(c, s[0]); x[1] = (float)m_sin(c, s[0]); x[2] = (float)m_cos(c, s[1]); x[3] = (float)m_sin(c, s[1]);
+    x[4] = (float)s[2]; x[5] = (float)s[3];
+}
+
+/* The env dispatch: the only code that depends on which env a config steps.  A discrete action arrives as its index in a float. */
+#define ENV_MAX_OBS 6 /* widest observation (Acrobot) */
+
+static int env_hidden_dim(const azo_config* c) {
+    switch (c->env) {
+        case AZO_ENV_MOUNTAIN_CAR_CONTINUOUS: case AZO_ENV_MOUNTAIN_CAR: return 2;
+        case AZO_ENV_ACROBOT: return 4;
+        default: return c->variant == AZO_DISCRETE ? 4 : 2;
+    }
+}
+
+static int env_step(const azo_config* c, const double* s, float action, double* o, double* reward) {
+    switch (c->env) {
+        case AZO_ENV_MOUNTAIN_CAR_CONTINUOUS: return mountain_car_continuous_step(c, s, action, o, reward);
+        case AZO_ENV_MOUNTAIN_CAR: return mountain_car_step(c, s, (int)action, o, reward);
+        case AZO_ENV_ACROBOT: return acrobot_step(c, s, (int)action, o, reward);
+        default: return c->variant == AZO_DISCRETE ? cartpole_step(c, s, (int)action, o, reward) : pendulum_step(c, s, action, o, reward);
+    }
+}
+
+/* the network input of a hidden state: Pendulum (cos th, sin th, thdot), Acrobot _get_ob, the others the state itself (f32) */
+static void env_obs(const azo_config* c, const double* s, float* x) {
+    if (c->env == AZO_ENV_ACROBOT) acrobot_obs(c, s, x);
+    else if (c->env == AZO_ENV_DEFAULT && c->variant == AZO_CONTINUOUS) pendulum_obs(c, s, x);
+    else for (int i = 0; i < env_hidden_dim(c); ++i) x[i] = (float)s[i];
+}
+
+int azo_env_step(const azo_config* c, const double* s_in, float action, double* s_out, double* reward, float* obs) {
+    const int term = env_step(c, s_in, action, s_out, reward);
+    if (obs) env_obs(c, s_out, obs);
     return term;
 }
 
-/* observation of a hidden env state: CartPole the state itself (f32), Pendulum (cos th, sin th, thdot) */
-void azo_obs(const azo_config* c, const double* s, float* obs) {
-    if (c->variant == AZO_DISCRETE) for (int i = 0; i < 4; ++i) obs[i] = (float)s[i];
-    else pendulum_obs(c, s, obs);
-}
+void azo_obs(const azo_config* c, const double* s, float* obs) { env_obs(c, s, obs); }
 
 int32_t azo_pw_limit(double c_pw, double kappa, int32_t n) { return (int32_t)ceil(c_pw * pow((double)(n + 1), kappa)); }
 
@@ -771,8 +894,8 @@ static void d_evaluate(const azo_config* c, const net_t* net, const azo_tapes* t
         V = tp->V[b * t->R + node];
         for (int a = 0; a < A; ++a) t->prior[node * A + a] = tp->prior[(b * t->R + node) * A + a];
     } else {
-        float x[4];
-        for (int i = 0; i < 4; ++i) x[i] = (float)t->state[node * 4 + i];
+        float x[ENV_MAX_OBS];
+        env_obs(c, t->state + node * 4, x);
         net_forward(net, c, x, &V, raw);
         azo_head_post(c, raw, t->prior + node * A);
         ctr[4]++;
@@ -788,7 +911,7 @@ static int search_discrete_one(const azo_config* c, const net_t* net, const azo_
     dtree_clear(t);
     t->n_nodes = 1;
     t->parent[0] = -1; t->paction[0] = -1; t->node_n[0] = root_n; t->terminal[0] = 0; t->r[0] = 0.0;
-    for (int i = 0; i < 4; ++i) t->state[i] = root_state[i];
+    for (int i = 0; i < env_hidden_dim(c); ++i) t->state[i] = root_state[i];
     d_evaluate(c, net, tp, b, t, 0, ctr);
     for (int it = 0; it < c->n_rollouts; ++it) {
         int node = 0, created = 0;
@@ -808,8 +931,10 @@ static int search_discrete_one(const azo_config* c, const net_t* net, const azo_
             if (child >= 0) { node = child; continue; }
             child = t->n_nodes++;
             double rew;
-            int term = cartpole_step(c, t->state + node * 4, a, t->state + child * 4, &rew);
-            rew = term ? c->reward_terminal : c->reward_step; /* rl/wrappers.py (1.0 / 1.0 without wrappers) */
+            int term = env_step(c, t->state + node * 4, (float)a, t->state + child * 4, &rew);
+            if (term == AZO_ERR_WRAP) return AZO_ERR_WRAP;
+            /* CartPole's reward wrappers (rl/wrappers.py): a constant per terminal flag; azo_search allows 1.0 / 1.0 only on other envs */
+            if (c->reward_step != 1.0 || c->reward_terminal != 1.0) rew = term ? c->reward_terminal : c->reward_step;
             t->parent[child] = node; t->paction[child] = a; t->node_n[child] = 0; t->terminal[child] = term; t->r[child] = rew;
             t->echild[node * A + a] = child;
             d_evaluate(c, net, tp, b, t, child, ctr);
@@ -868,8 +993,8 @@ static void c_evaluate(const azo_config* c, const net_t* net, const azo_tapes* t
     if (c->use_eval_tape) {
         V = tp->V[b * t->R + row];
     } else {
-        float obs[3], raw[3 * AZO_MAX_K];
-        pendulum_obs(c, t->state + row * 2, obs);
+        float obs[ENV_MAX_OBS], raw[3 * AZO_MAX_K];
+        env_obs(c, t->state + row * 2, obs);
         net_forward(net, c, obs, &V, raw);
         azo_head_post(c, raw, t->head + (size_t)row * t->K3);
         ctr[4]++;
@@ -908,7 +1033,7 @@ static int search_continuous_one(const azo_config* c, const net_t* net, const az
     t->n_rows = 1;
     t->parent[0] = -1; t->expanded[0] = 1; t->node_n[0] = 0; t->terminal[0] = 0; t->r[0] = 0.0; t->en[0] = 0; t->eW[0] = 0.0;
     t->action[0] = 0.0f;
-    t->state[0] = root_state[0]; t->state[1] = root_state[1];
+    for (int i = 0; i < env_hidden_dim(c); ++i) t->state[i] = root_state[i];
     c_evaluate(c, net, tp, b, t, 0, ctr);
     c_add_pw_action(c, tp, b, t, 0, g, ctr);
     const float g32 = (float)c->gamma;
@@ -936,7 +1061,7 @@ static int search_continuous_one(const azo_config* c, const net_t* net, const az
             path[depth++] = sel;
             if (t->expanded[sel]) { node = sel; continue; }
             double rew;
-            int term = pendulum_step(c, t->state + node * 2, t->action[sel], t->state + sel * 2, &rew);
+            int term = env_step(c, t->state + node * 2, t->action[sel], t->state + sel * 2, &rew);
             t->r[sel] = rew / PENDULUM_R_SCALE; /* mcts.py:687 */
             t->terminal[sel] = term; t->expanded[sel] = 1; t->node_n[sel] = 0;
             c_evaluate(c, net, tp, b, t, sel, ctr);
@@ -973,7 +1098,7 @@ static void* worker(void* arg) {
     job_t* J = (job_t*)arg;
     const azo_config* cfg = J->cfg;
     const int R = azo_rows(cfg);
-    const int A = cfg->num_actions, K = cfg->num_components, K3 = 3 * (K > 0 ? K : 1);
+    const int A = cfg->num_actions, K = cfg->num_components, K3 = 3 * (K > 0 ? K : 1), HS = env_hidden_dim(cfg);
     azo_results* res = J->res;
     dtree_t dt; ctree_t ct;
     if (cfg->variant == AZO_DISCRETE) dtree_alloc(&dt, R, A); else ctree_alloc(&ct, R, K3);
@@ -990,7 +1115,7 @@ static void* worker(void* arg) {
             }
             int e;
             if (cfg->variant == AZO_DISCRETE) {
-                e = search_discrete_one(cfg, J->net, J->tapes, b, J->root_state + b * 4, J->root_n_init ? J->root_n_init[b] : 0, &dt, &g, J->ctr);
+                e = search_discrete_one(cfg, J->net, J->tapes, b, J->root_state + b * HS, J->root_n_init ? J->root_n_init[b] : 0, &dt, &g, J->ctr);
                 if (!e && res) {
                     double Q[AZO_MAX_A] = {0};
                     res->n_children[b] = A;
@@ -1010,12 +1135,12 @@ static void* worker(void* arg) {
                     memcpy(dd->parent + o, dt.parent, R * 4); memcpy(dd->paction + o, dt.paction, R * 4);
                     memcpy(dd->node_n + o, dt.node_n, R * 4); memcpy(dd->terminal + o, dt.terminal, R * 4);
                     memcpy(dd->V + o, dt.V, R * 4); memcpy(dd->r + o, dt.r, R * 8);
-                    memcpy(dd->state + o * 4, dt.state, (size_t)R * 4 * 8);
+                    for (int i = 0; i < R; ++i) memcpy(dd->state + (o + i) * HS, dt.state + (size_t)i * 4, (size_t)HS * 8);
                     memcpy(dd->prior + o * A, dt.prior, (size_t)R * A * 4); memcpy(dd->eW + o * A, dt.eW, (size_t)R * A * 8);
                     memcpy(dd->en + o * A, dt.en, (size_t)R * A * 4); memcpy(dd->echild + o * A, dt.echild, (size_t)R * A * 4);
                 }
             } else {
-                e = search_continuous_one(cfg, J->net, J->tapes, b, J->root_state + b * 2, &ct, &g, J->pw_table, J->ctr);
+                e = search_continuous_one(cfg, J->net, J->tapes, b, J->root_state + b * HS, &ct, &g, J->pw_table, J->ctr);
                 if (!e && res) {
                     double Q[4096]; int32_t cnt[4096]; int C = 0;
                     Q[0] = 0.0;
@@ -1059,6 +1184,12 @@ int azo_search(const azo_config* cfg, const float* weights, int64_t n_weights, i
     if (cfg->variant == AZO_DISCRETE && (cfg->num_actions < 1 || cfg->num_actions > AZO_MAX_A)) return -2;
     if (cfg->variant == AZO_CONTINUOUS && (cfg->num_components < 1 || cfg->num_components > AZO_MAX_K)) return -2;
     if (cfg->use_eval_tape && !tapes) return -2;
+    const int disc = cfg->variant == AZO_DISCRETE, S = cfg->state_dim, A = cfg->num_actions;
+    if (cfg->env == AZO_ENV_MOUNTAIN_CAR_CONTINUOUS && !(!disc && S == 2)) return -2;
+    if (cfg->env == AZO_ENV_MOUNTAIN_CAR && !(disc && A == 3 && S == 2)) return -2;
+    if (cfg->env == AZO_ENV_ACROBOT && !(disc && A == 3 && S == 6)) return -2;
+    if (cfg->env < AZO_ENV_DEFAULT || cfg->env > AZO_ENV_ACROBOT) return -2;
+    if (!(disc && cfg->env == AZO_ENV_DEFAULT) && (cfg->reward_step != 1.0 || cfg->reward_terminal != 1.0)) return -2;
     net_t net;
     memset(&net, 0, sizeof net);
     if (!cfg->use_eval_tape && net_init(&net, cfg, weights, n_weights)) return -2;

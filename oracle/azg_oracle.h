@@ -23,8 +23,10 @@
  *                                      MLP trunk, value head, softmax / GMM head
  *   alphazero/network/distributions.py:50-63  bound*tanh(x)
  * Third-party arithmetic that is NOT under /root/reference (gym 0.17.2/0.19.0
- * classic_control CartPole-v0 / Pendulum-v0 `step`) is restated from the
- * published gym source; see SURVEY.md section 8(c).
+ * classic_control CartPole-v0 / Pendulum-v0 / MountainCarContinuous-v0 /
+ * MountainCar-v0 / Acrobot-v1 `step`) is restated from the published gym
+ * source; see SURVEY.md section 8(c).  The config's `env` picks the env a
+ * search steps; the search loops are the same for every env.
  *
  * Parity pinning: the reference has no tests or golden vectors.  This oracle is
  * pinned against outputs of the reference itself, generated in the build
@@ -65,11 +67,11 @@ extern "C" {
 #define AZO_MAX_A 8
 
 typedef struct {
-    int32_t variant;       /* AZO_DISCRETE (CartPole) | AZO_CONTINUOUS (Pendulum) */
+    int32_t variant;       /* AZO_DISCRETE | AZO_CONTINUOUS */
     int32_t n_rollouts;
     int32_t num_actions;   /* discrete: A */
     int32_t num_components;/* continuous: K (1 = DiagonalNormalPolicy, >1 = DiagonalGMMPolicy) */
-    int32_t state_dim;     /* network input: 4 CartPole, 3 Pendulum */
+    int32_t state_dim;     /* network input (the env's observation): 4 CartPole, 3 Pendulum, 2 MountainCar(Continuous), 6 Acrobot */
     int32_t hidden;        /* hidden width (all layers equal) */
     int32_t n_hidden;      /* number of hidden layers */
     int32_t activation;    /* AZO_ACT_* */
@@ -87,8 +89,17 @@ typedef struct {
      * CartPole: the reward of a step is a constant per terminal flag -- 1.0 / 1.0 plain, 0.005 / -1 with ReparametrizeWrapper (:78-105),
      * / 250.0 with ScaleRewardWrapper (:58-75).  (Pendulum's ScaleRewardWrapper returns np.float32, whose promotion through the backup
      * depends on the numpy version: not restated.) */
-    double reward_step, reward_terminal; /* discrete search */
+    double reward_step, reward_terminal; /* CartPole only: any other env requires 1.0 / 1.0 */
+    int32_t env;           /* AZO_ENV_* */
 } azo_config;
+#define AZO_ENV_DEFAULT 0                 /* the variant's own env: CartPole-v0 (discrete) / Pendulum-v0 (continuous) */
+#define AZO_ENV_MOUNTAIN_CAR_CONTINUOUS 1 /* continuous, state_dim 2 */
+#define AZO_ENV_MOUNTAIN_CAR 2            /* discrete, num_actions 3, state_dim 2 */
+#define AZO_ENV_ACROBOT 3                 /* discrete, num_actions 3, state_dim 6 */
+/* hidden env state (the tree's state rows hold it; 4 doubles per discrete row, 2 per continuous row):
+ *   CartPole x, xdot, th, thdot | Pendulum th, thdot | MountainCar(Continuous) position, velocity | Acrobot th1, th2, dth1, dth2 */
+
+#define AZO_ERR_WRAP -4 /* Acrobot: an angle needed more than 64 iterations of a wrap loop (gym's loop is unbounded) */
 #define AZO_RNG_PHILOX 0
 #define AZO_RNG_MT19937 1
 
@@ -121,7 +132,7 @@ typedef struct {
     int32_t* terminal;  /* [B][R] */
     float* V;           /* [B][R]   Node.V */
     double* r;          /* [B][R]   Node.r */
-    double* state;      /* [B][R][4] hidden env state */
+    double* state;      /* [B][R][HS] hidden env state: HS = 4 CartPole / Acrobot, 2 MountainCar */
     float* prior;       /* [B][R][A] */
     double* eW;         /* [B][R][A] Action.W */
     int32_t* en;        /* [B][R][A] Action.n */
@@ -141,7 +152,7 @@ typedef struct {
     int32_t* terminal;  /* [B][R] */
     float* V;           /* [B][R] */
     double* r;          /* [B][R]  (already divided by PENDULUM_R_SCALE) */
-    double* state;      /* [B][R][2] th, thdot */
+    double* state;      /* [B][R][2] hidden env state */
     float* head;        /* [B][R][3K] cached policy head: mu[K], sigma[K], prob[K] */
 } azo_dump_continuous;
 
@@ -165,10 +176,10 @@ typedef struct {
 
 /* Run B independent searches.  weights: flat f32 in state_dict order
  * (trunk.{0,2,..}.{weight,bias}, value_head.{weight,bias}, dist_head.{weight,bias}).
- * root_state: [B][4] (CartPole x,xdot,th,thdot) or [B][2] (Pendulum th,thdot).
+ * root_state: [B][HS] hidden env states (HS: see AZO_ENV_*).
  * root_n_init: [B] carried-over root visit count (discrete tree reuse quirk) or NULL.
  * tree_id0: global id of tree 0 (Philox stream key).  dump_* may be NULL.
- * Returns 0, or <0 on error (terminal root, NaN in UCT, bad config). */
+ * Returns 0, or <0 on error (-2 bad config, -3 NaN in UCT, AZO_ERR_WRAP). */
 int azo_search(const azo_config* cfg, const float* weights, int64_t n_weights, int32_t B, const double* root_state,
                const int32_t* root_n_init, int64_t tree_id0, const azo_tapes* tapes, azo_results* res,
                azo_dump_discrete* dd, azo_dump_continuous* dc, int32_t n_threads);
@@ -189,6 +200,7 @@ void azo_mlp_forward(const azo_config* cfg, const float* weights, int32_t n, con
 /* head post-processing: discrete softmax priors [A]; continuous (mu,sigma,prob)[3K] */
 void azo_head_post(const azo_config* cfg, const float* raw, float* out);
 float azo_sample_action(const azo_config* cfg, const float* head, float u_comp, const float* z);
+/* one env step of the config's env (discrete: the action index as float); returns terminal, or AZO_ERR_WRAP */
 int azo_env_step(const azo_config* cfg, const double* s_in, float action, double* s_out, double* reward, float* obs);
 void azo_obs(const azo_config* cfg, const double* s, float* obs); /* observation of a hidden env state */
 

@@ -23,6 +23,20 @@ MATH_LIBM, MATH_DET = 0, 1
 EVAL_FP32, EVAL_Q8 = 0, 1
 RNG_PHILOX, RNG_MT19937 = 0, 1
 VT = {"off_policy": 0, "on_policy": 1, "greedy": 2}
+# env names as alphazero_gym_b200.engine spells them (not imported: the oracle stays apart from the product package);
+# Config.env None = the variant's own env, CartPole-v0 / Pendulum-v0
+CARTPOLE, PENDULUM, MOUNTAIN_CAR_CONTINUOUS = "CartPole-v0", "Pendulum-v0", "MountainCarContinuous-v0"
+MOUNTAIN_CAR, ACROBOT = "MountainCar-v0", "Acrobot-v1"
+_ENV = {None: 0, MOUNTAIN_CAR_CONTINUOUS: 1, MOUNTAIN_CAR: 2, ACROBOT: 3}  # AZO_ENV_*
+# the config defaults each env needs (the env's action count / observation width / action bound)
+_ENV_DEFAULTS = {MOUNTAIN_CAR_CONTINUOUS: dict(state_dim=2, action_bound=1.0), MOUNTAIN_CAR: dict(num_actions=3, state_dim=2),
+                 ACROBOT: dict(num_actions=3, state_dim=6)}
+R_SCALE = 16.2736044  # the continuous search's reward divisor (mcts.py:20; PENDULUM_R_SCALE in azg_oracle.c)
+ERR_WRAP = -4  # AZO_ERR_WRAP
+
+
+class WrapCapReached(Exception):
+    """Acrobot: an angle needed more than 64 iterations of a wrap loop (gym itself loops on; the engine fails with AZG_EWRAP)."""
 
 
 def build(force: bool = False) -> str:
@@ -41,7 +55,7 @@ class _Cfg(C.Structure):
         ("c_uct", C.c_double), ("gamma", C.c_double), ("epsilon", C.c_double), ("c_pw", C.c_double), ("kappa", C.c_double),
         ("action_bound", C.c_float), ("log_std_min", C.c_float), ("log_std_max", C.c_float),
         ("seed", C.c_uint64), ("eval_mode", C.c_int32), ("rng_mode", C.c_int32),
-        ("reward_step", C.c_double), ("reward_terminal", C.c_double),
+        ("reward_step", C.c_double), ("reward_terminal", C.c_double), ("env", C.c_int32),
     ]
 
 
@@ -145,17 +159,25 @@ class Config:
     # reward wrappers (rl/wrappers.py) around CartPole: reward of a step / of the terminating step
     reward_step: float = 1.0
     reward_terminal: float = 1.0
+    env: Optional[str] = None  # None (the variant's own env) | MOUNTAIN_CAR_CONTINUOUS | MOUNTAIN_CAR | ACROBOT
 
     def c(self) -> _Cfg:
         return _Cfg(self.variant, self.n_rollouts, self.num_actions, self.num_components, self.state_dim, self.hidden,
                     self.n_hidden, self.activation, self.math_mode, VT[self.V_target_policy], self.puct_f32,
                     self.use_eval_tape, self.c_uct, self.gamma, self.epsilon, self.c_pw, self.kappa,
                     self.action_bound, self.log_std_min, self.log_std_max, self.seed, self.eval_mode, self.rng_mode,
-                    self.reward_step, self.reward_terminal)
+                    self.reward_step, self.reward_terminal, _ENV[self.env])
 
     @property
     def rows(self) -> int:
         return self.n_rollouts + 2
+
+    @property
+    def hidden_dim(self) -> int:
+        """Width of the env's hidden state (the search's root states and the dump's state rows)."""
+        if self.env is None:
+            return 4 if self.variant == DISCRETE else 2
+        return 4 if self.env == ACROBOT else 2
 
     @property
     def head_dim(self) -> int:
@@ -172,18 +194,20 @@ class Config:
         return max(pw_limit(self.c_pw, self.kappa, self.n_rollouts), pw_limit(self.c_pw, self.kappa, 0)) + 1
 
 
-def discrete_config(**kw) -> Config:
-    """run_discrete.yaml / MCTSDiscrete.yaml / DiscretePolicy.yaml defaults."""
+def discrete_config(env: Optional[str] = None, **kw) -> Config:
+    """run_discrete.yaml / MCTSDiscrete.yaml / DiscretePolicy.yaml defaults, with the env's own (see _ENV_DEFAULTS)."""
     d = dict(variant=DISCRETE, n_rollouts=8, num_actions=2, state_dim=4, hidden=128, n_hidden=2, activation=ACT_RELU,
-             c_uct=1.5, gamma=1.0, epsilon=0.1)
+             c_uct=1.5, gamma=1.0, epsilon=0.1, env=env)
+    d.update(_ENV_DEFAULTS.get(env, {}))
     d.update(kw)
     return Config(**d)
 
 
-def continuous_config(**kw) -> Config:
-    """run_continuous.yaml / MCTSContinuous.yaml / ContinuousPolicy.yaml defaults."""
+def continuous_config(env: Optional[str] = None, **kw) -> Config:
+    """run_continuous.yaml / MCTSContinuous.yaml / ContinuousPolicy.yaml defaults, with the env's own (see _ENV_DEFAULTS)."""
     d = dict(variant=CONTINUOUS, n_rollouts=25, num_components=2, state_dim=3, hidden=128, n_hidden=3,
-             activation=ACT_ELU, c_uct=0.05, c_pw=1.0, kappa=0.5, gamma=1.0, epsilon=0.0, action_bound=2.0)
+             activation=ACT_ELU, c_uct=0.05, c_pw=1.0, kappa=0.5, gamma=1.0, epsilon=0.0, action_bound=2.0, env=env)
+    d.update(_ENV_DEFAULTS.get(env, {}))
     d.update(kw)
     return Config(**d)
 
@@ -199,10 +223,11 @@ def _p(a: Optional[np.ndarray]):
 def search(cfg: Config, weights: Optional[np.ndarray], root_state: np.ndarray, root_n_init: Optional[np.ndarray] = None,
            tree_id0: int = 0, tapes: Optional[Dict[str, np.ndarray]] = None, dump: bool = True,
            n_threads: int = 1) -> Dict[str, np.ndarray]:
-    """Run B independent searches on the CPU oracle; returns root results (+ full tree dump)."""
+    """Run B independent searches on the CPU oracle from hidden env states [B, HS]; returns root results (+ full tree dump).
+    Raises WrapCapReached where the engine fails with AZG_EWRAP."""
     L = lib()
-    sd = 4 if cfg.variant == DISCRETE else 2
-    root_state = np.ascontiguousarray(root_state, dtype=np.float64).reshape(-1, sd)
+    HS = cfg.hidden_dim
+    root_state = np.ascontiguousarray(root_state, dtype=np.float64).reshape(-1, HS)
     B, R, A, K3 = root_state.shape[0], cfg.rows, cfg.num_actions, 3 * max(cfg.num_components, 1)
     cm = cfg.cmax
     out: Dict[str, np.ndarray] = dict(
@@ -214,7 +239,7 @@ def search(cfg: Config, weights: Optional[np.ndarray], root_state: np.ndarray, r
     if dump and cfg.variant == DISCRETE:
         d = dict(n_nodes=np.zeros(B, np.int32), parent=np.zeros((B, R), np.int32), paction=np.zeros((B, R), np.int32),
                  node_n=np.zeros((B, R), np.int32), terminal=np.zeros((B, R), np.int32), V=np.zeros((B, R), np.float32),
-                 r=np.zeros((B, R), np.float64), state=np.zeros((B, R, 4), np.float64),
+                 r=np.zeros((B, R), np.float64), state=np.zeros((B, R, HS), np.float64),
                  prior=np.zeros((B, R, A), np.float32), eW=np.zeros((B, R, A), np.float64),
                  en=np.zeros((B, R, A), np.int32), echild=np.zeros((B, R, A), np.int32))
         dd = _DumpD(*[_p(d[n]) for n, _ in _DumpD._fields_])
@@ -223,7 +248,7 @@ def search(cfg: Config, weights: Optional[np.ndarray], root_state: np.ndarray, r
         d = dict(n_rows=np.zeros(B, np.int32), parent=np.zeros((B, R), np.int32), action=np.zeros((B, R), np.float32),
                  eW=np.zeros((B, R), np.float64), en=np.zeros((B, R), np.int32), expanded=np.zeros((B, R), np.int32),
                  node_n=np.zeros((B, R), np.int32), terminal=np.zeros((B, R), np.int32), V=np.zeros((B, R), np.float32),
-                 r=np.zeros((B, R), np.float64), state=np.zeros((B, R, 2), np.float64),
+                 r=np.zeros((B, R), np.float64), state=np.zeros((B, R, HS), np.float64),
                  head=np.zeros((B, R, K3), np.float32))
         dc = _DumpC(*[_p(d[n]) for n, _ in _DumpC._fields_])
         out.update(d)
@@ -243,6 +268,8 @@ def search(cfg: Config, weights: Optional[np.ndarray], root_state: np.ndarray, r
     rc = L.azo_search(C.byref(cfg.c()), _p(w), 0 if w is None else w.size, B, _p(root_state), _p(rn), tree_id0,
                       None if tp is None else C.byref(tp), C.byref(res), None if dd is None else C.byref(dd),
                       None if dc is None else C.byref(dc), n_threads)
+    if rc == ERR_WRAP:
+        raise WrapCapReached("an angle reached the wrap cap")
     if rc != 0:
         raise ValueError({-1: "Can't do tree search from a terminal node", -2: "bad oracle config",
                           -3: "NaN in UCT"}.get(rc, f"oracle error {rc}"))
@@ -273,19 +300,26 @@ def sample_action(cfg: Config, head: np.ndarray, u: float, z: np.ndarray) -> flo
 
 
 def env_step(cfg: Config, state: np.ndarray, action: float):
+    """One step of the config's env (discrete: the action index) -> (next hidden state, reward, done, f32 observation).
+    Raises WrapCapReached where the engine fails with AZG_EWRAP."""
     s = np.ascontiguousarray(state, np.float64)
-    o = np.zeros_like(s)
+    o = np.zeros(cfg.hidden_dim, np.float64)
     obs = np.zeros(cfg.state_dim, np.float32)
     r = C.c_double()
     term = lib().azo_env_step(C.byref(cfg.c()), _p(s), C.c_float(action), _p(o), C.byref(r), _p(obs))
+    if term == ERR_WRAP:
+        raise WrapCapReached(state)
     return o, r.value, bool(term), obs
 
 
 def obs(cfg: Config, state: np.ndarray) -> np.ndarray:
+    """The network input (f32 observation) of a hidden state [HS] -> [S], or of states [n, HS] -> [n, S]."""
     s = np.ascontiguousarray(state, np.float64)
-    o = np.zeros(cfg.state_dim, np.float32)
-    lib().azo_obs(C.byref(cfg.c()), _p(s), _p(o))
-    return o
+    rows = s.reshape(-1, cfg.hidden_dim)
+    o = np.zeros((rows.shape[0], cfg.state_dim), np.float32)
+    for i in range(rows.shape[0]):
+        lib().azo_obs(C.byref(cfg.c()), _p(rows[i]), _p(o[i]))
+    return o if s.ndim == 2 else o[0]
 
 
 def rng_u32(seed: int, tree: int, stream: int, idx: int, block: int = 0, word: int = 0) -> int:

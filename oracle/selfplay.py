@@ -6,8 +6,8 @@ reset or reset_mcts / mcts_forward), ContinuousAgent.act (agents.py:522-537: act
 (agents.py:292-303: stable_normalizer + pi.argmax() / np.random.choice), helpers.stable_normalizer (helpers.py:9-27),
 MCTSDiscrete.forward (mcts.py:495-526; only the new root's visit count survives, SURVEY 7-7).  The searches are
 oracle/azo.search.  Randomness is injected exactly as in the engine: the Philox key of step s is
-seed + s * 0x9E3779B97F4A7C15 (mod 2^64); stream 2 = the discrete agent's action draw, stream 3 = Env.reset
-(gym: CartPole U(-0.05, 0.05)^4, Pendulum th ~ U(-pi, pi), thdot ~ U(-1, 1)); a 32-bit word x maps to (x + 0.5) / 2^32.
+seed + s * 0x9E3779B97F4A7C15 (mod 2^64); stream 2 = the discrete agent's action draw, stream 3 = Env.reset (RESETS);
+a 32-bit word x maps to (x + 0.5) / 2^32.
 """
 from __future__ import annotations
 
@@ -30,6 +30,20 @@ def _unit(x: int) -> float:
     return (float(x) + 0.5) * 2.3283064365386963e-10
 
 
+def _uniform(lo: float, hi: float, w: int) -> float:
+    return lo + (hi - lo) * _unit(w)
+
+
+# gym's Env.reset per env, from the four words of stream 3 at the episode's index
+RESETS = {
+    (azo.DISCRETE, None): lambda w: [_uniform(-0.05, 0.05, w[k]) for k in range(4)],            # CartPole U(-0.05, 0.05)^4
+    (azo.CONTINUOUS, None): lambda w: [_uniform(-np.pi, np.pi, w[0]), _uniform(-1.0, 1.0, w[1])],  # Pendulum th, thdot
+    (azo.CONTINUOUS, azo.MOUNTAIN_CAR_CONTINUOUS): lambda w: [_uniform(-0.6, -0.4, w[0]), 0.0],  # position, velocity 0
+    (azo.DISCRETE, azo.MOUNTAIN_CAR): lambda w: [_uniform(-0.6, -0.4, w[0]), 0.0],
+    (azo.DISCRETE, azo.ACROBOT): lambda w: [_uniform(-0.1, 0.1, w[k]) for k in range(4)],       # U(-0.1, 0.1)^4
+}
+
+
 def stable_normalizer(x: np.ndarray, temp: float) -> np.ndarray:
     x = (x / np.max(x)) ** temp  # helpers.py:26
     return np.abs(x / np.sum(x))
@@ -49,14 +63,14 @@ def run(cfg: azo.Config, weights: np.ndarray, states0: np.ndarray, steps: int, m
         key = step_seed(seed, s)
         c = dataclasses.replace(cfg, seed=key)
         res = azo.search(c, weights, state, root_n.copy() if disc else None, tree_id0=tree_id0, dump=disc, n_threads=n_threads)
-        rec = dict(obs=np.stack([azo.obs(c, state[t]) for t in range(B)]), actions=res["actions"].copy(),
+        rec = dict(obs=azo.obs(c, state), actions=res["actions"].copy(),
                    counts=res["counts"].copy(), Q=res["Q"].copy(), V_target=res["V_target"].copy(),
                    n_children=res["n_children"].copy(), action_taken=np.zeros(B, np.float32), reward=np.zeros(B, np.float64),
                    done=np.zeros(B, np.int32))
         for t in range(B):
             nk = int(res["n_children"][t])
             if disc:
-                x = (res["Q"][t, :2] if by_value else res["counts"][t, :2].astype(np.float64))
+                x = (res["Q"][t, :cfg.num_actions] if by_value else res["counts"][t, :cfg.num_actions].astype(np.float64))
                 pi = stable_normalizer(x, temperature)
                 if deterministic:
                     a = int(pi.argmax())
@@ -77,10 +91,7 @@ def run(cfg: azo.Config, weights: np.ndarray, states0: np.ndarray, steps: int, m
             if done:
                 episode[t] += 1
                 w = [azo.rng_u32(key, tree_id0 + t, 3, int(episode[t]), 0, k) for k in range(4)]
-                if disc:
-                    nxt = np.array([-0.05 + (0.05 - -0.05) * _unit(w[k]) for k in range(4)])
-                else:
-                    nxt = np.array([-np.pi + (np.pi - -np.pi) * _unit(w[0]), -1.0 + (1.0 - -1.0) * _unit(w[1])])
+                nxt = np.array(RESETS[cfg.variant, cfg.env](w))
             elif disc:
                 child = int(res["echild"][t, 0, a])
                 rn = 0 if child < 0 else int(res["node_n"][t, child])

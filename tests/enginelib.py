@@ -12,7 +12,7 @@ def engine_config(cfg: azo.Config, max_trees: int, **kw) -> EngineConfig:
              activation=cfg.activation, V_target_policy=cfg.V_target_policy, puct_f32=cfg.puct_f32, c_uct=cfg.c_uct,
              gamma=cfg.gamma, epsilon=cfg.epsilon, c_pw=cfg.c_pw, kappa=cfg.kappa, action_bound=cfg.action_bound,
              log_std_min=cfg.log_std_min, log_std_max=cfg.log_std_max, seed=cfg.seed,
-             eval_q8=cfg.eval_mode == azo.EVAL_Q8, rng_mt19937=cfg.rng_mode == azo.RNG_MT19937)
+             eval_q8=cfg.eval_mode == azo.EVAL_Q8, rng_mt19937=cfg.rng_mode == azo.RNG_MT19937, env=cfg.env)
     d.update(kw)
     return EngineConfig(**d)
 

@@ -1,4 +1,4 @@
-"""Acrobot-v1 on the CPU: the CPU reference's env (tests/acrobot_oracle.c) against gym's step() restated in plain Python, the wrap
+"""Acrobot-v1 on the CPU: the CPU oracle's env against gym's step() restated in plain Python, the wrap
 cap, its discrete search over three actions through ties, epsilon picks, terminal nodes and visit counts past 255, the self-play
 reset and observation rows, and the host-side plumbing that selects the env (no GPU needed)."""
 import itertools
@@ -9,8 +9,8 @@ import numpy as np
 import pytest
 
 from oracle import azo
-import acrobot_oracle as M
-from acrobot_oracle import AcrobotEnv, WrapCapReached, det_cos, det_sin
+from oracle import selfplay as osp
+from classic_control import AcrobotEnv, WrapCapReached, bound, det_cos, det_sin, wrap
 
 PI = np.pi
 
@@ -59,13 +59,13 @@ def terminal_line(s):
 
 @pytest.mark.parametrize("math_mode", [azo.MATH_LIBM, azo.MATH_DET])
 def test_env_step_equals_gym_restatement(math_mode):
-    """acrobot_oracle.env_step == AcrobotEnv.step bit for bit (state, reward, done, observation) with the same sin / cos."""
-    cfg = M.config()
+    """azo.env_step == AcrobotEnv.step bit for bit (state, reward, done, observation) with the same sin / cos."""
+    cfg = azo.discrete_config(azo.ACROBOT)
     cfg.math_mode = math_mode
     sin, cos = (math.sin, math.cos) if math_mode == azo.MATH_LIBM else (det_sin, det_cos)
     n_done = n_wrap = n_bound = n_nan = 0
     for s, a in edge_cases():
-        nxt, r, term, obs = M.env_step(cfg, np.array(s, np.float64), a)
+        nxt, r, term, obs = azo.env_step(cfg, np.array(s, np.float64), a)
         env = AcrobotEnv(s, sin=sin, cos=cos)
         gob, gr, gdone, _ = env.step(a)
         assert same(nxt, env.state), (s, a, nxt, env.state)
@@ -82,19 +82,19 @@ def test_env_step_equals_gym_restatement(math_mode):
 
 def test_wrap_bound_and_terminal_edges():
     # wrap: gym's loops, each direction and several turns; +-pi stay; NaN passes
-    assert M.wrap(PI + 0.5, -PI, PI) == (PI + 0.5) - 2 * PI and M.wrap(-PI - 0.5, -PI, PI) == (-PI - 0.5) + 2 * PI
+    assert wrap(PI + 0.5, -PI, PI) == (PI + 0.5) - 2 * PI and wrap(-PI - 0.5, -PI, PI) == (-PI - 0.5) + 2 * PI
     x = 40.0
     while x > PI:
         x = x - (PI - -PI)
-    assert M.wrap(40.0, -PI, PI) == x and M.wrap(PI, -PI, PI) == PI and M.wrap(-PI, -PI, PI) == -PI
-    assert np.isnan(M.wrap(np.nan, -PI, PI))
+    assert wrap(40.0, -PI, PI) == x and wrap(PI, -PI, PI) == PI and wrap(-PI, -PI, PI) == -PI
+    assert np.isnan(wrap(np.nan, -PI, PI))
     # bound: both limits, exactly and beyond; -0 stays -0; NaN passes
-    assert M.bound(13.0, -4 * PI, 4 * PI) == 4 * PI and M.bound(-13.0, -4 * PI, 4 * PI) == -4 * PI
-    assert M.bound(4 * PI, -4 * PI, 4 * PI) == 4 * PI and _bits(M.bound(-0.0, -1.0, 1.0)) == _bits(-0.0)
-    assert np.isnan(M.bound(np.nan, -1.0, 1.0))
+    assert bound(13.0, -4 * PI, 4 * PI) == 4 * PI and bound(-13.0, -4 * PI, 4 * PI) == -4 * PI
+    assert bound(4 * PI, -4 * PI, 4 * PI) == 4 * PI and _bits(bound(-0.0, -1.0, 1.0)) == _bits(-0.0)
+    assert np.isnan(bound(np.nan, -1.0, 1.0))
     # the engine's restatement agrees at those points (through a step whose velocities are large)
-    cfg = M.config()
-    s, _, _, _ = M.env_step(cfg, np.array([0.0, 0.0, 20.0, -40.0]), 1)
+    cfg = azo.discrete_config(azo.ACROBOT)
+    s, _, _, _ = azo.env_step(cfg, np.array([0.0, 0.0, 20.0, -40.0]), 1)
     assert s[2] == 4 * PI and s[3] == -9 * PI
     # the terminal line `> 1.`: approached from both sides by bisection on theta1 with theta2 = 0 (-2 cos(theta1) = 1 at 2 pi / 3)
     lo, hi = 2.0, 2.2
@@ -107,22 +107,22 @@ def test_wrap_bound_and_terminal_edges():
         else:
             lo = mid
     for th, want in ((lo, False), (hi, True)):
-        _, r, term, _ = M.env_step(cfg, np.array([th, 0.0, 0.0, 0.0]), 1)
+        _, r, term, _ = azo.env_step(cfg, np.array([th, 0.0, 0.0, 0.0]), 1)
         assert term == want and r == (0.0 if want else -1.0)
 
 
 def test_wrap_cap():
     """A huge finite angle reaches the cap in the C reference and in the restatement; the in-box maximum is far below it."""
-    cfg = M.config()
+    cfg = azo.discrete_config(azo.ACROBOT)
     for s in ((1e6, 0.0, 0.0, 0.0), (0.0, -1e6, 0.0, 0.0), (0.0, 1e12, 0.0, 0.0)):
         with pytest.raises(WrapCapReached):
-            M.env_step(cfg, np.array(s), 1)
+            azo.env_step(cfg, np.array(s), 1)
         with pytest.raises(WrapCapReached):
             AcrobotEnv(s, sin=det_sin, cos=det_cos).step(1)
     # 63 turns pass, the pre-wrap angle at 64 turns + pi does not
-    assert M.wrap(PI + 63.5 * (2 * PI), -PI, PI) < PI
+    assert wrap(PI + 63.5 * (2 * PI), -PI, PI) < PI
     with pytest.raises(WrapCapReached):
-        M.wrap(PI + 64.5 * (2 * PI), -PI, PI)
+        wrap(PI + 64.5 * (2 * PI), -PI, PI)
     # the measurement DESIGN.md records: pre-wrap |angle| over gym's box (random states and the corners, all three torques)
     env = AcrobotEnv(sin=np.sin, cos=np.cos)
     rng = np.random.default_rng(0)
@@ -161,9 +161,9 @@ def zero_head(cfg, w):
 def test_oracle_search_ties_and_terminals():
     """Near the goal: terminal expansions (V = 0, r = 0), traces that end on an existing terminal node (counters[6]), and three-way
     ties resolved by the random pick among the winners."""
-    cfg = M.config(n_rollouts=50, epsilon=0.0)
+    cfg = azo.discrete_config(azo.ACROBOT, n_rollouts=50, epsilon=0.0)
     w = zero_head(cfg, weights(cfg))
-    out = M.search(cfg, w, roots("goal", 64), n_threads=4)
+    out = azo.search(cfg, w, roots("goal", 64), n_threads=4)
     assert out["counters"][6] > 0
     term = out["terminal"].astype(bool)
     assert term.any() and not term[:, 0].any()
@@ -178,13 +178,13 @@ def test_oracle_search_ties_and_terminals():
     rs = roots("goal", 64)
     assert np.array_equal(out["state"][:, 0], rs)
     a = int(out["paction"][0, 1])
-    assert np.array_equal(out["state"][0, 1], M.env_step(cfg, rs[0], a)[0])
+    assert np.array_equal(out["state"][0, 1], azo.env_step(cfg, rs[0], a)[0])
 
 
 def test_oracle_search_epsilon_and_deep_counts():
     """epsilon = 0.25 makes random picks of every action; N = 300 pushes the root's visit count past 255."""
-    cfg = M.config(n_rollouts=300, epsilon=0.25, V_target_policy="on_policy", gamma=0.99)
-    out = M.search(cfg, weights(cfg), roots("reset", 8), n_threads=4)
+    cfg = azo.discrete_config(azo.ACROBOT, n_rollouts=300, epsilon=0.25, V_target_policy="on_policy", gamma=0.99)
+    out = azo.search(cfg, weights(cfg), roots("reset", 8), n_threads=4)
     assert out["counts"].sum() == 8 * 300 and out["node_n"][:, 0].max() == 300
     assert (out["en"][:, 0] > 0).all() and out["counters"][5] == 2 * out["counters"][1]
     tot = out["counts"].sum(1).astype(np.float64)
@@ -195,19 +195,19 @@ def test_oracle_search_epsilon_and_deep_counts():
 
 
 def test_oracle_search_wrap_cap():
-    cfg = M.config(n_rollouts=10)
+    cfg = azo.discrete_config(azo.ACROBOT, n_rollouts=10)
     rs = roots("reset", 4)
     rs[2, 0] = 1e6
     with pytest.raises(WrapCapReached):
-        M.search(cfg, weights(cfg), rs)
+        azo.search(cfg, weights(cfg), rs)
 
 
 def test_oracle_selfplay_reset_and_obs_rows():
     from oracle import selfplay as SP
-    cfg = M.config(n_rollouts=10)
+    cfg = azo.discrete_config(azo.ACROBOT, n_rollouts=10)
     cfg.math_mode = azo.MATH_DET
     r0 = roots("goal", 8)
-    steps = M.selfplay_run(cfg, weights(cfg), r0, steps=3, max_episode_length=2, seed=5)
+    steps = osp.run(cfg, weights(cfg), r0, steps=3, max_episode_length=2, seed=5)
     for k, rec in enumerate(steps):
         key = SP.step_seed(5, k)
         for t in np.nonzero(rec["done"])[0]:
@@ -217,7 +217,7 @@ def test_oracle_selfplay_reset_and_obs_rows():
     start = r0[0]
     want = np.array([det_cos(start[0]), det_sin(start[0]), det_cos(start[1]), det_sin(start[1]), start[2], start[3]]).astype(np.float32)
     assert np.array_equal(steps[0]["obs"][0], want)
-    assert np.array_equal(steps[1]["obs"], M.observe(cfg, steps[0]["env_state"]))
+    assert np.array_equal(steps[1]["obs"], azo.obs(cfg, steps[0]["env_state"]))
     assert set(np.concatenate([r["action_taken"] for r in steps]).tolist()) <= {0.0, 1.0, 2.0}
 
 
@@ -227,7 +227,7 @@ def test_engine_config_and_env_recognition():
     from alphazero_gym_b200.engine import ACROBOT, CARTPOLE, EngineConfig
     from alphazero_gym_b200.search.mcts import acrobot_obs, discrete_env, env_hidden_state, reward_model
     from alphazero_gym_b200.selfplay import initial_states
-    from mc_oracle import MountainCarEnv
+    from classic_control import MountainCarEnv
 
     c = EngineConfig(variant=DISCRETE, num_actions=3, state_dim=6, env=ACROBOT)
     assert c.c().flags & _cabi.FLAG_ENV_ACROBOT and _cabi.FLAG_ENV_ACROBOT == 64 and c.is_fused()

@@ -1,5 +1,5 @@
-"""Acrobot-v1 search on the GPU (AZG_FLAG_ENV_ACROBOT) against its CPU reference (tests/acrobot_oracle.py: the CPU oracle's discrete
-search with this env): the env step, every search schedule (one launch per simulation with FP32 and tensor-core evaluation, the
+"""Acrobot-v1 search on the GPU (AZG_FLAG_ENV_ACROBOT) against the CPU oracle's discrete
+search with this env: the env step, every search schedule (one launch per simulation with FP32 and tensor-core evaluation, the
 two-phase and the warpgroup whole-search kernels), the MT19937 and tape modes, sharding, the wrap cap, self-play and the drop-in
 classes.  Everything bit for bit on the tree dump, the root results and counters[:7]: same Philox streams, same deterministic sine
 and cosine, same RK4, same 6-input evaluation arithmetic, same three-way selection and tie-break."""
@@ -7,8 +7,8 @@ import numpy as np
 import pytest
 
 from oracle import azo
-import acrobot_oracle as M
-from acrobot_oracle import AcrobotEnv
+from oracle import selfplay as osp
+from classic_control import AcrobotEnv, det_cos, det_sin
 from parity import assert_tree_equal
 
 SMS = 148  # B200
@@ -28,7 +28,7 @@ def roots(kind, B, seed=3):
 def ac_config(act=azo.ACT_RELU, L=2, N=50, q8=False, hidden=128, **kw):
     d = dict(n_rollouts=N, n_hidden=L, activation=act, hidden=hidden, epsilon=0.0)
     d.update(kw)
-    cfg = M.config(**d)
+    cfg = azo.discrete_config(azo.ACROBOT, **d)
     cfg.math_mode, cfg.eval_mode = azo.MATH_DET, (azo.EVAL_Q8 if q8 else azo.EVAL_FP32)
     return cfg
 
@@ -46,8 +46,7 @@ def zero_head(cfg, w):
 
 def run(cfg, w, rs, **kw):
     import enginelib as E
-    from alphazero_gym_b200.engine import ACROBOT
-    return E.run_engine(cfg, w, rs, env=ACROBOT, kernel=True, **kw)
+    return E.run_engine(cfg, w, rs, kernel=True, **kw)
 
 
 def take(out, lo, hi):
@@ -55,7 +54,7 @@ def take(out, lo, hi):
 
 
 def check_full(cfg, w, rs, out, root_n=None):
-    ref = M.search(cfg, w, rs, root_n, n_threads=8)
+    ref = azo.search(cfg, w, rs, root_n, n_threads=8)
     assert_tree_equal(out, ref, discrete=True)
     assert np.array_equal(out["counters"][:7], ref["counters"][:7]), (out["counters"], ref["counters"])
     return ref
@@ -64,7 +63,7 @@ def check_full(cfg, w, rs, out, root_n=None):
 def check_slices(cfg, w, rs, out, n=256):
     B = rs.shape[0]
     for lo, hi in ((0, n), (B - n, B)):
-        ref = M.search(cfg, w, rs[lo:hi], tree_id0=lo, n_threads=8)
+        ref = azo.search(cfg, w, rs[lo:hi], tree_id0=lo, n_threads=8)
         assert_tree_equal(take(out, lo, hi), ref, discrete=True)
 
 
@@ -91,8 +90,8 @@ def test_env_step_equals_oracle_and_gym():
     cfg = ac_config()
     assert obs.shape == (len(cases), 6) and nxt.shape == (len(cases), 4)
     for i in range(len(cases)):
-        rn, rr, rt, ro = M.env_step(cfg, s[i], int(a[i]))
-        env = AcrobotEnv(s[i], sin=M.det_sin, cos=M.det_cos)
+        rn, rr, rt, ro = azo.env_step(cfg, s[i], int(a[i]))
+        env = AcrobotEnv(s[i], sin=det_sin, cos=det_cos)
         gob, gr, gd, _ = env.step(int(a[i]))
         for ref_s, ref_r, ref_t in ((rn, rr, rt), (env.state, gr, gd)):
             assert T.same(nxt[i], ref_s), (s[i], a[i])
@@ -196,9 +195,8 @@ def test_tape_mode():
     tapes = {"V": rng.uniform(-30, 0, (B, cfg.rows)).astype(np.float32), "prior": p / p.sum(-1, keepdims=True)}
     rs = roots("goal", B, seed=12)
     import enginelib as E
-    from alphazero_gym_b200.engine import ACROBOT
-    out = E.run_engine(cfg, None, rs, tapes=tapes, env=ACROBOT)
-    ref = M.search(cfg, None, rs, tapes=tapes, n_threads=8)
+    out = E.run_engine(cfg, None, rs, tapes=tapes)
+    ref = azo.search(cfg, None, rs, tapes=tapes, n_threads=8)
     assert_tree_equal(out, ref, discrete=True)
     assert np.array_equal(out["counters"][:4], ref["counters"][:4]) and out["counters"][6] == ref["counters"][6] > 0
 
@@ -213,7 +211,7 @@ def test_shard_offset_and_root_n():
     lo, hi = 300, 812
     part = run(cfg, w, rs[lo:hi], root_n_init=rn[lo:hi], tree_id0=lo)
     assert_tree_equal(take(full, lo, hi), part, discrete=True)
-    ref = M.search(cfg, w, rs[lo:lo + 64], rn[lo:lo + 64], tree_id0=lo, n_threads=8)
+    ref = azo.search(cfg, w, rs[lo:lo + 64], rn[lo:lo + 64], tree_id0=lo, n_threads=8)
     assert_tree_equal(take(full, lo, lo + 64), ref, discrete=True)
 
 
@@ -238,8 +236,8 @@ def test_wrap_cap_raises(fused):
     with pytest.raises(AzgError) as ei:
         run(cfg, weights(cfg), rs, fused=fused)
     assert ei.value.code == AZG_EWRAP
-    with pytest.raises(M.WrapCapReached):
-        M.search(cfg, weights(cfg), rs)
+    with pytest.raises(azo.WrapCapReached):
+        azo.search(cfg, weights(cfg), rs)
 
 
 # ------------------------------------------------------------------------------------------------------------------ self-play
@@ -248,16 +246,15 @@ def test_wrap_cap_raises(fused):
 @pytest.mark.parametrize("mode", ["det", "t1", "value"])
 def test_selfplay_equals_oracle(mode):
     import enginelib as E
-    from alphazero_gym_b200.engine import ACROBOT
     from alphazero_gym_b200.selfplay import SelfPlayDriver
     det, by_value, temp = mode == "det", mode == "value", {"value": 2.0}.get(mode, 1.0)
     cfg = ac_config(azo.ACT_RELU, 2, 30, q8=True)
     w = weights(cfg)
     B, steps, max_len = 64, 8, 4
     states0 = roots("goal", B, seed=21)
-    ref = M.selfplay_run(cfg, w, states0, steps, max_len, seed=cfg.seed, tree_id0=7, deterministic=det, by_value=by_value,
+    ref = osp.run(cfg, w, states0, steps, max_len, seed=cfg.seed, tree_id0=7, deterministic=det, by_value=by_value,
                          temperature=temp)
-    eng = E.SearchEngine(E.engine_config(cfg, B, env=ACROBOT))
+    eng = E.SearchEngine(E.engine_config(cfg, B))
     try:
         eng.set_weights(w)
         drv = SelfPlayDriver(eng, B, cfg.n_rollouts, max_episode_length=max_len, tree_id0=7, seed=cfg.seed, deterministic=det,
@@ -307,7 +304,7 @@ def test_dropin_search_agent_and_trainer():
                         V_target_policy="off_policy", device="cuda:0", root_state=None, seed=cfg.seed)
     mcts.search(Env=TimeLimit(AcrobotEnv(root[0])))
     state, actions, counts, Q, V = mcts.return_results("max_visit")
-    ref = M.search(cfg, w, root[:1], tree_id0=0)
+    ref = azo.search(cfg, w, root[:1], tree_id0=0)
     assert state.shape == (6,) and np.array_equal(state, acrobot_obs(root[0])) and np.array_equal(actions, [0, 1, 2])
     assert np.array_equal(counts, ref["counts"][0]) and np.array_equal(Q, ref["Q"][0]) and V == ref["V_target"][0]
     a = int(counts.argmax())
@@ -320,7 +317,7 @@ def test_dropin_search_agent_and_trainer():
                                                            epsilon=0.0, V_target_policy="off_policy", device="cuda:0",
                                                            root_state=None, seed=cfg.seed))
     action, s2, acts, cnts, Qs, V2 = agent.act(TimeLimit(AcrobotEnv(root[1])))
-    ref2 = M.search(cfg, w, root[1:2], tree_id0=0)
+    ref2 = azo.search(cfg, w, root[1:2], tree_id0=0)
     assert np.array_equal(cnts, ref2["counts"][0]) and np.array_equal(Qs, ref2["Q"][0]) and 0 <= int(action) < 3
     assert np.asarray(s2).shape == (6,)
     batch = {"obs": torch.tensor(np.stack([state, s2]), dtype=torch.float32, device="cuda"),

@@ -1,4 +1,4 @@
-"""MountainCarContinuous-v0 on the CPU: the CPU reference's env (tests/mcc_oracle.c) against gym's step() restated in plain Python,
+"""MountainCarContinuous-v0 on the CPU: the CPU oracle's env against gym's step() restated in plain Python,
 its continuous search through the env's terminal paths, and the host-side plumbing that selects the env (no GPU needed)."""
 import math
 import re
@@ -7,8 +7,9 @@ import numpy as np
 import pytest
 
 from oracle import azo
-import mcc_oracle as M
-from mcc_oracle import Continuous_MountainCarEnv, R_SCALE, det_cos
+from oracle import selfplay as osp
+from oracle.azo import R_SCALE
+from classic_control import Continuous_MountainCarEnv, det_cos
 
 
 def edge_cases():
@@ -36,13 +37,13 @@ def _bits(x):
 
 @pytest.mark.parametrize("math_mode", [azo.MATH_LIBM, azo.MATH_DET])
 def test_env_step_equals_gym_restatement(math_mode):
-    """mcc_oracle.env_step == Continuous_MountainCarEnv.step bit for bit (state, reward, done, observation) with the same cosine."""
-    cfg = M.config()
+    """azo.env_step == Continuous_MountainCarEnv.step bit for bit (state, reward, done, observation) with the same cosine."""
+    cfg = azo.continuous_config(azo.MOUNTAIN_CAR_CONTINUOUS)
     cfg.math_mode = math_mode
     cos = math.cos if math_mode == azo.MATH_LIBM else det_cos
     n_done = n_wall = 0
     for s, a in edge_cases():
-        nxt, r, term, obs = M.env_step(cfg, np.array(s, np.float64), float(a))
+        nxt, r, term, obs = azo.env_step(cfg, np.array(s, np.float64), float(a))
         env = Continuous_MountainCarEnv(s, cos=cos)
         gs, gr, gdone, _ = env.step(np.array([a], np.float32))
         assert np.array_equal(_bits(nxt), _bits(gs)), (s, a, nxt, gs)
@@ -55,20 +56,20 @@ def test_env_step_equals_gym_restatement(math_mode):
 
 
 def test_env_step_signed_zeros_and_reward():
-    cfg = M.config()
+    cfg = azo.continuous_config(azo.MOUNTAIN_CAR_CONTINUOUS)
     # a zero action pays +0.0 (0 - 0.0 with the int 0), not -0.0
-    _, r, term, _ = M.env_step(cfg, np.array([-0.5, 0.0]), 0.0)
+    _, r, term, _ = azo.env_step(cfg, np.array([-0.5, 0.0]), 0.0)
     assert not term and _bits(r) == _bits(0.0)
-    _, r, _, _ = M.env_step(cfg, np.array([-0.5, 0.0]), -0.0)
+    _, r, _, _ = azo.env_step(cfg, np.array([-0.5, 0.0]), -0.0)
     assert _bits(r) == _bits(0.0)
     # the reward uses the unclipped action: pow(a, 2) * 0.1 of an f32 is exact in f64 before the * 0.1
-    _, r, _, _ = M.env_step(cfg, np.array([-0.5, 0.0]), 3.0)
+    _, r, _, _ = azo.env_step(cfg, np.array([-0.5, 0.0]), 3.0)
     assert r == -(9.0 * 0.1)
     # the left wall: velocity becomes +0.0
-    s, _, _, _ = M.env_step(cfg, np.array([-1.2, -0.03]), -1.0)
+    s, _, _, _ = azo.env_step(cfg, np.array([-1.2, -0.03]), -1.0)
     assert s[0] == -1.2 and _bits(s[1]) == _bits(0.0)
     # the goal: done, reward 100 - 0.1 a^2
-    s, r, term, _ = M.env_step(cfg, np.array([0.449, 0.07]), 0.5)
+    s, r, term, _ = azo.env_step(cfg, np.array([0.449, 0.07]), 0.5)
     assert term and s[0] >= 0.45 and r == 100.0 - (0.5 * 0.5) * 0.1
     # velocity -0.0 at the goal line counts as >= goal_velocity (0)
     env = Continuous_MountainCarEnv((0.45, -0.0))
@@ -77,8 +78,8 @@ def test_env_step_signed_zeros_and_reward():
 
 def test_env_step_nan_action_passes_the_clip():
     """max(nan, -1.0) is nan in Python: a NaN action makes the velocity NaN (and the done test False), in both restatements."""
-    cfg = M.config()
-    s, r, term, _ = M.env_step(cfg, np.array([-0.5, 0.01]), float("nan"))
+    cfg = azo.continuous_config(azo.MOUNTAIN_CAR_CONTINUOUS)
+    s, r, term, _ = azo.env_step(cfg, np.array([-0.5, 0.01]), float("nan"))
     gs, gr, gdone, _ = Continuous_MountainCarEnv((-0.5, 0.01)).step(np.array([np.nan], np.float32))
     assert np.isnan(s).all() and np.isnan(gs).all() and np.isnan(r) and np.isnan(gr) and not term and not gdone
 
@@ -96,7 +97,7 @@ def valley_roots(B, seed=4):
 def mcc_config(**kw):
     d = dict(n_rollouts=100, num_components=2, n_hidden=2, activation=azo.ACT_RELU)
     d.update(kw)
-    return M.config(**d)
+    return azo.continuous_config(azo.MOUNTAIN_CAR_CONTINUOUS, **d)
 
 
 def mcc_weights(cfg, seed=34):
@@ -111,7 +112,7 @@ def test_oracle_search_terminal_paths():
     cfg = mcc_config()
     w = mcc_weights(cfg)
     roots = near_goal_roots(64)
-    out = M.search(cfg, w, roots, n_threads=4)
+    out = azo.search(cfg, w, roots, n_threads=4)
     assert out["counters"][6] > 0
     term = out["terminal"].astype(bool)
     assert term.sum() > 0 and not term[:, 0].any()  # the root is never terminal, even at the goal
@@ -135,11 +136,11 @@ def test_oracle_search_terminal_paths():
 
 def test_oracle_search_valley_roots_and_state_dim():
     cfg = mcc_config(n_rollouts=50)
-    out = M.search(cfg, mcc_weights(cfg), valley_roots(16), n_threads=4)
+    out = azo.search(cfg, mcc_weights(cfg), valley_roots(16), n_threads=4)
     assert out["counts"].sum() == 16 * 50
     assert (out["state"][:, 0] == valley_roots(16)).all()
     with pytest.raises(ValueError):  # the env needs state_dim 2
-        M.search(mcc_config(state_dim=3), mcc_weights(mcc_config(state_dim=3)), valley_roots(2))
+        azo.search(mcc_config(state_dim=3), mcc_weights(mcc_config(state_dim=3)), valley_roots(2))
 
 
 def test_oracle_selfplay_reset():
@@ -147,7 +148,7 @@ def test_oracle_selfplay_reset():
     from oracle import selfplay as SP
     cfg = mcc_config(n_rollouts=10)
     roots = near_goal_roots(8)
-    steps = M.selfplay_run(cfg, mcc_weights(cfg), roots, steps=3, max_episode_length=2, seed=5)
+    steps = osp.run(cfg, mcc_weights(cfg), roots, steps=3, max_episode_length=2, seed=5)
     for k, rec in enumerate(steps):
         key = SP.step_seed(5, k)
         for t in np.nonzero(rec["done"])[0]:

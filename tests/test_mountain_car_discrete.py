@@ -1,4 +1,4 @@
-"""MountainCar-v0 on the CPU: the CPU reference's env (tests/mc_oracle.c) against gym's step() restated in plain Python, its discrete
+"""MountainCar-v0 on the CPU: the CPU oracle's env against gym's step() restated in plain Python, its discrete
 search over three actions through ties, epsilon picks, terminal nodes and visit counts past 255, and the host-side plumbing that selects
 the env (no GPU needed)."""
 import math
@@ -8,8 +8,8 @@ import numpy as np
 import pytest
 
 from oracle import azo
-import mc_oracle as M
-from mc_oracle import MountainCarEnv, det_cos
+from oracle import selfplay as osp
+from classic_control import MountainCarEnv, det_cos
 
 
 def edge_cases():
@@ -34,13 +34,13 @@ def _bits(x):
 
 @pytest.mark.parametrize("math_mode", [azo.MATH_LIBM, azo.MATH_DET])
 def test_env_step_equals_gym_restatement(math_mode):
-    """mc_oracle.env_step == MountainCarEnv.step bit for bit (state, reward, done, observation) with the same cosine."""
-    cfg = M.config()
+    """azo.env_step == MountainCarEnv.step bit for bit (state, reward, done, observation) with the same cosine."""
+    cfg = azo.discrete_config(azo.MOUNTAIN_CAR)
     cfg.math_mode = math_mode
     cos = math.cos if math_mode == azo.MATH_LIBM else det_cos
     n_done = n_wall = 0
     for s, a in edge_cases():
-        nxt, r, term, obs = M.env_step(cfg, np.array(s, np.float64), a)
+        nxt, r, term, obs = azo.env_step(cfg, np.array(s, np.float64), a)
         gs, gr, gdone, _ = MountainCarEnv(s, cos=cos).step(a)
         gs = np.asarray(gs, np.float64)
         assert np.array_equal(_bits(nxt), _bits(gs)), (s, a, nxt, gs)
@@ -53,30 +53,30 @@ def test_env_step_equals_gym_restatement(math_mode):
 
 
 def test_env_step_edges():
-    cfg = M.config()
+    cfg = azo.discrete_config(azo.MOUNTAIN_CAR)
     # the left wall: velocity becomes +0.0 (the int 0)
-    s, _, _, _ = M.env_step(cfg, np.array([-1.2, -0.03]), 0)
+    s, _, _, _ = azo.env_step(cfg, np.array([-1.2, -0.03]), 0)
     assert s[0] == -1.2 and _bits(s[1]) == _bits(0.0)
     # action 1 applies zero force: the velocity change is the gravity term alone
-    s, _, _, _ = M.env_step(cfg, np.array([-0.5, 0.01]), 1)
+    s, _, _, _ = azo.env_step(cfg, np.array([-0.5, 0.01]), 1)
     assert s[1] == 0.01 + (0.0 + det_cos(3 * -0.5) * -0.0025)
     # pushing left / right differ by exactly 2 * force before rounding
-    s0, _, _, _ = M.env_step(cfg, np.array([-0.5, 0.0]), 0)
-    s2, _, _, _ = M.env_step(cfg, np.array([-0.5, 0.0]), 2)
+    s0, _, _, _ = azo.env_step(cfg, np.array([-0.5, 0.0]), 0)
+    s2, _, _, _ = azo.env_step(cfg, np.array([-0.5, 0.0]), 2)
     assert s0[1] < s2[1]
     # the goal line: done with velocity +0 and -0, not with a negative velocity, nor for a NaN state
     for v, want in ((0.0, True), (-0.0, True), (-1e-300, False)):
         env = MountainCarEnv((0.5, v))
         env.state = (0.5, v)
         assert bool(0.5 >= env.goal_position and v >= env.goal_velocity) == want
-    _, r, term, _ = M.env_step(cfg, np.array([0.499, 0.07]), 2)
+    _, r, term, _ = azo.env_step(cfg, np.array([0.499, 0.07]), 2)
     assert term and r == -1.0
-    s, _, term, _ = M.env_step(cfg, np.array([np.nan, 0.0]), 1)
+    s, _, term, _ = azo.env_step(cfg, np.array([np.nan, 0.0]), 1)
     assert np.isnan(s).all() and not term
     # both speed clips
-    s, _, _, _ = M.env_step(cfg, np.array([0.55, 0.07]), 2)  # cos(1.65) < 0: gravity pushes right too
+    s, _, _, _ = azo.env_step(cfg, np.array([0.55, 0.07]), 2)  # cos(1.65) < 0: gravity pushes right too
     assert s[1] == 0.07
-    s, _, _, _ = M.env_step(cfg, np.array([0.0, -0.07]), 0)
+    s, _, _, _ = azo.env_step(cfg, np.array([0.0, -0.07]), 0)
     assert s[1] == -0.07
 
 
@@ -102,9 +102,9 @@ def zero_head(cfg, w):
 def test_oracle_search_ties_and_terminals():
     """Near the goal: terminal expansions (V = 0, r = -1), traces that end on an existing terminal node (counters[6]), and three-way
     ties resolved by the random pick among the winners (all three actions taken first at some fresh node)."""
-    cfg = M.config(n_rollouts=50, epsilon=0.0)
+    cfg = azo.discrete_config(azo.MOUNTAIN_CAR, n_rollouts=50, epsilon=0.0)
     w = zero_head(cfg, weights(cfg))
-    out = M.search(cfg, w, roots("goal", 64), n_threads=4)
+    out = azo.search(cfg, w, roots("goal", 64), n_threads=4)
     assert out["counters"][6] > 0
     term = out["terminal"].astype(bool)
     assert term.any() and not term[:, 0].any()
@@ -121,8 +121,8 @@ def test_oracle_search_ties_and_terminals():
 
 def test_oracle_search_epsilon_and_deep_counts():
     """epsilon = 0.25 makes random picks of every action; N = 300 pushes the root's visit count past 255."""
-    cfg = M.config(n_rollouts=300, epsilon=0.25, V_target_policy="on_policy", gamma=0.99)
-    out = M.search(cfg, weights(cfg), roots("valley", 8), n_threads=4)
+    cfg = azo.discrete_config(azo.MOUNTAIN_CAR, n_rollouts=300, epsilon=0.25, V_target_policy="on_policy", gamma=0.99)
+    out = azo.search(cfg, weights(cfg), roots("valley", 8), n_threads=4)
     assert out["counts"].sum() == 8 * 300 and out["node_n"][:, 0].max() == 300
     assert (out["en"][:, 0, 2] > 0).all() and out["counters"][5] == 2 * out["counters"][1]
     tot = out["counts"].sum(1).astype(np.float64)
@@ -134,9 +134,9 @@ def test_oracle_search_epsilon_and_deep_counts():
 
 def test_oracle_selfplay_reset_and_reuse():
     from oracle import selfplay as SP
-    cfg = M.config(n_rollouts=10)
+    cfg = azo.discrete_config(azo.MOUNTAIN_CAR, n_rollouts=10)
     r0 = roots("goal", 8)
-    steps = M.selfplay_run(cfg, weights(cfg), r0, steps=3, max_episode_length=2, seed=5)
+    steps = osp.run(cfg, weights(cfg), r0, steps=3, max_episode_length=2, seed=5)
     for k, rec in enumerate(steps):
         key = SP.step_seed(5, k)
         for t in np.nonzero(rec["done"])[0]:
@@ -153,7 +153,7 @@ def test_engine_config_and_env_recognition():
     from alphazero_gym_b200.engine import CARTPOLE, MOUNTAIN_CAR, EngineConfig
     from alphazero_gym_b200.search.mcts import discrete_env, env_hidden_state, reward_model
     from alphazero_gym_b200.selfplay import initial_states
-    from mcc_oracle import Continuous_MountainCarEnv
+    from classic_control import Continuous_MountainCarEnv
 
     c = EngineConfig(variant=DISCRETE, num_actions=3, state_dim=2, env=MOUNTAIN_CAR)
     assert c.c().flags & _cabi.FLAG_ENV_MOUNTAIN_CAR and _cabi.FLAG_ENV_MOUNTAIN_CAR == 32 and c.is_fused()
@@ -189,7 +189,7 @@ def test_engine_config_and_env_recognition():
 def test_dropin_refusals_without_gpu():
     """MCTSDiscrete: MountainCar with num_actions other than 3 and the continuous env raise before any engine exists."""
     from alphazero_gym_b200.search.mcts import MCTSContinuous, MCTSDiscrete
-    from mcc_oracle import Continuous_MountainCarEnv
+    from classic_control import Continuous_MountainCarEnv
     m = MCTSDiscrete(model=None, num_actions=2, n_rollouts=8, c_uct=1.5, gamma=1.0, epsilon=0.0, V_target_policy="off_policy",
                      device="cuda:0", root_state=None)
     with pytest.raises(ValueError):

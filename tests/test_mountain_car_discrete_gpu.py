@@ -1,5 +1,5 @@
-"""MountainCar-v0 search on the GPU (AZG_FLAG_ENV_MOUNTAIN_CAR) against its CPU reference (tests/mc_oracle.py: the CPU oracle's
-discrete search with this env): the env step, every search schedule (one launch per simulation with FP32 and tensor-core evaluation,
+"""MountainCar-v0 search on the GPU (AZG_FLAG_ENV_MOUNTAIN_CAR) against the CPU oracle's
+discrete search with this env: the env step, every search schedule (one launch per simulation with FP32 and tensor-core evaluation,
 the two-phase and the warpgroup whole-search kernels), the MT19937 and tape modes, sharding, self-play and the drop-in classes.
 Everything bit for bit on the tree dump, the root results and counters[:7]: same Philox streams, same deterministic cosine, same
 evaluation arithmetic, same three-way selection and tie-break."""
@@ -7,8 +7,8 @@ import numpy as np
 import pytest
 
 from oracle import azo
-import mc_oracle as M
-from mc_oracle import MountainCarEnv
+from oracle import selfplay as osp
+from classic_control import MountainCarEnv, det_cos
 from parity import assert_tree_equal
 
 SMS = 148  # B200
@@ -28,7 +28,7 @@ def roots(kind, B, seed=3):
 def mc_config(act=azo.ACT_RELU, L=2, N=50, q8=False, hidden=128, **kw):
     d = dict(n_rollouts=N, n_hidden=L, activation=act, hidden=hidden, epsilon=0.0)
     d.update(kw)
-    cfg = M.config(**d)
+    cfg = azo.discrete_config(azo.MOUNTAIN_CAR, **d)
     cfg.math_mode, cfg.eval_mode = azo.MATH_DET, (azo.EVAL_Q8 if q8 else azo.EVAL_FP32)
     return cfg
 
@@ -46,8 +46,7 @@ def zero_head(cfg, w):
 
 def run(cfg, w, rs, **kw):
     import enginelib as E
-    from alphazero_gym_b200.engine import MOUNTAIN_CAR
-    return E.run_engine(cfg, w, rs, env=MOUNTAIN_CAR, kernel=True, **kw)
+    return E.run_engine(cfg, w, rs, kernel=True, **kw)
 
 
 def take(out, lo, hi):
@@ -55,7 +54,7 @@ def take(out, lo, hi):
 
 
 def check_full(cfg, w, rs, out, root_n=None):
-    ref = M.search(cfg, w, rs, root_n, n_threads=8)
+    ref = azo.search(cfg, w, rs, root_n, n_threads=8)
     assert_tree_equal(out, ref, discrete=True)
     assert np.array_equal(out["counters"][:7], ref["counters"][:7]), (out["counters"], ref["counters"])
     return ref
@@ -64,7 +63,7 @@ def check_full(cfg, w, rs, out, root_n=None):
 def check_slices(cfg, w, rs, out, n=256):
     B = rs.shape[0]
     for lo, hi in ((0, n), (B - n, B)):
-        ref = M.search(cfg, w, rs[lo:hi], tree_id0=lo, n_threads=8)
+        ref = azo.search(cfg, w, rs[lo:hi], tree_id0=lo, n_threads=8)
         assert_tree_equal(take(out, lo, hi), ref, discrete=True)
 
 
@@ -86,8 +85,8 @@ def test_env_step_equals_oracle_and_gym():
     cfg = mc_config()
     assert obs.shape == (len(cases), 2) and nxt.shape == (len(cases), 2)
     for i in range(len(cases)):
-        rn, rr, rt, ro = M.env_step(cfg, s[i], int(a[i]))
-        gs, gr, gd, _ = MountainCarEnv(s[i], cos=M.det_cos).step(int(a[i]))
+        rn, rr, rt, ro = azo.env_step(cfg, s[i], int(a[i]))
+        gs, gr, gd, _ = MountainCarEnv(s[i], cos=det_cos).step(int(a[i]))
         for ref_s, ref_r, ref_t in ((rn, rr, rt), (gs, gr, gd)):
             assert np.array_equal(nxt[i].view(np.uint64), np.asarray(ref_s, np.float64).view(np.uint64)), (s[i], a[i])
             assert rew[i] == ref_r == -1.0 and bool(term[i]) == bool(ref_t)
@@ -191,9 +190,8 @@ def test_tape_mode():
     tapes = {"V": rng.uniform(-30, 0, (B, cfg.rows)).astype(np.float32), "prior": p / p.sum(-1, keepdims=True)}
     rs = roots("goal", B, seed=12)
     import enginelib as E
-    from alphazero_gym_b200.engine import MOUNTAIN_CAR
-    out = E.run_engine(cfg, None, rs, tapes=tapes, env=MOUNTAIN_CAR)
-    ref = M.search(cfg, None, rs, tapes=tapes, n_threads=8)
+    out = E.run_engine(cfg, None, rs, tapes=tapes)
+    ref = azo.search(cfg, None, rs, tapes=tapes, n_threads=8)
     assert_tree_equal(out, ref, discrete=True)
     assert np.array_equal(out["counters"][:4], ref["counters"][:4]) and out["counters"][6] == ref["counters"][6] > 0
 
@@ -211,7 +209,7 @@ def test_shard_offset_and_root_n():
     halves = [run(cfg, w, rs[a:b], root_n_init=rn[a:b], tree_id0=a) for a, b in ((0, 512), (512, 1024))]
     for k in ("counts", "Q", "V_target", "eW", "en", "node_n"):
         assert np.array_equal(np.concatenate([h[k] for h in halves]), full[k]), k
-    ref = M.search(cfg, w, rs[lo:lo + 64], rn[lo:lo + 64], tree_id0=lo, n_threads=8)
+    ref = azo.search(cfg, w, rs[lo:lo + 64], rn[lo:lo + 64], tree_id0=lo, n_threads=8)
     assert_tree_equal(take(full, lo, lo + 64), ref, discrete=True)
 
 
@@ -231,16 +229,15 @@ def test_nan_weights_raise():
 @pytest.mark.parametrize("mode", ["det", "t05", "t1", "t2", "value"])
 def test_selfplay_equals_oracle(mode):
     import enginelib as E
-    from alphazero_gym_b200.engine import MOUNTAIN_CAR
     from alphazero_gym_b200.selfplay import SelfPlayDriver
     det, by_value, temp = mode == "det", mode == "value", {"t05": 0.5, "t2": 2.0, "value": 2.0}.get(mode, 1.0)
     cfg = mc_config(azo.ACT_RELU, 2, 30, q8=True)
     w = weights(cfg)
     B, steps, max_len = 64, 8, 4
     states0 = roots("goal", B, seed=21)
-    ref = M.selfplay_run(cfg, w, states0, steps, max_len, seed=cfg.seed, tree_id0=7, deterministic=det, by_value=by_value,
+    ref = osp.run(cfg, w, states0, steps, max_len, seed=cfg.seed, tree_id0=7, deterministic=det, by_value=by_value,
                          temperature=temp)
-    eng = E.SearchEngine(E.engine_config(cfg, B, env=MOUNTAIN_CAR))
+    eng = E.SearchEngine(E.engine_config(cfg, B))
     try:
         eng.set_weights(w)
         drv = SelfPlayDriver(eng, B, cfg.n_rollouts, max_episode_length=max_len, tree_id0=7, seed=cfg.seed, deterministic=det,
@@ -289,18 +286,18 @@ def test_dropin_search_agent_and_trainer():
                         V_target_policy="off_policy", device="cuda:0", root_state=None, seed=cfg.seed)
     mcts.search(Env=TimeLimit(MountainCarEnv(root[0])))
     state, actions, counts, Q, V = mcts.return_results("max_visit")
-    ref = M.search(cfg, w, root[:1], tree_id0=0)
+    ref = azo.search(cfg, w, root[:1], tree_id0=0)
     assert np.array_equal(state, root[0]) and np.array_equal(actions, [0, 1, 2])
     assert np.array_equal(counts, ref["counts"][0]) and np.array_equal(Q, ref["Q"][0]) and V == ref["V_target"][0]
     a = int(counts.argmax())
-    nxt, _, _, _ = M.env_step(cfg, root[0], a)
+    nxt, _, _, _ = azo.env_step(cfg, root[0], a)
     mcts.forward(a, nxt)
     assert mcts.root_node is not None and mcts.root_node.n == ref["node_n"][0, ref["echild"][0, 0, a]]
     agent = DiscreteAgent.from_modules(model, MCTSDiscrete(model=model, num_actions=3, n_rollouts=50, c_uct=cfg.c_uct, gamma=cfg.gamma,
                                                            epsilon=0.0, V_target_policy="off_policy", device="cuda:0",
                                                            root_state=None, seed=cfg.seed))
     action, s2, acts, cnts, Qs, V2 = agent.act(TimeLimit(MountainCarEnv(root[1])))
-    ref2 = M.search(cfg, w, root[1:2], tree_id0=0)
+    ref2 = azo.search(cfg, w, root[1:2], tree_id0=0)
     assert np.array_equal(cnts, ref2["counts"][0]) and np.array_equal(Qs, ref2["Q"][0]) and 0 <= int(action) < 3
     batch = {"obs": torch.tensor(np.stack([state, s2]), dtype=torch.float32, device="cuda"),
              "actions": torch.tensor(np.stack([actions, acts]), dtype=torch.float32, device="cuda"),

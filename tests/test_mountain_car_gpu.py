@@ -1,5 +1,5 @@
-"""MountainCarContinuous-v0 search on the GPU (AZG_FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS) against its CPU reference (tests/mcc_oracle.py:
-the CPU oracle's search with this env): the env step, every
+"""MountainCarContinuous-v0 search on the GPU (AZG_FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS) against the CPU oracle's
+search with this env: the env step, every
 search schedule (one launch per simulation with FP32 and tensor-core evaluation, the two-phase and the warpgroup whole-search
 kernels), the MT19937 and tape modes, sharding, self-play and the drop-in classes.  Everything bit for bit: same Philox streams,
 same deterministic cosine, same evaluation arithmetic.  Roots near the goal make the search expand terminal nodes (V = 0) and
@@ -8,8 +8,8 @@ import numpy as np
 import pytest
 
 from oracle import azo
-import mcc_oracle as M
-from mcc_oracle import Continuous_MountainCarEnv
+from oracle import selfplay as osp
+from classic_control import Continuous_MountainCarEnv, det_cos
 from parity import assert_tree_equal
 
 SMS = 148  # B200
@@ -34,7 +34,7 @@ def roots(kind, B, seed=3):
 
 
 def mcc_config(K=2, act=azo.ACT_RELU, L=2, N=100, q8=False, hidden=128, **kw):
-    cfg = M.config(n_rollouts=N, num_components=K, n_hidden=L, activation=act, hidden=hidden, **kw)
+    cfg = azo.continuous_config(azo.MOUNTAIN_CAR_CONTINUOUS, n_rollouts=N, num_components=K, n_hidden=L, activation=act, hidden=hidden, **kw)
     cfg.math_mode, cfg.eval_mode = azo.MATH_DET, (azo.EVAL_Q8 if q8 else azo.EVAL_FP32)
     return cfg
 
@@ -46,12 +46,11 @@ def weights(cfg, seed=34):
 
 def run(cfg, w, rs, **kw):
     import enginelib as E
-    from alphazero_gym_b200.engine import MOUNTAIN_CAR_CONTINUOUS
-    return E.run_engine(cfg, w, rs, env=MOUNTAIN_CAR_CONTINUOUS, kernel=True, **kw)
+    return E.run_engine(cfg, w, rs, kernel=True, **kw)
 
 
 def oracle_slice(cfg, w, rs, lo, hi, **kw):
-    return M.search(cfg, w, rs[lo:hi], tree_id0=lo, n_threads=8, **kw)
+    return azo.search(cfg, w, rs[lo:hi], tree_id0=lo, n_threads=8, **kw)
 
 
 def take(out, lo, hi):
@@ -67,7 +66,7 @@ def fit(out, ref):
 
 def check_full(cfg, w, rs, out):
     """dump + results + counters[:7] of the whole batch bit for bit."""
-    ref = M.search(cfg, w, rs, n_threads=8)
+    ref = azo.search(cfg, w, rs, n_threads=8)
     assert_tree_equal(fit(out, ref), ref, discrete=False)
     assert np.array_equal(out["counters"][:7], ref["counters"][:7]), (out["counters"], ref["counters"])
     return ref
@@ -100,8 +99,8 @@ def test_env_step_equals_oracle_and_gym():
     cfg = mcc_config()
     assert obs.shape == (len(cases), 2)
     for i in range(len(cases)):
-        rn, rr, rt, ro = M.env_step(cfg, s[i], float(a[i]))
-        gs, gr, gd, _ = Continuous_MountainCarEnv(s[i], cos=M.det_cos).step(a[i:i + 1])
+        rn, rr, rt, ro = azo.env_step(cfg, s[i], float(a[i]))
+        gs, gr, gd, _ = Continuous_MountainCarEnv(s[i], cos=det_cos).step(a[i:i + 1])
         for ref_s, ref_r, ref_t in ((rn, rr, rt), (gs, gr, gd)):
             assert np.array_equal(nxt[i].view(np.uint64), np.asarray(ref_s, np.float64).view(np.uint64)), (s[i], a[i])
             assert rew[i:i + 1].view(np.uint64)[0] == np.float64(ref_r).view(np.uint64), (s[i], a[i], rew[i], ref_r)
@@ -189,9 +188,8 @@ def test_tape_mode():
     tapes = {"V": rng.uniform(-1, 1, (B, cfg.rows)).astype(np.float32), "action": rng.uniform(-1.2, 1.2, (B, cfg.rows)).astype(np.float32)}
     rs = roots("goal", B, seed=12)
     import enginelib as E
-    from alphazero_gym_b200.engine import MOUNTAIN_CAR_CONTINUOUS
-    out = E.run_engine(cfg, None, rs, tapes=tapes, env=MOUNTAIN_CAR_CONTINUOUS)
-    ref = M.search(cfg, None, rs, tapes=tapes, n_threads=8)
+    out = E.run_engine(cfg, None, rs, tapes=tapes)
+    ref = azo.search(cfg, None, rs, tapes=tapes, n_threads=8)
     assert_tree_equal(fit(out, ref), ref, discrete=False, skip=("head",))
     assert np.array_equal(out["counters"][:4], ref["counters"][:4]) and out["counters"][6] == ref["counters"][6] > 0
 
@@ -213,14 +211,13 @@ def test_shard_with_offset_tree_ids():
 @pytest.mark.parametrize("by_value", [False, True])
 def test_selfplay_equals_oracle(by_value):
     import enginelib as E
-    from alphazero_gym_b200.engine import MOUNTAIN_CAR_CONTINUOUS
     from alphazero_gym_b200.selfplay import SelfPlayDriver
     cfg = mcc_config(2, azo.ACT_ELU, 3, 30, q8=True)
     w = weights(cfg)
     B, steps, max_len = 64, 8, 4
     states0 = roots("goal", B, seed=21)
-    ref = M.selfplay_run(cfg, w, states0, steps, max_len, seed=cfg.seed, tree_id0=7, by_value=by_value)
-    eng = E.SearchEngine(E.engine_config(cfg, B, env=MOUNTAIN_CAR_CONTINUOUS))
+    ref = osp.run(cfg, w, states0, steps, max_len, seed=cfg.seed, tree_id0=7, by_value=by_value)
+    eng = E.SearchEngine(E.engine_config(cfg, B))
     try:
         eng.set_weights(w)
         drv = SelfPlayDriver(eng, B, cfg.n_rollouts, max_episode_length=max_len, tree_id0=7, seed=cfg.seed,
@@ -271,7 +268,7 @@ def test_dropin_search_agent_and_trainer():
                           V_target_policy="off_policy", device="cuda:0", root_state=None, seed=cfg.seed)
     mcts.search(Env=env)
     state, actions, counts, Q, V = mcts.return_results("max_visit")
-    ref = M.search(cfg, w, root[:1], tree_id0=0)
+    ref = azo.search(cfg, w, root[:1], tree_id0=0)
     C = int(ref["n_children"][0])
     assert np.array_equal(state, root[0]) and actions.shape == (C,)
     assert np.array_equal(counts, ref["counts"][0, :C]) and np.array_equal(Q, ref["Q"][0, :C]) and V == ref["V_target"][0]
@@ -280,7 +277,7 @@ def test_dropin_search_agent_and_trainer():
     agent = ContinuousAgent.from_modules(model, mcts)
     env2 = Continuous_MountainCarEnv(root[1])
     action, s2, acts, cnts, Qs, V2 = agent.act(env2)
-    ref2 = M.search(cfg, w, root[1:2], tree_id0=1)
+    ref2 = azo.search(cfg, w, root[1:2], tree_id0=1)
     C2 = int(ref2["n_children"][0])
     assert np.array_equal(cnts, ref2["counts"][0, :C2]) and np.array_equal(Qs, ref2["Q"][0, :C2])
     assert action[0] == acts[cnts.argmax()] and np.array_equal(s2, root[1])
@@ -300,7 +297,7 @@ def test_dropin_search_agent_and_trainer():
     eng.search(torch.from_numpy(root[:1]).cuda(), 50)
     eng.status()
     got = eng.root_results()
-    ref3 = M.search(cfg, after.cpu().numpy(), root[:1], tree_id0=0)
+    ref3 = azo.search(cfg, after.cpu().numpy(), root[:1], tree_id0=0)
     assert np.array_equal(got["counts"].cpu().numpy()[0, :ref3["counts"].shape[1]], ref3["counts"][0])
     mcts.close()
 
