@@ -23,6 +23,7 @@
 #include "common.cuh"
 #include "env.cuh"
 #include "mlp.cuh"
+#include "mlp_stream.cuh"
 #include "qmlp.cuh"
 #include "qmlp2.cuh"
 #include "search_wg.cuh"
@@ -49,6 +50,8 @@ struct azg_engine {
     int64_t n_weights = 0;
     int wcount = 0;
     size_t mlp_smem = 0;
+    bool mlp_stream = false;  // hidden width other than 64 / 128: the evaluation streams the hidden layers (mlp_stream.cuh)
+    MlpStreamPlan splan;
     int sm_count = 0;
     // device memory
     DRow* drows = nullptr;
@@ -174,7 +177,7 @@ extern "C" int azg_create(const azg_config* cfg, azg_engine** out) {
     const azg_config& c = *cfg;
     if (c.variant != AZG_DISCRETE && c.variant != AZG_CONTINUOUS) return fail(AZG_EINVAL, "variant must be AZG_DISCRETE or AZG_CONTINUOUS");
     if (c.max_rollouts < 1 || c.max_trees < 1) return fail(AZG_EINVAL, "max_rollouts and max_trees must be >= 1");
-    if (c.hidden != 128 && c.hidden != 64) return fail(AZG_EINVAL, "hidden width must be 64 or 128 (weights are staged in shared memory)");
+    if (c.hidden < 32 || c.hidden > 256 || c.hidden % 32 != 0) return fail(AZG_EINVAL, "hidden width must be a multiple of 32 from 32 to 256");
     if (c.n_hidden < 1 || c.n_hidden > 4) return fail(AZG_EINVAL, "n_hidden must be in 1..4");
     if (c.activation < AZG_ACT_RELU || c.activation > AZG_ACT_HARDSWISH) return fail(AZG_EINVAL, "activation must be one of AZG_ACT_*");
     if ((c.flags & AZG_FLAG_EVAL_Q8) && c.activation > AZG_ACT_ELU)
@@ -227,10 +230,27 @@ extern "C" int azg_create(const azg_config* cfg, azg_engine** out) {
     nw += H + 1 + (int64_t)e->P * H + e->P;
     e->n_weights = nw;
     e->wcount = c.state_dim * H + H + (c.n_hidden - 1) * (H * H + H) + H * e->PO_PAD + e->PO_PAD;
-    e->mlp_smem = ((size_t)e->wcount + (size_t)MLP_NGRP * (H + e->PO_PAD) * MLP_UNIT) * sizeof(float);
-    if (e->mlp_smem > (size_t)prop.sharedMemPerBlockOptin) {
-        delete e;
-        return fail(AZG_EINVAL, "network does not fit in shared memory");
+    e->mlp_stream = H != 64 && H != 128;
+    if (!e->mlp_stream) {  // k_mlp stages the whole network in shared memory
+        e->mlp_smem = ((size_t)e->wcount + (size_t)MLP_NGRP * (H + e->PO_PAD) * MLP_UNIT) * sizeof(float);
+        if (e->mlp_smem > (size_t)prop.sharedMemPerBlockOptin) {
+            delete e;
+            return fail(AZG_EINVAL, "network does not fit in shared memory");
+        }
+    } else {  // k_mlp_stream: up to 16 warps of 64 x 32 tiles, as many 64-row blocks per pass as shared memory holds
+        MlpStreamPlan& sp = e->splan;
+        sp.H = H;
+        sp.NB = H / 32;
+        sp.RB = std::max(1, MLPS_MAX_THREADS / 32 / sp.NB);
+        while (sp.RB > 1 && mlp_stream_smem_bytes(H, c.state_dim, e->PO_PAD, 64 * sp.RB) > (size_t)prop.sharedMemPerBlockOptin) --sp.RB;
+        sp.RP = 64 * sp.RB;
+        sp.w0_floats = c.state_dim * H + H;
+        sp.head_off = e->wcount - (H * e->PO_PAD + e->PO_PAD);
+        e->mlp_smem = mlp_stream_smem_bytes(H, c.state_dim, e->PO_PAD, sp.RP);
+        if (e->mlp_smem > (size_t)prop.sharedMemPerBlockOptin) {
+            delete e;
+            return fail(AZG_EINVAL, "network does not fit in shared memory");
+        }
     }
     e->q8 = (c.flags & AZG_FLAG_EVAL_Q8) != 0;
     if (e->q8) {
@@ -384,7 +404,7 @@ extern "C" int32_t azg_head_dim(const azg_engine* e) {
     return e->cfg.variant == AZG_DISCRETE ? e->cfg.num_actions : e->K3;
 }
 
-// state_dict order -> packed k-major layout consumed by k_mlp
+// state_dict order -> packed k-major layout consumed by k_mlp and k_mlp_stream
 static void pack_weights(const azg_engine* e, const float* w, std::vector<float>& out) {
     const int H = e->cfg.hidden, S = e->cfg.state_dim, L = e->cfg.n_hidden, P = e->P, PO = e->PO_PAD;
     out.assign(e->wcount, 0.0f);
@@ -580,6 +600,14 @@ static cudaError_t launch_mlp_t(const azg_engine* e, const MlpParams& m, cudaStr
     return launch_ex(e, k_mlp<H, S, ACT>, grid, MLP_THREADS(H), e->mlp_smem, st, m);
 }
 
+template <int S, int ACT>
+static cudaError_t launch_mlp_stream_t(const azg_engine* e, const MlpParams& m, cudaStream_t st, bool set_attr) {
+    if (set_attr) return cudaFuncSetAttribute(k_mlp_stream<S, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)e->mlp_smem);
+    // one CTA per 64 rows up to one per SM: a thin batch spreads over more SMs in one-block passes instead of filling a few CTAs' passes
+    const int grid = std::max(1, std::min((m.n + 63) / 64, e->sm_count));
+    return launch_ex(e, k_mlp_stream<S, ACT>, grid, 32 * e->splan.NB * e->splan.RB, e->mlp_smem, st, m, e->splan);
+}
+
 // ENV (env.cuh) selects the tree and env of the whole-search kernels; the evaluation-only launch reads ENV::S (layer 0) alone
 template <class ENV, int ACT, int NL>
 static cudaError_t launch_qmlp_t(const azg_engine* e, const MlpParams& m, cudaStream_t st, bool set_attr) {
@@ -729,6 +757,16 @@ static cudaError_t launch_mlp(const azg_engine* e, const MlpParams& m, cudaStrea
         QMLP_CASE(4, 0, 1) QMLP_CASE(4, 1, 1) QMLP_CASE(3, 0, 1) QMLP_CASE(3, 1, 1)
         QMLP_CASE(4, 0, 2) QMLP_CASE(4, 1, 2) QMLP_CASE(3, 0, 2) QMLP_CASE(3, 1, 2)
 #undef QMLP_CASE
+        return cudaErrorInvalidValue;
+    }
+    if (e->mlp_stream) {  // hidden widths k_mlp cannot stage: S is the env's input width (2 both MountainCars, 3 Pendulum, 4 CartPole, 6 Acrobot)
+#define MLP_STREAM_CASE(s, a) \
+    if (S == s && A == a) return launch_mlp_stream_t<s, a>(e, m, st, set_attr);
+        MLP_STREAM_CASE(4, 0) MLP_STREAM_CASE(4, 1) MLP_STREAM_CASE(4, 2) MLP_STREAM_CASE(4, 3) MLP_STREAM_CASE(4, 4) MLP_STREAM_CASE(4, 5)
+        MLP_STREAM_CASE(3, 0) MLP_STREAM_CASE(3, 1) MLP_STREAM_CASE(3, 2) MLP_STREAM_CASE(3, 3) MLP_STREAM_CASE(3, 4) MLP_STREAM_CASE(3, 5)
+        MLP_STREAM_CASE(2, 0) MLP_STREAM_CASE(2, 1) MLP_STREAM_CASE(2, 2) MLP_STREAM_CASE(2, 3) MLP_STREAM_CASE(2, 4) MLP_STREAM_CASE(2, 5)
+        MLP_STREAM_CASE(6, 0) MLP_STREAM_CASE(6, 1) MLP_STREAM_CASE(6, 2) MLP_STREAM_CASE(6, 3) MLP_STREAM_CASE(6, 4) MLP_STREAM_CASE(6, 5)
+#undef MLP_STREAM_CASE
         return cudaErrorInvalidValue;
     }
     if (e->ac) {  // layer 0 with six inputs (Acrobot)

@@ -70,6 +70,9 @@ __device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t by
                  "l"(src), "r"(bytes), "r"(smem_u32(bar))
                  : "memory");
 }
+__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
+}
 __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
     uint32_t ok;
     asm volatile(

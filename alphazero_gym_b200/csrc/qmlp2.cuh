@@ -99,9 +99,6 @@ __device__ __forceinline__ void tmem_st4f(uint32_t taddr, float a, float b, floa
 }
 __device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
 // Phase boundary of the whole-search kernel: every participant arrives (release) and waits for the phase to complete (acquire), so
 // the global-memory writes of one phase (tree tables, X) are visible to the readers of the next.  An mbarrier like every other
 // cross-role synchronisation of this kernel (a 640-thread named barrier next to the MMA warpgroup parked at barrier 0 computes the

@@ -48,10 +48,12 @@ class EngineConfig:
     use_graph: bool = True
     # AZG_FLAG_EVAL_Q8: hidden x hidden layers on tcgen05 as exact int8-sliced products (include/azg.h).  None = on wherever the
     # tensor-core kernel serves the network (hidden 128, 2 or 3 hidden layers, at most 15 head outputs): the drop-in classes, the
-    # self-play driver and bench.py all run the same evaluation; False selects the FP32 FMA kernel (mlp.cuh)
+    # self-play driver and bench.py all run the same evaluation; False selects the FP32 FMA kernel (mlp.cuh).  Every other hidden
+    # width (a multiple of 32 up to 256) runs the FP32 kernel that streams the hidden layers (mlp_stream.cuh), which None picks
     eval_q8: Optional[bool] = None
     rng_mt19937: bool = False  # AZG_FLAG_RNG_MT19937: CPython's generator for the discrete search's selection draws (include/azg.h)
-    fused: Optional[bool] = None  # AZG_FLAG_FUSED: whole search in one persistent kernel; None = on where supported (eval_q8)
+    fused: Optional[bool] = None  # AZG_FLAG_FUSED: whole search in one persistent kernel; None = on where supported (eval_q8, so
+    # hidden 128 only: the other widths run one launch per simulation)
     # the env the search steps: None = the variant's own (CartPole-v0 / Pendulum-v0); MOUNTAIN_CAR_CONTINUOUS (continuous variant,
     # state_dim 2) sets AZG_FLAG_ENV_MOUNTAIN_CAR_CONTINUOUS; MOUNTAIN_CAR (discrete variant, num_actions 3, state_dim 2) sets
     # AZG_FLAG_ENV_MOUNTAIN_CAR; ACROBOT (discrete variant, num_actions 3, state_dim 6) sets AZG_FLAG_ENV_ACROBOT

@@ -58,7 +58,9 @@ typedef struct azg_config {
     int32_t num_actions;    /* discrete: 2 (CartPole), 3 (MountainCar-v0, Acrobot-v1) */
     int32_t num_components; /* continuous: K mixture components (1 = DiagonalNormalPolicy) */
     int32_t state_dim;      /* network input width: 4 CartPole, 3 Pendulum, 2 MountainCarContinuous and MountainCar, 6 Acrobot */
-    int32_t hidden;         /* hidden width (all hidden layers equal; 128 in both shipped configs) */
+    int32_t hidden;         /* hidden width (all hidden layers equal; 128 in both shipped configs): a multiple of 32 from 32 to 256.
+                               64 and 128 stage the whole network in shared memory; the other widths stream the hidden layers
+                               through it (FP32 only, one launch per simulation) */
     int32_t n_hidden;       /* hidden layers: 2 (DiscretePolicy.yaml) / 3 (ContinuousPolicy.yaml) */
     int32_t activation;     /* AZG_ACT_* */
     int32_t v_target;       /* AZG_VT_* (V_target_policy) */
